@@ -47,9 +47,9 @@ def test_population_rollout_at_n64_matches_oracle():
         np.testing.assert_allclose(fitness[m], f, rtol=1e-12)
 
 
-@pytest.mark.parametrize("N,P,W,n,max_steps", [(16, 6, 32, 4, 200), (8, 5, 20, 6, 150), (64, 3, 8, 6, 90)])
+@pytest.mark.parametrize("N,P,W,n,max_steps", [(64, 3, 8, 6, 90)])
 def test_fused_population_segments_equal_the_per_step_path(monkeypatch, N, P, W, n, max_steps):
-    """Population rollouts run as fused 64-step segments (policy inside the persistent kernels, per-step agent states recorded,
+    """Population rollouts run as fused 64-step segments (policy inside the persistent 64x64 kernel, per-step agent states recorded,
     members' bookkeeping in one post-pass, k_pop_post); DW_POP_UNFUSED=1 keeps the per-step launch sequence: same fitness bit
     for bit (same summation order), same stopping steps and step totals."""
     from therldaisyworld_b200.es import evaluate_population
@@ -57,7 +57,6 @@ def test_fused_population_segments_equal_the_per_step_path(monkeypatch, N, P, W,
     members = rng.randn(P, 1808) * 0.7
     members[0] = 0.0
     out = []
-    monkeypatch.setenv("DW_MLP_FUSE_SUB64", "1")          # the sub-64 kernel's in-kernel policy is opt-in (slower on this shape)
     for unfused in (False, True):
         if unfused:
             monkeypatch.setenv("DW_POP_UNFUSED", "1")

@@ -115,34 +115,3 @@ def test_in_kernel_mlp_equals_the_per_step_policy_path(monkeypatch):
     np.testing.assert_array_equal(a[4][0], b[4][0])
     np.testing.assert_array_equal(a[4][1], b[4][1])
     assert len(np.unique(a[1])) > 10          # the agents did move around
-
-
-@pytest.mark.parametrize("N,n,B", [(16, 4, 70), (8, 3, 200), (32, 9, 12)])
-def test_in_kernel_mlp_sub64_equals_the_per_step_policy_path(monkeypatch, N, n, B):
-    """The same comparison for the sub-64 persistent kernel (several worlds per CTA, four agents per warp pass, partially
-    filled CTAs, agent counts that are not a multiple of four)."""
-    from therldaisyworld_b200 import RLDaisyWorld
-    monkeypatch.setenv("DW_MLP_FUSE_SUB64", "1")          # opt-in path, see mlp_fusable (csrc/dw_run.inl)
-    rng = np.random.RandomState(12)
-    params = rng.randn(1808) * 1.5
-    out = []
-    for unfused in (False, True):
-        if unfused:
-            monkeypatch.setenv("DW_MLP_UNFUSED", "1")
-        else:
-            monkeypatch.delenv("DW_MLP_UNFUSED", raising=False)
-        np.random.seed(6)
-        env = RLDaisyWorld(grid_dimension=N, n_agents=n)
-        env.batch_size = B
-        env.reset()
-        env.set_mlp(params)
-        env.reset_lifespans()
-        env.run(2, policy="mlp")
-        env.run(45, policy="mlp")
-        obs = env.observe()
-        out.append((env.grid.copy(), env.agent_indices.copy(), env.agent_states.copy(), obs, env.lifespans()))
-    a, b = out
-    for i in range(4):
-        np.testing.assert_array_equal(a[i], b[i])
-    np.testing.assert_array_equal(a[4][0], b[4][0])
-    np.testing.assert_array_equal(a[4][1], b[4][1])

@@ -141,26 +141,3 @@ def test_device_reset_is_banding_invariant_and_fast_path_is_used():
     assert cov.max() > 0.05 and (cov * 1000 == np.rint(cov * 1000)).all()
     # the literal fallback must be the exception, not the rule
     assert one.band.slow_count() < 1e-3 * steps * N * N
-
-
-def test_persistent_stencil_ctas_equal_one_tile_per_cta(monkeypatch):
-    """k_tiled_step can walk several tiles per CTA with two staged TMA tiles (DW_TILED_PERSISTENT=1: only the resident CTAs are
-    launched; 2048 x 2048 = 1024 tiles > 4 x 148): same world as with the default one tile per CTA."""
-    N, n, steps = 2048, 600, 14
-    res = []
-    for persistent in (True, False):
-        if persistent:
-            monkeypatch.setenv("DW_TILED_PERSISTENT", "1")
-        else:
-            monkeypatch.delenv("DW_TILED_PERSISTENT", raising=False)
-        w = _world(N, n)
-        w.reset_on_device(seed=9)
-        w.run(steps, "greedy")
-        res.append((w.local_covers().copy(), w.agents(), w.lifespans(), w.cover_checksum()))
-    a, b = res
-    np.testing.assert_array_equal(a[0], b[0])
-    np.testing.assert_array_equal(a[1][0], b[1][0])
-    np.testing.assert_array_equal(a[1][1], b[1][1])
-    assert a[2][0] == b[2][0] and a[3] == b[3]
-    np.testing.assert_array_equal(a[2][1], b[2][1])
-    assert a[0].max() > 0.05

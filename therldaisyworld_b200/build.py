@@ -21,14 +21,6 @@ def sources():
     return [os.path.join(d, f) for f in os.listdir(d)] + [inc]
 
 
-def build_variant(name, defines, verbose=False):
-    """Kernel-tuning helper: build libdaisyworld_b200.<name>.so with extra -D flags (select it with DW_LIB=...)."""
-    out = os.path.join(PKG, f"libdaisyworld_b200.{name}.so")
-    cmd = [NVCC] + FLAGS + [f"-D{d}" for d in defines] + (["-Xptxas", "-v"] if verbose else []) + ["-o", out, SRC]
-    subprocess.check_call(cmd)
-    return out
-
-
 def build(force=False, verbose=False):
     if not force and os.path.exists(OUT) and all(os.path.getmtime(OUT) >= os.path.getmtime(s) for s in sources()):
         return OUT

@@ -102,7 +102,6 @@ struct dw_handle {
     unsigned int *persist_sync = nullptr;      // [1 + B] work queue + per-world progress of the persistent kernel
     int persist_blocks = 0, sub64_blocks = 0;  // resident CTAs of the persistent kernels on this device
     int sub64_blocks_series = 0;               // sub-64 kernel in series mode
-    int sub64_blocks_mlp = 0;                  // sub-64 kernel with the in-kernel MLP policy
     // statistics-only lifespan runs (dw_run_chunk_masked / dw_trim_lifespans): per-agent "not done" bits of the last chunk
     unsigned long long *alive_mask = nullptr;
     bool mask_on = false, mask_complete = false;
@@ -110,7 +109,7 @@ struct dw_handle {
     bool pop_rew_on = false;
     int persist_blocks_mlp = 0;                // the same for the kernel with the in-kernel MLP policy (more shared memory)
     int tile4_threads = 0;                     // block size chosen for k_fused_tile4
-    int tile4_blocks = 0, tile4_blocks_threads = 0;   // resident CTAs of the persistent 4x4-tile kernel (for that block size)
+    int tile4_blocks = 0, tile4_blocks_series = 0;    // resident CTAs of the persistent 4x4-tile kernel (plain / series mode)
     // profiling (dw_set_profiling): kernel launch count, and device time of the fused kernel via events
     dw_profile prof{};
     bool profiling = false;
@@ -267,7 +266,7 @@ template <class Src>
 static void launch_forward(dw_handle *h, const DevParams &P, double SL, Src src, double *out, double *writeback_b0,
                            unsigned long long *world_max, int zero6) {
     const size_t total = (size_t)P.B * h->NN;
-    if ((P.N & 1) == 0 && !getenv("DW_FORWARD_X1"))
+    if ((P.N & 1) == 0)
         k_forward_x2<Src><<<grid_for(total / 2), 256, 0, h->stream>>>(P, SL, src, out, writeback_b0, world_max, zero6);
     else
         k_forward<Src><<<grid_for(total), 256, 0, h->stream>>>(P, SL, src, out, writeback_b0, world_max, zero6);
@@ -275,7 +274,7 @@ static void launch_forward(dw_handle *h, const DevParams &P, double SL, Src src,
 template <class Src>
 static void launch_forward_lattice(dw_handle *h, const DevParams &P, double SL, Src src, uint32_t *lat_out, unsigned long long *world_max) {
     const size_t total = (size_t)P.B * h->NN;
-    if ((P.N & 1) == 0 && !getenv("DW_FORWARD_X1"))
+    if ((P.N & 1) == 0)
         k_forward_lattice_x2<Src><<<grid_for(total / 2), 256, 0, h->stream>>>(P, SL, src, lat_out, world_max);
     else
         k_forward_lattice<Src><<<grid_for(total), 256, 0, h->stream>>>(P, SL, src, lat_out, world_max);
@@ -644,9 +643,9 @@ static bool dw_fused_supported(const dw_handle *h);
 // step() keeps the state where the fused kernels keep it (packed lattice / lean reset planes) whenever the physics is one
 // the fast path covers: one K = 1 launch of the fused kernel instead of materialising the fp64 [B,7,N,N] grid (64 B per
 // cell). env.grid, diagnostics and observations are rebuilt on demand from the pre-state the step started from.
-// Partial actions (ab < B or am < n) and exotic kernels take the materialising path. DW_STEP_MATERIALISE=1 forces it.
+// Partial actions (ab < B or am < n) and exotic kernels take the materialising path.
 static bool lean_step_ok(const dw_handle *h, const int64_t *action, int32_t ab, int32_t am) {
-    if (!dw_fused_supported(h) || getenv("DW_STEP_MATERIALISE")) return false;
+    if (!dw_fused_supported(h)) return false;
     if (h->cfg.n_agents > 0 && action && (ab != h->cfg.batch || am != h->cfg.n_agents)) return false;
     return h->lat_valid || h->cov_valid || h->grid_valid;
 }

@@ -15,15 +15,8 @@
 #include <type_traits>
 #include "dw_common.cuh"
 
-#ifndef DW_N64_ROW_UNROLL
-#define DW_N64_ROW_UNROLL 4             // unroll factor of the 4-row tile loop (1 keeps the body inside the i-cache)
-#endif
-#ifndef DW_N64_MIN_BLOCKS
-#define DW_N64_MIN_BLOCKS 4
-#endif
-#ifndef DW_CELL_ILP
-#define DW_CELL_ILP 2                    // cells advanced in lockstep by the fast path (1, 2 or 4)
-#endif
+constexpr int kTileRowUnroll = 4;       // unroll factor of the 4-row tile loop (1 keeps the body inside the i-cache)
+constexpr int kN64MinBlocks = 4;        // resident CTAs per SM the 64x64 and sub-64 kernels are compiled for (64 registers)
 #define DW_FUSED_MAX_STEPS 4096        // longest launch (coefficient table / alive counters)
 #define DW_FUSED_MAX_AGENTS 1024
 #define DW_FIX_BITS 20                 // fixed-point fraction bits of the rounding trick (ulp of 1.5*2^32)
@@ -43,14 +36,13 @@ struct FastCoef {        // launch-constant coefficients of the fast path (host-
     // rounding + tie filter (see DW rounding note below): magic = 1.5*2^32 + 0.5 + eps*2^-FIX, tie_thresh = (2 eps) << (32-FIX)
     double magic;
     unsigned int tie_thresh, pad_;
-    // exponent-biased operands (DW_BIAS_MASK, dw_half2d): constants of the linear forms with the 2^20 offsets of the biased
-    // operands taken out -- rc: start value of rho's accumulation, magic_b: magic minus the offset of the centre cover,
-    // t0_b: t0 of the series mode
-    double rc, magic_b, t0_b;
+    // Unused. Keeps sizeof(FastCoef) and the offsets of the members after it in FusedArgs / LookArgs: the kernels that take
+    // them sit at 64 registers and their register allocation (and local-memory use) reacts to parameter offsets.
+    double pad_layout_[3];
 };
 struct StepCoef {        // per-step (luminosity dependent) coefficients
     double x0;           // g^2 * (cL + (q-cL)*A0 + (q2-q)*Al0 - q2*al)
-    double x0_b;         // x0 minus 2^20 * (the X coefficients of the exponent-biased operands), dw_fast_cells only
+    double pad_layout_;  // unused; keeps the 48-byte layout (without it k_tiled_step spills inside the DFMA chain)
     double xs_l, xs_d;   // g^2 * (q-cL)*a*(al-ab)/1000, g^2 * (q-cL)*a*(ad-ab)/1000   (a = adjacent tap)
     double SL;           // S*L for the literal path
     int policy, pad_;    // the policy of this step (DW_POLICY_EPS_GREEDY resolved to GREEDY / RANDOM on the host)
@@ -100,43 +92,11 @@ struct FusedArgs {
 __device__ __forceinline__ double dw_u2d(uint32_t k) {        // exact u32 -> f64 through the 2^52 trick
     return __hiloint2double(0x43300000, (int)k) - 4503599627370496.0;
 }
-// Packed half -> f64.  Two exact routes on different pipes: the 2^52 trick (LOP + MOV + DADD: 3 issue slots, 2 cycles of
-// the FP64 pipe) or I2F.F64.U16 (1 issue slot, 8 cycles of the XU pipe, which the MUFU seeds also use; measured on
-// B200 with tools/micro/thr.cu).  DW_I2F_MASK picks the route per operand (bit 0..5 = kl,kd,Sl,Sd,El,Ed) to balance
-// the issue port, the FP64 pipe and the XU pipe.
-#ifndef DW_I2F_MASK
-#define DW_I2F_MASK 0x3F
-#endif
-// Third route, no conversion at all: the 16-bit half k is dropped into the top mantissa bits of 2^20 by ONE byte permute
-// (hi word = 0x41300000 | k, lo word = 0), which IS the double 2^20 + k exactly (k < 2^20). Every use is a linear form
-// accumulated by FMAs, so the 2^20 offsets are taken out of the forms' constants on the host (FastCoef::rc, magic_b,
-// StepCoef::x0_b). Price: the partial sums are ~2^20 * coefficient instead of ~2^13 * coefficient, i.e. each FMA rounds
-// at a 2^7 times coarser ulp -- 2^-53 * 2^20 * (w0 + w12 + w2) * 3 = 1e-10 milli-cover on rho and 4 * 2^-53 * 2^20 * |xs| / X
-// = 5e-14 relative on X, both far inside the fast path's error budget (DESIGN.md section 2). DW_BIAS_MASK: same bit per
-// operand as DW_I2F_MASK (kl and kd share bit 0 and 1 -- they must use the same route because of magic_b).
-#ifndef DW_BIAS_MASK
-#define DW_BIAS_MASK 0x00
-#endif
-#ifndef DW_ROOT_ALT
-#define DW_ROOT_ALT 1                  // Newton step of the fourth root with one fp64 operation less (see dw_fast_cells)
-#endif
-#ifndef DW_AGENT_WARP
-#define DW_AGENT_WARP 0                // which warp of the 64x64 persistent kernel runs the agent phase (scheduling experiment)
-#endif
-#define DW_BIAS_OFFSET 1048576.0        // 2^20
-static_assert(((DW_BIAS_MASK & 1) != 0) == ((DW_BIAS_MASK & 2) != 0) && ((DW_BIAS_MASK & 4) != 0) == ((DW_BIAS_MASK & 8) != 0) &&
-              ((DW_BIAS_MASK & 16) != 0) == ((DW_BIAS_MASK & 32) != 0), "the two species of an operand share the conversion route (rc, magic_b)");
-template <int BIT>
+// Packed half -> f64 by I2F.F64.U16: one issue slot on the XU pipe. The 2^52 trick of dw_u2d costs three issue slots and
+// two cycles of the FP64 pipe, which bounds dw_fast_cells (DESIGN.md section 4).
+template <bool HI>
 __device__ __forceinline__ double dw_half2d(uint32_t p) {
-    if (DW_BIAS_MASK & (1 << BIT))
-        return __hiloint2double((int)__byte_perm(p, 0x41300000u, (BIT & 1) ? 0x7632 : 0x7610), 0);
-    if (BIT & 1) {
-        if (DW_I2F_MASK & (1 << BIT)) return (double)(unsigned short)(p >> 16);
-        return dw_u2d(p >> 16);
-    } else {
-        if (DW_I2F_MASK & (1 << BIT)) return (double)(unsigned short)(p & 0xffffu);
-        return dw_u2d(p & 0xffffu);
-    }
+    return HI ? (double)(unsigned short)(p >> 16) : (double)(unsigned short)(p & 0xffffu);
 }
 // Rounding of x (milli units) to the lattice with the tie filter folded into ONE add: f = low word of
 // x + (1.5*2^32 + 0.5 + EPS*2^-FIX) = round((x + 0.5) * 2^FIX) + EPS as a signed fixed-point number.
@@ -178,30 +138,27 @@ __device__ __forceinline__ void dw_fast_cells(const FastCoef &F, const StepCoef 
                                               const uint32_t (&S)[W], unsigned *tiemin, uint32_t (&out)[W], double *tsum = nullptr) {
     double kl[W], kd[W], El[W], Ed[W], Sl[W], Sd[W], Rl[W], Rd[W], rb[W], Xl[W], Xd[W];
 #pragma unroll
-    for (int i = 0; i < W; ++i) { kl[i] = dw_half2d<0>(pc[i]); kd[i] = dw_half2d<1>(pc[i]); }
+    for (int i = 0; i < W; ++i) { kl[i] = dw_half2d<false>(pc[i]); kd[i] = dw_half2d<true>(pc[i]); }
 #pragma unroll
-    for (int i = 0; i < W; ++i) { Sl[i] = dw_half2d<2>(S[i]); Sd[i] = dw_half2d<3>(S[i]); }
+    for (int i = 0; i < W; ++i) { Sl[i] = dw_half2d<false>(S[i]); Sd[i] = dw_half2d<true>(S[i]); }
 #pragma unroll
-    for (int i = 0; i < W; ++i) Xl[i] = __fma_rn(F.xk_l, kl[i], __fma_rn(F.xk_d, kd[i], DW_BIAS_MASK ? C.x0_b : C.x0));
+    for (int i = 0; i < W; ++i) Xl[i] = __fma_rn(F.xk_l, kl[i], __fma_rn(F.xk_d, kd[i], C.x0));
 #pragma unroll
     for (int i = 0; i < W; ++i) Xl[i] = __fma_rn(C.xs_l, Sl[i], __fma_rn(C.xs_d, Sd[i], Xl[i]));
 #pragma unroll
     for (int i = 0; i < W; ++i) Xd[i] = Xl[i] + F.xdd;
     if (DIAG) {              // series mode: the (unrounded) temperature of the cell itself, sqrt(g)*T, summed per thread
 #pragma unroll
-        for (int i = 0; i < W; ++i) *tsum += dw_root4_fast(__fma_rn(F.tk_l, kl[i], __fma_rn(F.tk_d, kd[i], Xl[i] + (DW_BIAS_MASK ? F.t0_b : F.t0))));
+        for (int i = 0; i < W; ++i) *tsum += dw_root4_fast(__fma_rn(F.tk_l, kl[i], __fma_rn(F.tk_d, kd[i], Xl[i] + F.t0)));
     }
     // seeds first: the MUFU latency (27 cycles) overlaps the rho arithmetic below
     double s1l[W], s1d[W], y0l[W], y0d[W];
 #pragma unroll
     for (int i = 0; i < W; ++i) { s1l[i] = dw_rsqrt_approx(Xl[i]); s1d[i] = dw_rsqrt_approx(Xd[i]); }
 #pragma unroll
-    for (int i = 0; i < W; ++i) { El[i] = dw_half2d<4>(E[i]); Ed[i] = dw_half2d<5>(E[i]); }
+    for (int i = 0; i < W; ++i) { El[i] = dw_half2d<false>(E[i]); Ed[i] = dw_half2d<true>(E[i]); }
 #pragma unroll
-    for (int i = 0; i < W; ++i) {
-        if (DW_BIAS_MASK) { Rl[i] = __fma_rn(F.w0, kl[i], F.rc); Rd[i] = __fma_rn(F.w0, kd[i], F.rc); }
-        else { Rl[i] = F.w0 * kl[i]; Rd[i] = F.w0 * kd[i]; }
-    }
+    for (int i = 0; i < W; ++i) { Rl[i] = F.w0 * kl[i]; Rd[i] = F.w0 * kd[i]; }
 #pragma unroll
     for (int i = 0; i < W; ++i) { y0l[i] = dw_rsqrt_approx(s1l[i]); y0d[i] = dw_rsqrt_approx(s1d[i]); }
 #pragma unroll
@@ -212,9 +169,8 @@ __device__ __forceinline__ void dw_fast_cells(const FastCoef &F, const StepCoef 
     for (int i = 0; i < W; ++i) rb[i] = __fma_rn(-F.dtm, Rl[i] + Rd[i], F.dtp);
     // Newton step on y^4 = X for both species of all cells, stage by stage
     double zl[W], zd[W], al[W], ad[W];
-#if DW_ROOT_ALT
-    // Same step, one fp64 operation less per root: T = y0 + (X - y0^4) * (s1/2)^2 * y0 with s1/2 made by an integer subtract on the
-    // exponent (ALU pipe; the MUFU seed's low word is zero), and Topt - T folded into the last FMA:
+    // The step of dw_root4_fast with one fp64 operation less per root: T = y0 + (X - y0^4) * (s1/2)^2 * y0 with s1/2 made by an
+    // integer subtract on the exponent (ALU pipe; the MUFU seed's low word is zero), and Topt - T folded into the last FMA:
     // dT = (Topt - y0) - ((X - y0^4) * (s1/2)^2) * y0.
 #pragma unroll
     for (int i = 0; i < W; ++i) {
@@ -227,18 +183,6 @@ __device__ __forceinline__ void dw_fast_cells(const FastCoef &F, const StepCoef 
     for (int i = 0; i < W; ++i) { zl[i] = zl[i] * al[i]; zd[i] = zd[i] * ad[i]; al[i] = F.topt - y0l[i]; ad[i] = F.topt - y0d[i]; }
 #pragma unroll
     for (int i = 0; i < W; ++i) { zl[i] = __fma_rn(-zl[i], y0l[i], al[i]); zd[i] = __fma_rn(-zd[i], y0d[i], ad[i]); }   // sqrt(g)*(Topt-T)
-#else
-#pragma unroll
-    for (int i = 0; i < W; ++i) { zl[i] = y0l[i] * y0l[i]; zd[i] = y0d[i] * y0d[i]; al[i] = s1l[i] * s1l[i]; ad[i] = s1d[i] * s1d[i]; }
-#pragma unroll
-    for (int i = 0; i < W; ++i) { zl[i] = __fma_rn(-zl[i], zl[i], Xl[i]); zd[i] = __fma_rn(-zd[i], zd[i], Xd[i]); al[i] = al[i] * y0l[i]; ad[i] = ad[i] * y0d[i]; }
-#pragma unroll
-    for (int i = 0; i < W; ++i) { zl[i] = zl[i] * al[i]; zd[i] = zd[i] * ad[i]; }
-#pragma unroll
-    for (int i = 0; i < W; ++i) { zl[i] = __fma_rn(zl[i], 0.25, y0l[i]); zd[i] = __fma_rn(zd[i], 0.25, y0d[i]); }      // T_l, T_d
-#pragma unroll
-    for (int i = 0; i < W; ++i) { zl[i] = F.topt - zl[i]; zd[i] = F.topt - zd[i]; }                                   // sqrt(g)*(Topt-T)
-#endif
 #pragma unroll
     for (int i = 0; i < W; ++i) { zl[i] = __fma_rn(-zl[i], zl[i], 1.0); zd[i] = __fma_rn(-zd[i], zd[i], 1.0); }       // beta_l, beta_d
 #pragma unroll
@@ -247,8 +191,7 @@ __device__ __forceinline__ void dw_fast_cells(const FastCoef &F, const StepCoef 
     for (int i = 0; i < W; ++i) { zl[i] = __fma_rn(Rl[i], zl[i], kl[i]); zd[i] = __fma_rn(Rd[i], zd[i], kd[i]); }     // l + dt*dl (milli)
 #pragma unroll
     for (int i = 0; i < W; ++i) {
-        const double mg = (DW_BIAS_MASK & 1) ? F.magic_b : F.magic;     // biased centre: zl = x + 2^20, the offset is in magic_b
-        const int fl = __double2loint(zl[i] + mg), fd = __double2loint(zd[i] + mg);
+        const int fl = __double2loint(zl[i] + F.magic), fd = __double2loint(zd[i] + F.magic);
         *tiemin = __vimin3_u32(*tiemin, (unsigned)fl << (32 - DW_FIX_BITS), (unsigned)fd << (32 - DW_FIX_BITS));
         const unsigned packed = __byte_perm((unsigned)(fl >> DW_FIX_BITS), (unsigned)(fd >> DW_FIX_BITS), 0x5410);
         out[i] = __vimin_s16x2_relu(packed, 1000u | (1000u << 16));
@@ -529,8 +472,7 @@ __device__ __forceinline__ uint32_t dw_tile_core(const FastCoef &F, const StepCo
     uint32_t mx = 0;
     Row6 top = rows.load(-1);
     Row6 mid = rows.load(0);
-    constexpr int kRowUnroll = DW_N64_ROW_UNROLL;
-#pragma unroll kRowUnroll
+#pragma unroll kTileRowUnroll
     for (int i = 0; i < 4; ++i) {
         const Row6 bot = rows.load(i + 1);
         uint32_t E[4], S8[4];
@@ -540,11 +482,7 @@ __device__ __forceinline__ uint32_t dw_tile_core(const FastCoef &F, const StepCo
             S8[c] = E[c] + top.hp[c] + bot.hp[c];
         }
         uint32_t q[4];
-#if DW_CELL_ILP == 1
-#pragma unroll
-        for (int c = 0; c < 4; ++c) q[c] = dw_fast_cell(F, C, mid.p[c], E[c], S8[c], tiemin);
-#elif DW_CELL_ILP == 2
-        {
+        {                                  // two cells in lockstep, twice (one or four at a time measured slower, DESIGN.md section 4)
             const uint32_t pa[2] = {mid.p[0], mid.p[1]}, ea[2] = {E[0], E[1]}, sa[2] = {S8[0], S8[1]};
             const uint32_t pb[2] = {mid.p[2], mid.p[3]}, eb[2] = {E[2], E[3]}, sb[2] = {S8[2], S8[3]};
             uint32_t qa[2], qb[2];
@@ -552,9 +490,6 @@ __device__ __forceinline__ uint32_t dw_tile_core(const FastCoef &F, const StepCo
             dw_fast_cells<2, DIAG>(F, C, pb, eb, sb, tiemin, qb, tsum);
             q[0] = qa[0]; q[1] = qa[1]; q[2] = qb[0]; q[3] = qb[1];
         }
-#else
-        dw_fast_cells<4, DIAG>(F, C, mid.p, E, S8, tiemin, q, tsum);
-#endif
         if (Store::kMasks) {               // k_fused_tile4, padded sides: the store zeroes entries that lie outside the world
             store(i, q);
 #pragma unroll
@@ -583,7 +518,7 @@ __device__ __forceinline__ uint32_t dw_tile_step64(const FusedArgs &A, int j, co
     return mx;
 }
 
-__global__ void __launch_bounds__(256, DW_N64_MIN_BLOCKS) k_fused_n64(const __grid_constant__ FusedArgs A) {
+__global__ void __launch_bounds__(256, kN64MinBlocks) k_fused_n64(const __grid_constant__ FusedArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int N = 64, NN = N * N;
     const int n = A.P.n_agents;
@@ -667,7 +602,7 @@ __global__ void __launch_bounds__(256, DW_N64_MIN_BLOCKS) k_fused_n64(const __gr
 
 // ---- 64x64, persistent: one world per CTA-item, dynamic work queue ----------------------------------------------------
 // Work item = (world, chunk of Kc steps), handed out chunk-major from a global counter: all worlds of the ensemble
-// advance together and every SM keeps DW_N64_MIN_BLOCKS CTAs busy until the end of the launch, which removes the
+// advance together and every SM keeps kN64MinBlocks CTAs busy until the end of the launch, which removes the
 // wave quantisation of a one-CTA-per-world grid (1000 worlds on 148 SMs x 4 CTAs = 1.69 waves).
 // Shared memory is STATIC (compile-time addresses: no pointer registers, immediate LDS/STS offsets) and the agent
 // phase is the single-pass warp version below, so this kernel takes worlds with at most DW_N64_MAX_AGENTS agents;
@@ -743,133 +678,14 @@ __device__ __forceinline__ void dw_agents_phase32(const FusedArgs &A, int j, int
 // still holds the post-graze state the previous step started from, so the nine window cells are re-evaluated from it exactly
 // as forward stored them (screened cell, literal next to ties; b' from the unrounded covers, rounded temperatures, agent
 // stamp: last agent on a cell wins) -- the same arithmetic as k_obs_mlp, which stays the path of every other kernel family.
-// One warp per agent: lanes 0..8 the window cells, then lanes = output neurons (16, 32, 9), sequential sums in k order.
-// Four agents of one world per warp (lane utilisation: one warp per agent keeps 9-16 of 32 lanes busy and costs ~1200
-// warp-instructions per agent; packed it is ~1700 per four agents). Every output neuron is still ONE accumulator summed in k
-// order with separate multiply and add, so the values are those of k_mlp_act / k_obs_mlp bit for bit.
-struct MlpScratch {            // per warp; h2 aliases x (dead after layer 1), o aliases h1 (dead after layer 2)
-    double x[4][64];
-    double h1[4][16];
-};
+// One warp per agent: lanes 0..8 the window cells, then lanes = output neurons (16, 32, 9). Every output neuron is ONE
+// accumulator summed in k order with separate multiply and add, so the values are those of k_mlp_act / k_obs_mlp bit for bit.
 #define DW_MLP_W1 (63 * 16)
 #define DW_MLP_W2 (16 * 32)
 #define DW_MLP_NPARAMS (63 * 16 + 16 * 32 + 32 * 9)
 
-// pb: the post-graze lattice the previous step started from, 64 words per row, world of side N at (r0w, c0w); xyw / stw: the
-// world's agents (x | y << 16, state after the previous step); agents a0 .. a0+3 (those < n) get their action in actw[].
-// wset[q]: weight set of agent a0 + q.
-template <int N>
-__device__ __noinline__ void dw_mlp_decide4(const FusedArgs *Ap, double SL, const uint32_t *pb, int r0w, int c0w, const int *xyw,
-                                            const double *stw, int n, int a0, const int (&wset)[4], MlpScratch *ms, int *actw, int lane) {
-    const FusedArgs &A = *Ap;
-    const DevParams &P = A.P;
-    // ---- observation windows: task t = cell * 4 + agent (the corner cell 8 of all four agents forms the second pass, which a
-    // Von Neumann mask skips); cells with a zero mask contribute exact zeros and are not evaluated
-#pragma unroll 1
-    for (int pass = 0; pass < 2; ++pass) {
-        const int t = lane + 32 * pass;
-        const int cell = t >> 2, q = t & 3, a = a0 + q;
-        const bool in = t < 36;
-        const double m = in ? P.mask[cell] : 0.0;
-        const bool eval = in && a < n && m != 0.0;
-        if (pass == 1 && !__any_sync(0xffffffffu, eval)) {
-            if (in) for (int ch = 0; ch < 7; ++ch) ms->x[q][ch * 9 + cell] = 0.0;
-            break;
-        }
-        double v[7] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-        if (eval) {
-            const int cx = ((xyw[a] & 0xffff) + cell / 3 + N - 1) & (N - 1), cy = ((xyw[a] >> 16) + cell % 3 + N - 1) & (N - 1);
-            double l9[9], d9[9];
-#pragma unroll
-            for (int i = 0; i < 3; ++i)
-#pragma unroll
-                for (int c = 0; c < 3; ++c) {
-                    const uint32_t k = pb[(r0w + ((cx + i + N - 1) & (N - 1))) * 64 + c0w + ((cy + c + N - 1) & (N - 1))];
-                    l9[i * 3 + c] = dw_milli(k & 0xffffu);
-                    d9[i * 3 + c] = dw_milli(k >> 16);
-                }
-            ScrCell c;
-            if (!(P.screen && dw_screened_cell(P, SL / P.sigma, l9, d9, c))) dw_literal_rounded(P, SL, l9, d9, c);
-            double ch4 = dw_k2v(c.k[4]);
-            for (int k = 0; k < n; ++k)
-                if ((xyw[k] & 0xffff) == cx && (xyw[k] >> 16) == cy) ch4 = stw[k];
-            v[0] = dw_k2v(c.k[0]) * m; v[1] = dw_k2v(c.k[1]) * m; v[2] = dw_k2v(c.k[2]) * m; v[3] = dw_k2v(c.k[3]) * m;
-            v[4] = ch4 * m; v[5] = dw_k2v(c.k[5]) * m; v[6] = 0.0 * m;
-        }
-        if (in) {
-#pragma unroll
-            for (int ch = 0; ch < 7; ++ch) ms->x[q][ch * 9 + cell] = v[ch];
-        }
-    }
-    __syncwarp();
-    const double *wq[4];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) wq[q] = A.mlp_w + (size_t)wset[q] * DW_MLP_NPARAMS;
-    // ---- layer 1: lane = (agent pair, neuron); products 21 at a time, then the sums in k order
-    {
-        const int g = lane >> 4, o = lane & 15;
-        const double *wa = wq[2 * g], *wb = wq[2 * g + 1];
-        const double *xa = ms->x[2 * g], *xb = ms->x[2 * g + 1];
-        double ha = 0.0, hb = 0.0;
-#pragma unroll 1
-        for (int k0 = 0; k0 < 63; k0 += 21) {
-            double pa[21], pbv[21];
-#pragma unroll
-            for (int k = 0; k < 21; ++k) {
-                pa[k] = xa[k0 + k] * __ldg(wa + (k0 + k) * 16 + o);
-                pbv[k] = xb[k0 + k] * __ldg(wb + (k0 + k) * 16 + o);
-            }
-#pragma unroll
-            for (int k = 0; k < 21; ++k) { ha = ha + pa[k]; hb = hb + pbv[k]; }
-        }
-        __syncwarp();                           // every lane is done reading x before h1 ... (h2 below aliases x)
-        ms->h1[2 * g][o] = ha * (ha > 0.0 ? 1.0 : 0.0);
-        ms->h1[2 * g + 1][o] = hb * (hb > 0.0 ? 1.0 : 0.0);
-    }
-    __syncwarp();
-    // ---- layer 2: lane = neuron, four agents
-    double (*h2)[32] = reinterpret_cast<double (*)[32]>(&ms->x[0][0]);          // [4][32]
-    {
-        double h[4] = {0.0, 0.0, 0.0, 0.0};
-#pragma unroll
-        for (int k = 0; k < 16; ++k) {
-#pragma unroll
-            for (int q = 0; q < 4; ++q) h[q] = h[q] + ms->h1[q][k] * __ldg(wq[q] + DW_MLP_W1 + k * 32 + lane);
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q) h2[q][lane] = h[q] * (h[q] > 0.0 ? 1.0 : 0.0);
-    }
-    __syncwarp();
-    // ---- layer 3: lane = (agent, output 0..7), then output 8 of the four agents on lanes 0..3
-    double (*outv)[16] = ms->h1;                                                 // [4][16], h1 is dead
-    {
-        const int q = lane >> 3, o = lane & 7;
-        const double *w3 = wq[q] + DW_MLP_W1 + DW_MLP_W2;
-        double s8 = 0.0, s9 = 0.0;
-#pragma unroll
-        for (int k = 0; k < 32; ++k) s8 = s8 + h2[q][k] * __ldg(w3 + k * 9 + o);
-        if (lane < 4) {
-            const double *w3b = wq[lane] + DW_MLP_W1 + DW_MLP_W2;
-#pragma unroll
-            for (int k = 0; k < 32; ++k) s9 = s9 + h2[lane][k] * __ldg(w3b + k * 9 + 8);
-        }
-        __syncwarp();                           // layer-2 reads of h1 are long done; outv aliases it
-        outv[q][o] = s8;
-        if (lane < 4) outv[lane][8] = s9;
-    }
-    __syncwarp();
-    if (lane < 4 && a0 + lane < n) {
-        int best = 0;
-        double bv = outv[lane][0];
-#pragma unroll
-        for (int o = 1; o < 9; ++o) if (outv[lane][o] > bv) { bv = outv[lane][o]; best = o; }
-        actw[a0 + lane] = best;
-    }
-    __syncwarp();
-}
-
-// One warp per agent (the 64x64 kernel): lanes 0..8 the window cells, then lanes = output neurons (16, 32, 9). Measured
-// against the packed routine above inside k_fused_n64_persist at 1000 worlds x 4 agents: 8.7 ms vs 10.6 ms per 383 steps --
+// Measured against a packed routine (four agents of one world per warp, ~1700 warp-instructions per four agents against ~1200
+// per agent) inside k_fused_n64_persist at 1000 worlds x 4 agents: 8.7 ms vs 10.6 ms per 383 steps --
 // with 4 CTAs per SM the policy phase is bound by the latency of its dependent chain, not by its instruction count, so four
 // agents on four warps beat four agents on one.
 __device__ __noinline__ void dw_mlp_decide64(const FusedArgs *Ap, double SL, const uint32_t *pb, const N64Smem *smp, double *scr, int *act, int n,
@@ -953,7 +769,7 @@ struct MlpSmem {
 };
 
 template <bool DIAG, bool MLP = false>
-__global__ void __launch_bounds__(256, DW_N64_MIN_BLOCKS) k_fused_n64_persist(const __grid_constant__ FusedArgs A) {
+__global__ void __launch_bounds__(256, kN64MinBlocks) k_fused_n64_persist(const __grid_constant__ FusedArgs A) {
     __shared__ N64Smem sm;
     __shared__ double s_tsum;
     __shared__ unsigned int s_cov[2];
@@ -1019,10 +835,8 @@ __global__ void __launch_bounds__(256, DW_N64_MIN_BLOCKS) k_fused_n64_persist(co
                 mlp_act = s_mlp.act;
                 __syncthreads();
             }
-            if (warp == DW_AGENT_WARP && n > 0) dw_agents_phase32(A, j, b, cb, sm, lane, n, mlp_act);
-#ifndef DW_X_NOSYNC1            // timing experiments only (results are garbage without the barriers): upper bound of what removing
-            __syncthreads();    // a barrier could buy, see DESIGN.md section 4
-#endif
+            if (warp == 0 && n > 0) dw_agents_phase32(A, j, b, cb, sm, lane, n, mlp_act);
+            __syncthreads();
             if (!MLP && j == A.K - 1) {
                 uint4 *gp = reinterpret_cast<uint4 *>(A.lat_pre + (size_t)b * NN);
 #pragma unroll
@@ -1047,9 +861,7 @@ __global__ void __launch_bounds__(256, DW_N64_MIN_BLOCKS) k_fused_n64_persist(co
                 cd = __reduce_add_sync(0xffffffffu, cd);
                 if (lane == 0) { atomicAdd(&s_tsum, tsum); atomicAdd(&s_cov[0], cl); atomicAdd(&s_cov[1], cd); }
             }
-#ifndef DW_X_NOSYNC2
             __syncthreads();
-#endif
             if (DIAG && tid == 0) {
                 atomicAdd(A.series_T + j, s_tsum);
                 atomicAdd(A.series_l + j, (unsigned long long)s_cov[0]);
@@ -1194,7 +1006,7 @@ __device__ __noinline__ bool dw_fix_warp_sub(const FusedArgs *A, const StepCoef 
 // independent, so the warps of a CTA run their agent phases concurrently.
 template <int N>
 __device__ __forceinline__ void dw_agents_phase_sub(const FusedArgs &A, int j, int group, uint32_t *cb, Sub64Smem<N> &sm, int lane, int n,
-                                                    int a_lo, int n_act, const int *mlp_act = nullptr) {
+                                                    int a_lo, int n_act) {
     constexpr int WX = 64 / N, W = WX * WX;
     const int pol = A.sc[j].policy;
     // pass 1: every agent decides from the pre-move state
@@ -1203,8 +1015,7 @@ __device__ __forceinline__ void dw_agents_phase_sub(const FusedArgs &A, int j, i
         const int x = sm.xy[a] & 0xffff, y = sm.xy[a] >> 16;
         const size_t gw = (size_t)group * W + wl;
         int act = 0;
-        if (pol == DW_POLICY_MLP) act = mlp_act[a];          // decided by dw_mlp_decide4 before this phase
-        else if (pol == DW_POLICY_REPLAY) act = A.actions[((size_t)j * A.P.B + gw) * n + i];
+        if (pol == DW_POLICY_REPLAY) act = A.actions[((size_t)j * A.P.B + gw) * n + i];
         else if (pol == DW_POLICY_RANDOM) act = (int)(dw_hash_rng(A.seed, A.world0 + (uint32_t)gw, i, A.step0 + j) % 9u);
         else if (pol != DW_POLICY_NONE) {
             const int r = (wl / WX) * N, c = (wl % WX) * N;
@@ -1255,19 +1066,14 @@ __device__ __forceinline__ void dw_agents_phase_sub(const FusedArgs &A, int j, i
             sm.xy[a] = x | (y << 16);
             sm.ada[a] += (st < 0.1) ? 0 : 1;
             if (A.alive_mask && !(st < 0.1)) sm.am[a] |= 1ull << (j & 63);
-            if (A.rew_series) A.rew_series[((size_t)j * A.P.B + (size_t)group * W) * n + a] = st;
         }
         __syncwarp();
     }
 }
 
-// MLP = true: DW_POLICY_MLP inside the kernel like k_fused_n64_persist<.., true>; every warp runs the policy of its own worlds'
-// agents, four at a time (dw_mlp_decide4). Dynamic shared memory: 8 MlpScratch + int[DW_SUB64_MAX_AGENTS] actions.
-#define DW_SUB64_MLP_SMEM (8 * sizeof(MlpScratch) + DW_SUB64_MAX_AGENTS * sizeof(int))
-template <int N, bool DIAG = false, bool MLP = false>
-__global__ void __launch_bounds__(256, MLP ? 3 : DW_N64_MIN_BLOCKS) k_fused_sub64_persist(const __grid_constant__ FusedArgs A) {
+template <int N, bool DIAG = false>
+__global__ void __launch_bounds__(256, kN64MinBlocks) k_fused_sub64_persist(const __grid_constant__ FusedArgs A) {
     constexpr int WX = 64 / N, W = WX * WX, TX = N / 4;
-    extern __shared__ __align__(16) unsigned char dyn_smem[];
     __shared__ Sub64Smem<N> sm;
     __shared__ double s_tsum;               // series mode (DIAG): per-step sums over the CTA's worlds, see k_fused_n64_persist
     __shared__ unsigned int s_cov[2];
@@ -1308,15 +1114,6 @@ __global__ void __launch_bounds__(256, MLP ? 3 : DW_N64_MIN_BLOCKS) k_fused_sub6
             if (w < n_worlds) v = __ldcg(reinterpret_cast<const uint4 *>(A.lat + ((size_t)g * W + w) * (N * N) + (R % N) * N + (C4 % N)));
             reinterpret_cast<uint4 *>(sm.buf[0])[q] = v;
         }
-        if (MLP) {   // the post-graze state the step before this item started from (observation windows of the item's first step)
-            for (int q = tid; q < 1024; q += 256) {
-                const int R = q >> 4, C4 = (q & 15) * 4;
-                const int w = (R / N) * WX + C4 / N;
-                uint4 v = make_uint4(0u, 0u, 0u, 0u);
-                if (w < n_worlds) v = __ldcg(reinterpret_cast<const uint4 *>(A.lat_pre + ((size_t)g * W + w) * (N * N) + (R % N) * N + (C4 % N)));
-                reinterpret_cast<uint4 *>(sm.buf[1])[q] = v;
-            }
-        }
         for (int a = tid; a < n_act; a += 256) {
             const size_t ga = (size_t)g * W * n + a;
             sm.st[a] = __ldcg(A.agent_state + ga);
@@ -1336,30 +1133,10 @@ __global__ void __launch_bounds__(256, MLP ? 3 : DW_N64_MIN_BLOCKS) k_fused_sub6
             {   // warp k moves the agents of worlds [k * WPW, (k + 1) * WPW) of the group
                 constexpr int WPW = (W + 7) / 8;
                 const int w_lo = warp * WPW, w_hi = min(w_lo + WPW, n_worlds);
-                const int *mlp_act = nullptr;
-                if constexpr (MLP) {
-                    MlpScratch *scr = reinterpret_cast<MlpScratch *>(dyn_smem) + warp;
-                    int *acts = reinterpret_cast<int *>(dyn_smem + 8 * sizeof(MlpScratch));
-                    mlp_act = acts;
-                    if (n > 0 && A.sc[j].policy == DW_POLICY_MLP) {
-                        const double SLp = j == 0 ? A.SL_prev : A.sc[j - 1].SL;
-                        for (int w = w_lo; w < w_hi; ++w) {
-                            const int gw = g * W + w;
-                            for (int a0 = 0; a0 < n; a0 += 4) {
-                                int wset[4];
-#pragma unroll
-                                for (int q = 0; q < 4; ++q) wset[q] = A.mlp_wpm > 0 ? (a0 + q < A.mlp_half ? gw / A.mlp_wpm : A.mlp_adv) : 0;
-                                dw_mlp_decide4<N>(&A, SLp, nb, (w / WX) * N, (w % WX) * N, sm.xy + w * n, sm.st + w * n, n, a0, wset, scr,
-                                                  acts + w * n, lane);
-                            }
-                        }
-                    }
-                    // the warp's own worlds only: decisions (reads of nb, xy, st) and moves (writes of cb, xy, st) need no CTA barrier
-                }
-                if (w_lo < w_hi && n > 0) dw_agents_phase_sub<N>(A, j, g, cb, sm, lane, n, w_lo * n, w_hi * n, mlp_act);
+                if (w_lo < w_hi && n > 0) dw_agents_phase_sub<N>(A, j, g, cb, sm, lane, n, w_lo * n, w_hi * n);
             }
             __syncthreads();
-            if (!MLP && j == A.K - 1) {                // post-graze state of the launch's last step (lazy materialisation)
+            if (j == A.K - 1) {                        // post-graze state of the launch's last step (lazy materialisation)
                 for (int q = tid; q < 1024; q += 256) {
                     const int R = q >> 4, C4 = (q & 15) * 4;
                     const int w = (R / N) * WX + C4 / N;
@@ -1420,9 +1197,6 @@ __global__ void __launch_bounds__(256, MLP ? 3 : DW_N64_MIN_BLOCKS) k_fused_sub6
             if (w < n_worlds) {
                 *reinterpret_cast<uint4 *>(A.lat + ((size_t)g * W + w) * (N * N) + (R % N) * N + (C4 % N)) =
                     reinterpret_cast<const uint4 *>(sm.buf[kc & 1])[q];
-                if (MLP)        // post-graze state of the item's last step: next item's windows / lazy materialisation
-                    *reinterpret_cast<uint4 *>(A.lat_pre + ((size_t)g * W + w) * (N * N) + (R % N) * N + (C4 % N)) =
-                        reinterpret_cast<const uint4 *>(sm.buf[(kc + 1) & 1])[q];
             }
         }
         for (int a = tid; a < n_act; a += 256) {

@@ -490,9 +490,6 @@ __device__ __noinline__ uint32_t dwt_fix_warp(const TiledArgs *A, const uint32_t
     return __vmaxu2(mine ? 0u : mx, extra);
 }
 
-// A CTA walks the tiles blockIdx.x, blockIdx.x + gridDim.x, ... of the launch with TWO staged tiles: the TMA load of the next
-// tile is issued before the current one is computed. The default launch is one tile per CTA (gridDim.x = number of tiles);
-// the persistent form (gridDim.x = resident CTAs, DW_TILED_PERSISTENT=1) was measured slower, see dwt_stencil_grid.
 __device__ __forceinline__ void dwt_issue_tile(const CUtensorMap *tmap, const TiledArgs &A, int t, uint32_t smem_tile, uint32_t bar_a) {
     const int tc = t % A.tiles_x;
     int tr = A.tr_first + t / A.tiles_x;
@@ -504,47 +501,43 @@ __device__ __forceinline__ void dwt_issue_tile(const CUtensorMap *tmap, const Ti
                  : "memory");
 }
 
-template <int STAGES>        // 1: the default one-tile-per-CTA launch (19 KB of shared memory); 2: persistent form with prefetch
+// One tile per CTA (gridDim.x = number of tiles, 19 KB of shared memory). A grid of fewer CTAs also works: a CTA then walks
+// the tiles blockIdx.x, blockIdx.x + gridDim.x, ... and loads the next one once the current one is computed.
 __global__ void __launch_bounds__(256, 4) k_tiled_step(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ TiledArgs A,
                                                        int n_tiles) {
-    constexpr int kStageWords = ((DWT_TILE_BYTES + 127) / 128) * 32;      // a TMA destination must be 128-byte aligned: 19008 -> 19072 B
-    __shared__ __align__(128) uint32_t tile[STAGES][kStageWords];
-    __shared__ __align__(8) unsigned long long bar[2];
+    constexpr int kTileWords = ((DWT_TILE_BYTES + 127) / 128) * 32;       // a TMA destination must be 128-byte aligned: 19008 -> 19072 B
+    __shared__ __align__(128) uint32_t tile[kTileWords];
+    __shared__ __align__(8) unsigned long long bar;
     __shared__ int smax[2];
     const int tid = threadIdx.x, lane = tid & 31;
     const int tx = tid & 15, r0 = (tid >> 4) * 4;
-    const uint32_t bar_a[2] = {dwt_smem_u32(&bar[0]), dwt_smem_u32(&bar[1])};
-    const uint32_t tile_a[2] = {dwt_smem_u32(tile[0]), dwt_smem_u32(tile[STAGES - 1])};
+    const uint32_t bar_a = dwt_smem_u32(&bar), tile_a = dwt_smem_u32(tile);
     int t = blockIdx.x;
     if (tid == 0) {
         smax[0] = 0; smax[1] = 0;
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a[0]));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a[1]));
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        if (t < n_tiles) dwt_issue_tile(&tmap, A, t, tile_a[0], bar_a[0]);
+        if (t < n_tiles) dwt_issue_tile(&tmap, A, t, tile_a, bar_a);
     }
-    __syncthreads();                                     // barriers initialised (and the first one armed) before anyone polls
+    __syncthreads();                                     // barrier initialised (and armed) before anyone polls
     const int tile_off = (1 + r0) * DWT_TILE_PITCH + 4 + 4 * tx;
     uint32_t mx_all = 0;
     for (int k = 0; t < n_tiles; ++k, t += gridDim.x) {
-        const int s = STAGES == 2 ? (k & 1) : 0;
-        // the other stage was last read in iteration k-1, which ended with a CTA barrier: free to be refilled
-        if (STAGES == 2 && tid == 0 && t + (int)gridDim.x < n_tiles) dwt_issue_tile(&tmap, A, t + gridDim.x, tile_a[s ^ 1], bar_a[s ^ 1]);
         {
-            const uint32_t parity = (uint32_t)(STAGES == 2 ? (k >> 1) : k) & 1u;
+            const uint32_t parity = (uint32_t)k & 1u;
             uint32_t ok = 0;
             while (!ok)
                 asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                             : "=r"(ok) : "r"(bar_a[s]), "r"(parity) : "memory");
+                             : "=r"(ok) : "r"(bar_a), "r"(parity) : "memory");
         }
         const int tc = t % A.tiles_x;
         int tr = A.tr_first + t / A.tiles_x;
         if (tr >= A.tr_skip_lo) tr += A.tr_skip_hi - A.tr_skip_lo;
         const long long out_off = (long long)(tr * DWT_TILE + 1 + r0) * A.pitch + 4 + tc * DWT_TILE + 4 * tx;
         unsigned tiemin = 0xffffffffu;
-        uint32_t mx = dw_tile_core(A.F, A.C, RowsTile72{tile[s] + tile_off}, StoreGlobal{A.out + out_off, A.pitch}, &tiemin);
+        uint32_t mx = dw_tile_core(A.F, A.C, RowsTile72{tile + tile_off}, StoreGlobal{A.out + out_off, A.pitch}, &tiemin);
         const unsigned flagged = __ballot_sync(0xffffffffu, tiemin < A.F.tie_thresh);
-        if (flagged) mx = dwt_fix_warp(&A, tile[s], flagged, mx, tile_off, out_off, lane);
+        if (flagged) mx = dwt_fix_warp(&A, tile, flagged, mx, tile_off, out_off, lane);
         // ghost columns of the produced rows: the two threads of a row group that hold column 0 / N-1 copy their (final) cells
         if (tx == 0 && tc == 0) {
             uint32_t *o = A.out + out_off;
@@ -556,8 +549,8 @@ __global__ void __launch_bounds__(256, 4) k_tiled_step(const __grid_constant__ C
             for (int i = 0; i < 4; ++i) o[(size_t)i * A.pitch - A.N] = o[(size_t)i * A.pitch];
         }
         mx_all = __vmaxu2(mx_all, mx);
-        __syncthreads();                                 // every read of tile[s] is done before the next iteration refills it
-        if (STAGES == 1 && tid == 0 && t + (int)gridDim.x < n_tiles) dwt_issue_tile(&tmap, A, t + gridDim.x, tile_a[0], bar_a[0]);
+        __syncthreads();                                 // every read of the tile is done before the next iteration refills it
+        if (tid == 0 && t + (int)gridDim.x < n_tiles) dwt_issue_tile(&tmap, A, t + gridDim.x, tile_a, bar_a);
     }
     const unsigned ml = __reduce_max_sync(0xffffffffu, mx_all & 0xffffu), md = __reduce_max_sync(0xffffffffu, mx_all >> 16);
     if (lane == 0) { atomicMax(&smax[0], (int)ml); atomicMax(&smax[1], (int)md); }

@@ -109,9 +109,6 @@ def simulate_lifespan(shard, policy="greedy", actions=None, seed=0, max_steps=10
     steps = 0
     hit = False
     can_trim = getattr(shard, "trim_supported", None)
-    import os
-    if segment is None and os.environ.get("DW_SEGMENT"):        # measurement override
-        segment = int(os.environ["DW_SEGMENT"])
     auto = segment is None
     short = 64
     if auto and hasattr(shard, "suggest_segment"):

@@ -1,7 +1,7 @@
 """The drop-in step() path as a reference caller uses it (daisy/agents/greedy.py:39-89, daisy/evo/sges.py:152-175): one
 env.step(action) per iteration with a host policy, observation / reward / done downloaded every step -- against
 step_policy (action chosen on the device) with and without the observation download. The state stays lattice-resident
-(K = 1 launches of the fused kernel); DW_STEP_MATERIALISE=1 gives the old materialising path for comparison."""
+(K = 1 launches of the fused kernel)."""
 import json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np

@@ -1,4 +1,6 @@
-"""Time the fused path in isolation: B worlds of 64x64, T steps from a post-first-step checkpoint."""
+"""Time the fused path in isolation: B worlds of 64x64, T steps from a post-first-step checkpoint.
+python tools/fused_bench.py [quick | mlp]. `quick` is the short set the kernel tuning in DESIGN.md section 4 was measured on;
+run it once per build (DW_LIB=<path to the .so>) to compare two builds."""
 import sys, os, time, ctypes as C
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -28,7 +30,8 @@ if __name__ == "__main__":
         print("lib:", os.environ.get("DW_LIB", "default"))
         bench(1000, 4, "greedy"); bench(4736, 4, "greedy"); bench(4736, 0, "none")
         sys.exit(0)
-    if len(sys.argv) > 1 and sys.argv[1] == "mlp":     # wall time is the measure (DW_MLP_UNFUSED=1: policy between one-step launches)
+    if len(sys.argv) > 1 and sys.argv[1] == "mlp":     # wall time is the measure (DW_MLP_UNFUSED=1: policy between one-step launches,
+                                                       # the reference path the tests compare the in-kernel policy with)
         for B in (1000, 10000, 100000):
             bench(B, 4, "mlp", T=128 if B > 20000 else 383)
         sys.exit(0)

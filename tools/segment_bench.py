@@ -10,10 +10,9 @@ B = int(sys.argv[1]) if len(sys.argv) > 1 else 100000
 np.random.seed(0)
 env = RLDaisyWorld(grid_dimension=64)
 env.batch_size = B
-for label, envs in (("auto (trimmed)", {}), ("segment 64 trimmed", {"DW_SEGMENT": "64"}), ("segment 32 trimmed", {"DW_SEGMENT": "32"}),
-                    ("segment 16 trimmed", {"DW_SEGMENT": "16"}), ("segment 64 checkpoint+replay", {"DW_SEGMENT": "64", "DW_NO_TRIM": "1"})):
-    for k in ("DW_SEGMENT", "DW_NO_TRIM"):
-        os.environ.pop(k, None)
+for label, segment, envs in (("auto (trimmed)", None, {}), ("segment 64 trimmed", 64, {}), ("segment 32 trimmed", 32, {}),
+                             ("segment 16 trimmed", 16, {}), ("segment 64 checkpoint+replay", 64, {"DW_NO_TRIM": "1"})):
+    os.environ.pop("DW_NO_TRIM", None)
     os.environ.update(envs)
     best = None
     for rep in range(3):
@@ -21,7 +20,7 @@ for label, envs in (("auto (trimmed)", {}), ("segment 64 trimmed", {"DW_SEGMENT"
         env.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        r = simulate_lifespan(DeviceShard(env), policy="greedy", seed=7, device="cuda")
+        r = simulate_lifespan(DeviceShard(env), policy="greedy", seed=7, device="cuda", segment=segment)
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
