@@ -83,10 +83,23 @@ int dwt_get_ptrs(dwt_handle *h, dwt_ptrs *out);
 int dwt_run(dwt_handle *h, int64_t K, int32_t policy, const int8_t *actions /*[K,n] or NULL*/, uint64_t seed);
 /* Close a chunk of `K` steps whose per-step maxima sit in stepmax (all-reduced MAX over ranks by the caller when there
    are several): done_at += #steps whose max(light, dark) > 5 (notebook cell 2: grid_done = max <= 0.005);
-   first_all_done = first step index of the chunk with the world done, or -1. Clears stepmax. */
+   first_all_done = first step index of the chunk with the world done, or -1. Clears stepmax and the series rows. */
 int dwt_end_chunk(dwt_handle *h, int32_t K, int32_t *first_all_done);
 int dwt_reset_lifespans(dwt_handle *h);
 int dwt_get_lifespans(dwt_handle *h, int64_t *done_at /*[1]*/, int64_t *agents_done_at /*[n]*/);
+
+/* ---- climate series: per-step sums over the band's own cells, reduced inside the stencil kernels -----------------------
+ * With series mode on, step j of a chunk adds to row j of a device buffer [4096, 3] (doubles):
+ *   column 0: sum of sqrt(g) * T, T the unrounded global temperature of the step's forward (the reference's env.temp);
+ *   columns 1, 2: sum of the new light / dark milli-covers (1000 * cover; integers, exact and order-independent in fp64).
+ * Ghost rows and columns never count, so the rows are additive over the bands of a world: a multi-rank caller all-reduces
+ * (SUM) the K rows of dwt_get_series_ptr before dwt_get_series. dwt_end_chunk, dwt_upload_covers and dwt_init_random clear
+ * the rows. Switching series mode while a chunk is open fails with DW_E_STATE; it needs g > 0 (DW_E_UNSUPPORTED). */
+int dwt_set_series(dwt_handle *h, int32_t on);
+int dwt_get_series_ptr(dwt_handle *h, double **series /* device [4096, 3] */);
+/* [K, 3] host: sum of T (kelvin), sum of milli-light, sum of milli-dark of the chunk's first K steps; call before
+   dwt_end_chunk. Synchronises. */
+int dwt_get_series(dwt_handle *h, int32_t K, double *out);
 
 /* ---- peer-memory mode: one process per GPU, no collective on the step path -----------------------------------------
  * Every rank maps every other rank's exchange vector, barrier flags and lattice buffers (CUDA IPC over NVLink/NVSwitch).
@@ -120,7 +133,8 @@ int dwt_cover_checksum(dwt_handle *h, uint64_t *out /*[4]*/);
 int dwt_debug_slow_count(dwt_handle *h, uint64_t *count);
 /* Measurement hook: average duration (microseconds, CUDA events) of `reps` back-to-back launches of the band's stencil
    kernel on the current state -- the compute floor of one step, against which bench.py states the per-step exchange /
-   agent overhead. Overwrites the recorded pre-state (dwt_get_grid needs a new step afterwards). */
+   agent overhead. Overwrites the recorded pre-state (dwt_get_grid needs a new step afterwards). Always times the kernel
+   with series mode off and records nothing into the series rows. */
 int dwt_debug_time_stencil(dwt_handle *h, int32_t reps, double *us_per_launch);
 
 #ifdef __cplusplus

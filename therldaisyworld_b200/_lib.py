@@ -51,7 +51,7 @@ TILED_SYMBOLS = [
     "dwt_finish_agents", "dwt_stencil", "dwt_halo_wrap", "dwt_get_ptrs", "dwt_run", "dwt_end_chunk",
     "dwt_reset_lifespans", "dwt_get_lifespans", "dwt_get_agents", "dwt_get_reward_done", "dwt_get_covers", "dwt_get_grid",
     "dwt_debug_slow_count", "dwt_debug_time_stencil", "dwt_cover_checksum", "dwt_ipc_export", "dwt_ipc_attach", "dwt_get_peer_buffers", "dwt_attach_peers", "dwt_step_p2p",
-    "dwt_flush_p2p", "dwt_peer_status",
+    "dwt_flush_p2p", "dwt_peer_status", "dwt_set_series", "dwt_get_series_ptr", "dwt_get_series",
 ]
 
 
@@ -184,6 +184,9 @@ def load():
         "dwt_step_p2p": (C.c_int, [vp, i32, pi8, u64]),
         "dwt_flush_p2p": (C.c_int, [vp]),
         "dwt_peer_status": (C.c_int, [vp, pi32]),
+        "dwt_set_series": (C.c_int, [vp, i32]),
+        "dwt_get_series_ptr": (C.c_int, [vp, C.POINTER(vp)]),
+        "dwt_get_series": (C.c_int, [vp, i32, pd]),
     }
     assert set(tsig) == set(TILED_SYMBOLS)
     sig.update(tsig)

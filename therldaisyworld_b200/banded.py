@@ -12,7 +12,8 @@ NCCL over NVLink on GPUs, gloo in the CPU tests -- plumbing only, the data path 
     clip, reward/done) is deferred until the decisions of step j exist, so both vectors travel together;
   * after the edge tile rows of the stencil: the band's first/last row goes to the upper/lower neighbour's ghost row
     (ring, toroidal) on a side stream while the interior tile rows are still being computed;
-  * per chunk of steps: MAX all-reduce of the per-step cover maxima (lifespan bookkeeping, ``grid_done``).
+  * per chunk of steps: MAX all-reduce of the per-step cover maxima (lifespan bookkeeping, ``grid_done``), and in
+    ``run_series`` a SUM all-reduce of the per-step temperature and cover sums next to it.
 
 ``world_size == 1`` needs none of them (``dwt_halo_wrap`` closes the torus locally).
 
@@ -231,6 +232,17 @@ class DeviceBand:
         self._check(self._lib.dwt_run(self._h, int(K), DW_POLICY[policy], None if a is None else a.ctypes.data_as(C.POINTER(C.c_int8)),
                                       C.c_uint64(seed)), "dwt_run")
 
+    def set_series(self, on):
+        """Series mode: every step also sums sqrt(g)*T and the new milli-covers of the band's cells (dwt_set_series)."""
+        self._check(self._lib.dwt_set_series(self._h, 1 if on else 0), "dwt_set_series")
+
+    def take_series(self, K):
+        """[K, 3] of the open chunk: sum of T (kelvin), sum of milli-light, sum of milli-dark (after any all-reduce of
+        series_tensor)."""
+        out = np.zeros((int(K), 3))
+        self._check(self._lib.dwt_get_series(self._h, int(K), out.ctypes.data_as(C.POINTER(C.c_double))), "dwt_get_series")
+        return out
+
     def end_chunk(self, K):
         first = C.c_int32(-1)
         self._check(self._lib.dwt_end_chunk(self._h, int(K), C.byref(first)), "dwt_end_chunk")
@@ -257,6 +269,12 @@ class DeviceBand:
 
     def stepmax_tensor(self, K):
         return self._view(self._ptrs().stepmax, (4096 * 2,), "<i4")[:2 * K]
+
+    def series_tensor(self, K):
+        """The first K rows of the device series buffer [4096, 3] (partial sums of this band, additive over bands)."""
+        p = C.c_void_p()
+        self._check(self._lib.dwt_get_series_ptr(self._h, C.byref(p)), "dwt_get_series_ptr")
+        return self._view(p.value, (4096, 3), "<f8")[:K]
 
     def halo_tensors(self):
         """(send_top, send_bottom, recv_top, recv_bottom): whole stored rows (N + 8 words, ghost columns included) of the
@@ -334,6 +352,7 @@ class BandedDaisyWorld:
         self._pending = 0          # steps recorded since the last end_chunk
         self._gain_pending = False # multi-rank: gains of the last step not yet summed / applied
         self.first_done_step = None
+        self._series = None        # run_series: [k, 3] sums of the chunks closed so far
         self.mode = mode if self.world_size > 1 else "local"
         if self.mode == "p2p" and comm is None:
             # one-off exchange of the CUDA IPC handles (any transport would do; torch.distributed is at hand)
@@ -422,6 +441,10 @@ class BandedDaisyWorld:
             return
         if self.comm is not None:
             self.comm.all_reduce_max(self.band.stepmax_tensor(K))
+        if self._series is not None:
+            if self.comm is not None:
+                self.comm.all_reduce_sum(self.band.series_tensor(K))
+            self._series.append(self.band.take_series(K))
         first = self.band.end_chunk(K)
         self._check_peers()
         if first >= 0 and self.first_done_step is None:
@@ -448,6 +471,24 @@ class BandedDaisyWorld:
                 self.end_chunk()
         self.end_chunk()
         return K
+
+    def run_series(self, K, policy="greedy", actions=None, seed=0, chunk=256):
+        """run() that also returns the per-step means of the whole world [K, 3] = (global mean temperature of that step's
+        forward -- env.temp.mean() of the reference --, mean light cover, mean dark cover after the step), the layout of
+        RLDaisyWorld.run_series. Reduced inside the stencil kernels (series mode) and summed over the ranks once per chunk;
+        every rank returns the same array. Needs g > 0."""
+        self.end_chunk()
+        self.band.set_series(True)
+        self._series = []
+        try:
+            self.run(K, policy, actions=actions, seed=seed, chunk=chunk)
+            sums = np.concatenate(self._series) if self._series else np.zeros((0, 3))
+        finally:
+            self._series = None
+            if self._pending == 0:
+                self.band.set_series(False)
+        cells = float(self.dim) * self.dim
+        return sums / np.array([cells, 1000.0 * cells, 1000.0 * cells])
 
     # ---- results
     def lifespans(self):

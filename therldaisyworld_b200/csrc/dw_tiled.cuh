@@ -381,11 +381,14 @@ __global__ void __launch_bounds__(256) k_band_ghost_rows_wrap(BandGeom G, uint32
 }
 
 // ---- first step: literal forward from the off-lattice fp64 cover planes [(R+2) x N] onto the padded lattice ---------
+// SERIES: also adds {sum sqrt(g)*T, sum milli-light, sum milli-dark} of the band's cells to series[0..2] (see k_tiled_step)
+template <bool SERIES = false>
 __global__ void __launch_bounds__(256) k_band_first_step(DevParams P, double SL, BandGeom Gp, const double *__restrict__ l,
                                                          const double *__restrict__ d, BandGeom Gl, uint32_t *__restrict__ lat_out,
-                                                         int *stepmax) {
+                                                         int *stepmax, double sqrt_g = 0.0, double *series = nullptr) {
     const size_t total = (size_t)Gp.R * Gp.N;
     uint32_t mx = 0;
+    double ser[3] = {0.0, 0.0, 0.0};     // series mode; the cover sums are integers below 2^53, so exact in fp64
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const int r = (int)(i / Gp.N), y = (int)(i - (size_t)r * Gp.N);
         const int ys[3] = {y == 0 ? Gp.N - 1 : y - 1, y, y == Gp.N - 1 ? 0 : y + 1};
@@ -405,9 +408,22 @@ __global__ void __launch_bounds__(256) k_band_first_step(DevParams P, double SL,
         if (y == 0) orow[Gl.c0 + Gl.N] = q;              // ghost columns of the produced row
         if (y == Gl.N - 1) orow[Gl.c0 - 1] = q;
         mx = __vmaxu2(mx, q);
+        if (SERIES) {
+            ser[0] += sqrt_g * o.T;
+            ser[1] += (double)(q & 0xffffu);
+            ser[2] += (double)(q >> 16);
+        }
     }
     const unsigned ml = __reduce_max_sync(0xffffffffu, mx & 0xffffu), md = __reduce_max_sync(0xffffffffu, mx >> 16);
     if ((threadIdx.x & 31) == 0) { atomicMax(stepmax, (int)ml); atomicMax(stepmax + 1, (int)md); }
+    if (SERIES) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            double v = ser[c];
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+            if ((threadIdx.x & 31) == 0) atomicAdd(series + c, v);
+        }
+    }
 }
 
 // ---- steady state: one stencil step of the band, 64x64 tiles, TMA-staged halo tile ---------------------------------
@@ -446,10 +462,25 @@ struct StoreGlobal {
         *reinterpret_cast<uint4 *>(o + (size_t)i * pitch) = make_uint4(q[0], q[1], q[2], q[3]);
     }
 };
+// series mode: StoreGlobal that also sums the packed cells it stores. Each half of a packed cell is at most 1000, so the
+// 16 cells of a thread's 4x4 tile sum to at most 16000 per half and the halves cannot carry into each other.
+struct StoreGlobalSum {
+    static constexpr bool kMasks = false;
+    uint32_t *o;
+    int pitch;
+    uint32_t *sum;
+    __device__ __forceinline__ void operator()(int i, uint32_t (&q)[4]) const {
+        *reinterpret_cast<uint4 *>(o + (size_t)i * pitch) = make_uint4(q[0], q[1], q[2], q[3]);
+        *sum += (q[0] + q[1]) + (q[2] + q[3]);
+    }
+};
 
 // rare path, warp-cooperative: for every lane whose 4x4 tile hit the tie filter, lanes 0..15 re-evaluate one cell of that
 // tile each from the staged tile; cells on a rounding tie are recomputed in literal order and patched in the output.
 // tile_off / out_off: each lane's offsets of its first cell inside the staged tile / the output lattice.
+// One copy per k_tiled_step instantiation (SERIES is otherwise unused): with a single caller the compiler propagates the
+// address of that kernel's shared tile into it, which the default kernel's code and shared-memory layout depend on.
+template <bool SERIES>
 __device__ __noinline__ uint32_t dwt_fix_warp(const TiledArgs *A, const uint32_t *tile, unsigned flagged, uint32_t mx, int tile_off,
                                               long long out_off, int lane) {
     uint32_t extra = 0;
@@ -503,8 +534,12 @@ __device__ __forceinline__ void dwt_issue_tile(const CUtensorMap *tmap, const Ti
 
 // One tile per CTA (gridDim.x = number of tiles, 19 KB of shared memory). A grid of fewer CTAs also works: a CTA then walks
 // the tiles blockIdx.x, blockIdx.x + gridDim.x, ... and loads the next one once the current one is computed.
+// SERIES: the step also adds the sums of its produced cells to series[0..2], one atomicAdd per column and CTA:
+// {sqrt(g)*T of the forward (unrounded, from the staged pre-state), new milli-light, new milli-dark}. `series` is the last
+// parameter (not a member of TiledArgs), so that every parameter offset of the default kernel stays where it was.
+template <bool SERIES = false>
 __global__ void __launch_bounds__(256, 4) k_tiled_step(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ TiledArgs A,
-                                                       int n_tiles) {
+                                                       int n_tiles, double *series = nullptr) {
     constexpr int kTileWords = ((DWT_TILE_BYTES + 127) / 128) * 32;       // a TMA destination must be 128-byte aligned: 19008 -> 19072 B
     __shared__ __align__(128) uint32_t tile[kTileWords];
     __shared__ __align__(8) unsigned long long bar;
@@ -522,6 +557,8 @@ __global__ void __launch_bounds__(256, 4) k_tiled_step(const __grid_constant__ C
     __syncthreads();                                     // barrier initialised (and armed) before anyone polls
     const int tile_off = (1 + r0) * DWT_TILE_PITCH + 4 + 4 * tx;
     uint32_t mx_all = 0;
+    double tsum = 0.0;                                   // series mode: sqrt(g)*T, light and dark milli-covers of the thread's cells
+    uint32_t cl = 0, cd = 0;
     for (int k = 0; t < n_tiles; ++k, t += gridDim.x) {
         {
             const uint32_t parity = (uint32_t)k & 1u;
@@ -535,9 +572,28 @@ __global__ void __launch_bounds__(256, 4) k_tiled_step(const __grid_constant__ C
         if (tr >= A.tr_skip_lo) tr += A.tr_skip_hi - A.tr_skip_lo;
         const long long out_off = (long long)(tr * DWT_TILE + 1 + r0) * A.pitch + 4 + tc * DWT_TILE + 4 * tx;
         unsigned tiemin = 0xffffffffu;
-        uint32_t mx = dw_tile_core(A.F, A.C, RowsTile72{tile + tile_off}, StoreGlobal{A.out + out_off, A.pitch}, &tiemin);
+        uint32_t mx, cov = 0;
+        if constexpr (SERIES)
+            mx = dw_tile_core<RowsTile72, StoreGlobalSum, true>(A.F, A.C, RowsTile72{tile + tile_off}, StoreGlobalSum{A.out + out_off, A.pitch, &cov},
+                                                                &tiemin, &tsum);
+        else
+            mx = dw_tile_core(A.F, A.C, RowsTile72{tile + tile_off}, StoreGlobal{A.out + out_off, A.pitch}, &tiemin);
         const unsigned flagged = __ballot_sync(0xffffffffu, tiemin < A.F.tie_thresh);
-        if (flagged) mx = dwt_fix_warp(&A, tile, flagged, mx, tile_off, out_off, lane);
+        if (flagged) {
+            mx = dwt_fix_warp<SERIES>(&A, tile, flagged, mx, tile_off, out_off, lane);
+            if constexpr (SERIES) {
+                if ((flagged >> lane) & 1u) {            // literal fix-ups were patched into this lane's cells: sum them again
+                    const uint32_t *o = A.out + out_off;
+                    cov = 0;
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) {
+                        const uint4 v = *reinterpret_cast<const uint4 *>(o + (size_t)i * A.pitch);
+                        cov += (v.x + v.y) + (v.z + v.w);
+                    }
+                }
+            }
+        }
+        if constexpr (SERIES) { cl += cov & 0xffffu; cd += cov >> 16; }
         // ghost columns of the produced rows: the two threads of a row group that hold column 0 / N-1 copy their (final) cells
         if (tx == 0 && tc == 0) {
             uint32_t *o = A.out + out_off;
@@ -554,6 +610,21 @@ __global__ void __launch_bounds__(256, 4) k_tiled_step(const __grid_constant__ C
     }
     const unsigned ml = __reduce_max_sync(0xffffffffu, mx_all & 0xffffu), md = __reduce_max_sync(0xffffffffu, mx_all >> 16);
     if (lane == 0) { atomicMax(&smax[0], (int)ml); atomicMax(&smax[1], (int)md); }
+    if constexpr (SERIES) {
+        // per warp, then per CTA (fixed order), then one global add per column: 3 same-address atomics per CTA and step
+        __shared__ double s_ser[256 / 32][3];
+        for (int o = 16; o > 0; o >>= 1) tsum += __shfl_xor_sync(0xffffffffu, tsum, o);
+        cl = __reduce_add_sync(0xffffffffu, cl);
+        cd = __reduce_add_sync(0xffffffffu, cd);
+        if (lane == 0) { s_ser[tid >> 5][0] = tsum; s_ser[tid >> 5][1] = (double)cl; s_ser[tid >> 5][2] = (double)cd; }
+        __syncthreads();
+        if (tid < 3) {
+            double v = 0.0;
+#pragma unroll
+            for (int w = 0; w < 256 / 32; ++w) v += s_ser[w][tid];
+            atomicAdd(series + tid, v);
+        }
+    }
     __syncthreads();
     if (tid == 0) {
         if (smax[0] > 0) atomicMax(A.stepmax, smax[0]);
