@@ -70,7 +70,9 @@ typedef struct dw_config {
     int32_t device;       /* CUDA device ordinal */
     double p, g, S, sigma, gamma, q, q2, temp_optimal, dt, agent_gamma;
     double albedo_bare, albedo_light, albedo_dark;
-    double daisy_kernel[9];     /* env.daisy_kernel, row-major 3x3 (daisy_world_rl.py:270-273) */
+    /* Both kernels are given as the env holds them, row-major 3x3. The step convolves with them like ft_convolve
+       (daisy/nn/functional.py:12-49): out[i][j] = sum over a, b of k[a][b] * x[i+1-a][j+1-b], toroidal. */
+    double daisy_kernel[9];     /* env.daisy_kernel (daisy_world_rl.py:270-273) */
     double adjacent_kernel[9];  /* env.adjacent_albedo_kernel (daisy_world_rl.py:278-281) */
     double obs_mask[9];         /* env.neighborhood for kr=1 (daisy/nn/functional.py:93-103) */
 } dw_config;
@@ -253,7 +255,8 @@ int dw_trim_lifespans(dw_handle *h, int32_t j);
 int dw_run_chunk(dw_handle *h, int32_t K, int32_t policy, const int8_t *actions, uint64_t seed, uint64_t *done_mask);
 /* dw_run that also returns, for every step, the ensemble means the reference's plot helpers read (notebook_helpers.py:
    45-57): out[K][3] = {global mean of the unrounded temperature of that step's forward (env.temp.mean()), mean light cover,
-   mean dark cover after the step}, reduced inside the fused kernel. 64x64 worlds, n_agents <= 32, K <= 4096. */
+   mean dark cover after the step}, reduced inside the fused kernel. K <= 4096. Shapes and configurations without an
+   in-kernel series (see dw_run_series in csrc/dw_run.inl) fail with DW_E_UNSUPPORTED before any step has run. */
 int dw_run_series(dw_handle *h, int64_t K, int32_t policy, const int8_t *actions, uint64_t seed, double *out);
 int dw_reset_lifespans(dw_handle *h);
 int dw_get_lifespans(dw_handle *h, int64_t *done_at /*[B]*/, int64_t *agents_done_at /*[B,n]*/);

@@ -54,6 +54,8 @@ const char *dwt_last_error(const dwt_handle *h);
 /* cfg->dim = N, cfg->n_agents = n, cfg->batch must be 1; rows/row0: the band of this handle; n_ranks: number of bands */
 int dwt_create(const dw_config *cfg, int32_t rows, int32_t row0, int32_t n_ranks, dwt_handle **out);
 int dwt_destroy(dwt_handle *h);
+/* New constants for the handle. Refuses with DW_E_UNSUPPORTED what dwt_create refuses (the tiled kernels need D4-symmetric
+   kernels, a zero-centre uniform albedo kernel and g > 0) and keeps the old configuration then. */
 int dwt_set_config(dwt_handle *h, const dw_config *cfg);
 int dwt_set_clock(dwt_handle *h, const dw_clock *clk);
 int dwt_get_clock(dwt_handle *h, dw_clock *clk);

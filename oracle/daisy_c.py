@@ -15,7 +15,7 @@ class Params(C.Structure):
     _fields_ = [("B", C.c_int32), ("N", C.c_int32), ("n_agents", C.c_int32), ("ch", C.c_int32)] + \
                [(k, C.c_double) for k in ("p", "g", "S", "sigma", "gamma", "q", "q2", "temp_optimal", "dt",
                                           "agent_gamma", "albedo_bare", "albedo_light", "albedo_dark")] + \
-               [("mask", C.c_double * 9), ("w", C.c_double * 9)]
+               [("mask", C.c_double * 9), ("w", C.c_double * 9), ("adj", C.c_double * 9)]
 
 
 class Clock(C.Structure):
@@ -58,8 +58,13 @@ class COracleWorld:
                         albedo_bare=env.albedo_bare, albedo_light=env.albedo_light, albedo_dark=env.albedo_dark)
         mask = getattr(env, "neighborhood", neighborhood_mask(1, "von_neumann"))
         w = getattr(env, "daisy_kernel", daisy_weights())
+        adj = getattr(env, "adjacent_albedo_kernel", None)
+        if adj is None:
+            adj = np.full((3, 3), 0.125)
+            adj[1, 1] = 0.0
         self.P.mask[:] = list(np.asarray(mask, dtype=np.float64).ravel())
         self.P.w[:] = list(np.asarray(w, dtype=np.float64).ravel())
+        self.P.adj[:] = list(np.asarray(adj, dtype=np.float64).ravel())
         self.clk = Clock(L=env.L, dL=env.dL, min_L=env.min_L, max_L=env.max_L, ddL=env.ddL,
                          step_count=env.step_count, ramp_period=env.ramp_period,
                          ramp_up_down=int(bool(env.ramp_up_down)))

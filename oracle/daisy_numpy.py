@@ -14,18 +14,22 @@ against trajectories recorded from the live, unmodified reference by
 
 Two convolution modes:
   * ``conv="stencil"`` (default): the 3x3 toroidal stencil that the reference's FFT
-    convolution (``daisy/nn/functional.py:12-49``) is mathematically equal to.  The tap order
-    below is the *canonical arithmetic order* that ``oracle/daisy_oracle.c`` and the CUDA
-    materialising kernel reproduce operation for operation.
+    convolution (``daisy/nn/functional.py:12-49``) is mathematically equal to.  ``ft_convolve``
+    multiplies the two spectra, so it is a true circular convolution, not a correlation:
+    out[i,j] = sum w[a,b]*x[i+1-a, j+1-b].  The tap order below is the *canonical arithmetic
+    order* that ``oracle/daisy_oracle.c`` and the CUDA materialising kernel reproduce operation
+    for operation.
   * ``conv="fft"``: circular convolution through ``np.fft`` like the reference, used only as
     the CPU *baseline* (same cost profile as the reference's NumPy path).
 
 Canonical arithmetic order (IEEE binary64, no FMA contraction), per cell:
   b   = (p - l) - d                                            # daisy_world_rl.py:381
   Al  = ((ab*b) + al*l) + ad*d                                 # :388-390
-  nb8(x) = 0.125*x[-1,-1] + 0.125*x[-1,0] + ... row-major, centre skipped, left-to-right
-  A   = ((ab*nb8(b)) + al*nb8(l)) + ad*nb8(d)                  # :391
-  rho(x) = sum over the 9 taps, row-major, of w_tap*x_tap, left-to-right   # :423-432, :270-273
+  conv(x, w) = sum over the neighbour offsets (di, dj), row-major from (-1,-1) to (+1,+1), of
+               w[1-di, 1-dj]*x[i+di, j+dj], left to right; the centre term is skipped only when
+               its tap is exactly 0.0 (the default adjacent-albedo kernel)
+  A   = ((ab*conv(b, adj)) + al*conv(l, adj)) + ad*conv(d, adj)   # :391, :278-281
+  rho(x) = conv(x, daisy_kernel)                               # :423-432, :270-273
   Te  = root4(((S*L)*(1-A))/sigma)                             # :403-404
   T   = root4(q*(A-Al) + pow4(Te))                             # :409
   Tl  = root4(q2*(Al-al) + pow4(T));  Td likewise with ad      # :411-412
@@ -78,13 +82,15 @@ def _shift(x, di, dj):
 
 
 def stencil9(x, w):
-    """sum_taps w[a,b]*x[i+a-1, j+b-1], taps row-major, accumulated left to right."""
+    """Circular convolution like ft_convolve: sum over the offsets (di, dj), row-major, of w[1-di, 1-dj]*x[i+di, j+dj],
+    accumulated left to right; a centre tap of exactly 0.0 is skipped."""
     acc = None
-    for a in range(3):
-        for b in range(3):
-            if w[a, b] == 0.0 and (a, b) == (1, 1):
-                continue  # the adjacent-albedo kernel skips its zero centre tap
-            term = w[a, b] * _shift(x, a - 1, b - 1)
+    for di in (-1, 0, 1):
+        for dj in (-1, 0, 1):
+            tap = w[1 - di, 1 - dj]
+            if tap == 0.0 and (di, dj) == (0, 0):
+                continue  # the default adjacent-albedo kernel skips its zero centre tap
+            term = tap * _shift(x, di, dj)
             acc = term if acc is None else acc + term
     return acc
 
@@ -131,8 +137,8 @@ class OracleDaisyWorld:
         self.initial_L = self.min_L
         self.neighborhood = neighborhood_mask(self.kr, self.neighborhood_mode)
         self.daisy_kernel = daisy_weights()
-        self.adjacent_kernel = np.full((3, 3), 0.125)
-        self.adjacent_kernel[1, 1] = 0.0
+        self.adjacent_albedo_kernel = np.full((3, 3), 0.125)    # the reference's attribute name (:278-281)
+        self.adjacent_albedo_kernel[1, 1] = 0.0
         self.init_agents()
         self.reset()
 
@@ -169,6 +175,7 @@ class OracleDaisyWorld:
 
     # ---- physics (reference :340-432) -----------------------------------------------
     def _conv(self, x, w):
+        w = np.asarray(w, dtype=np.float64).reshape(3, 3)    # (3, 3) or the reference's (1, 1, 3, 3)
         return stencil9(x, w) if self.conv == "stencil" else fft_circular(x, w)
 
     def fields(self, l, d):
@@ -176,8 +183,8 @@ class OracleDaisyWorld:
         ab, al, ad = self.albedo_bare, self.albedo_light, self.albedo_dark
         b = self.p - l - d
         Al = ab * b + al * l + ad * d
-        A = ab * self._conv(b, self.adjacent_kernel) + al * self._conv(l, self.adjacent_kernel) \
-            + ad * self._conv(d, self.adjacent_kernel)
+        adj = self.adjacent_albedo_kernel
+        A = ab * self._conv(b, adj) + al * self._conv(l, adj) + ad * self._conv(d, adj)
         rho_l = self._conv(l, self.daisy_kernel)
         rho_d = self._conv(d, self.daisy_kernel)
         SL = self.S * self.L

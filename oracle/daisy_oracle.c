@@ -28,6 +28,7 @@ typedef struct {
     double mask[9];                        /* observation neighbourhood, row-major 3x3 */
     double w[9];                           /* daisy-spread kernel (reference :270-273), computed by the
                                               caller with NumPy exactly as the reference does */
+    double adj[9];                         /* adjacent-albedo kernel (reference :278-281), row-major 3x3 */
 } dwo_params;
 
 static inline double root4(double x) { return sqrt(sqrt(x)); }
@@ -40,7 +41,8 @@ void dwo_forward(const dwo_params *P, double L, double *grid, const int64_t *age
                  const double *agent_state, double *out, double *diag) {
     const int N = P->N, B = P->B;
     const size_t NN = (size_t)N * N;
-    const double *w = P->w;
+    const double *w = P->w, *adj = P->adj;
+    const int skip_centre = adj[4] == 0.0;   /* the default adjacent kernel: its zero centre term is not added */
     const double ab = P->albedo_bare, al = P->albedo_light, ad = P->albedo_dark;
     const double SL = P->S * L;
 #pragma omp parallel for schedule(static)
@@ -56,14 +58,17 @@ void dwo_forward(const dwo_params *P, double L, double *grid, const int64_t *age
                 size_t c = (size_t)x * N + y;
                 double nb_b = 0, nb_l = 0, nb_d = 0, rho_l = 0, rho_d = 0;
                 int first = 1, first9 = 1;
+                /* circular convolution like ft_convolve (daisy/nn/functional.py:12-49): the neighbour at offset
+                   (a-1, b-1), visited row-major, is weighted by the tap turned 180 degrees, w[2-a][2-b] */
                 for (int a = 0; a < 3; ++a)
                     for (int b = 0; b < 3; ++b) {
                         size_t k = (size_t)xs[a] * N + ys[b];
-                        double tl = w[a * 3 + b] * lt[k], td = w[a * 3 + b] * dk[k];
+                        const int t = 8 - (a * 3 + b);
+                        double tl = w[t] * lt[k], td = w[t] * dk[k];
                         if (first9) { rho_l = tl; rho_d = td; first9 = 0; }
                         else { rho_l = rho_l + tl; rho_d = rho_d + td; }
-                        if (a == 1 && b == 1) continue;
-                        double vb = 0.125 * bare[k], vl = 0.125 * lt[k], vd = 0.125 * dk[k];
+                        if (a == 1 && b == 1 && skip_centre) continue;
+                        double vb = adj[t] * bare[k], vl = adj[t] * lt[k], vd = adj[t] * dk[k];
                         if (first) { nb_b = vb; nb_l = vl; nb_d = vd; first = 0; }
                         else { nb_b = nb_b + vb; nb_l = nb_l + vl; nb_d = nb_d + vd; }
                     }

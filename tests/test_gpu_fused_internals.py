@@ -84,21 +84,6 @@ def test_fused_equals_materialising_path(N, B, n, policy):
     assert a[8] < 1e-3 * cells + 10
 
 
-def test_unsupported_kernels_use_materialising_path():
-    """An asymmetric daisy kernel is outside the fused fast path; dw_run must still be right (vs single steps)."""
-    env = _env(8, 2, 2, seed=3)
-    k = env.daisy_kernel.copy()
-    k[0, 0, 0, 1] *= 1.5
-    env.daisy_kernel = k / k.sum()
-    env2 = _env(8, 2, 2, seed=3)
-    env2.daisy_kernel = env.daisy_kernel.copy()
-    env.run(20, policy="greedy")
-    for _ in range(20):
-        env2.step_policy("greedy")
-    np.testing.assert_array_equal(env.grid, env2.grid)
-    np.testing.assert_array_equal(env.agent_states, env2.agent_states)
-
-
 def test_division_free_rounding_is_exact_on_device():
     env = _env()
     bad = C.c_uint32(123)

@@ -123,7 +123,10 @@ def test_banded_series_equals_single_band(bands, mode):
     np.testing.assert_array_equal(np.concatenate([out[r][1] for r in range(bands)], axis=1), one.local_covers())
 
 
-def test_refused_series_configurations():
+def test_refused_series_configurations_and_zero_g_at_reset():
+    """Series mode cannot be switched inside an open chunk and has nothing to read while off. g = 0 never reaches the
+    handle: the temperature is summed as sqrt(g) * T and the tiled kernels scale by g^2, so dwt_set_config refuses it at
+    reset (like dwt_create) and keeps the old constants, with which the world still runs its series."""
     from therldaisyworld_b200 import DaisyWorldError
     N, n = 64, 4
     light, dark, ai, st = make_state(N, n, seed=3)
@@ -135,7 +138,11 @@ def test_refused_series_configurations():
     with pytest.raises(DaisyWorldError, match="dwt_get_series"):    # series mode is off: nothing to read
         w.band.take_series(1)
     w.end_chunk()
-    w.g = 0.0                                            # the temperature is summed as sqrt(g) * T: g = 0 is refused
+    g = w.g
+    w.g = 0.0
+    with pytest.raises(DaisyWorldError, match="dwt_set_config.*g > 0"):
+        w.load_state(light, dark, ai, st)
+    w.g = g
     w.load_state(light, dark, ai, st)
-    with pytest.raises(DaisyWorldError, match="g > 0"):
-        w.run_series(4, "greedy")
+    s = w.run_series(4, "greedy")
+    assert s.shape == (4, 3) and np.isfinite(s).all() and (s[:, 0] > 200).all()

@@ -1,4 +1,5 @@
 """C oracle == NumPy oracle == reference-recorded fixtures (all value-identical in fp64)."""
+import itertools
 import json
 import os
 
@@ -6,6 +7,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN_DIR, golden_names
+from kernel_sets import DRAWS, KERNEL_SETS, apply_draw, set_kernels
 from oracle.daisy_c import COracleWorld
 from oracle.daisy_numpy import OracleDaisyWorld, OracleGreedy, env_from_golden, lifespan_loop
 
@@ -54,12 +56,19 @@ def test_c_oracle_lifespan_run(name, policy):
 
 
 def test_c_oracle_matches_numpy_oracle_random_states():
-    """Arbitrary (off-lattice) states, odd N, many agents: bit-identical to the NumPy oracle."""
+    """Arbitrary (off-lattice) states, odd N, many agents, degenerate 1x1 and 2x2 tori, every kernel set and constant
+    draw of tests/kernel_sets.py: bit-identical to the NumPy oracle."""
+    names = list(KERNEL_SETS)
+    cases = [(name, None) for name in names] + [(names[(i + 1) % len(names)], d) for i, d in enumerate(DRAWS)]
     rng = np.random.RandomState(123)
-    for N, B, n in [(3, 2, 1), (4, 2, 3), (6, 3, 2), (9, 2, 5), (33, 2, 7)]:
+    for (N, B, n), (kernels, draw) in itertools.product([(1, 2, 1), (2, 2, 1), (3, 2, 1), (4, 2, 3), (6, 3, 2), (9, 2, 5), (33, 2, 7)],
+                                                        cases):
         np.random.seed(N)
         env = OracleDaisyWorld(grid_dimension=N, n_agents=n)
         env.batch_size = B
+        if draw is not None:
+            apply_draw(env, draw)
+        set_kernels(env, kernels)
         env.reset()
         env.grid[:, 1] = rng.rand(B, N, N) * 0.6
         env.grid[:, 2] = rng.rand(B, N, N) * 0.4

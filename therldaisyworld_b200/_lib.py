@@ -7,6 +7,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DW_LIB", os.path.join(PKG, "libdaisyworld_b200.so"))   # DW_LIB: another build, e.g. to compare two
 
 DW_POLICY = {"none": 0, "greedy": 1, "antigreedy": 2, "replay": 3, "random": 4, "eps_greedy": 5, "mlp": 6}
+DW_E_UNSUPPORTED = -3       # include/daisyworld_b200.h: configuration outside what the kernels implement
 DW_DIAG = {"temp": 0, "temp_light": 1, "temp_dark": 2, "temp_effective": 3, "beta": 4, "beta_l": 5, "beta_d": 6,
            "growth": 7}
 

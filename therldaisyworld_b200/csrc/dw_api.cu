@@ -149,7 +149,8 @@ static DevParams make_params_cfg(const dw_config &c) {
     P.p = c.p; P.g = c.g; P.S = c.S; P.sigma = c.sigma; P.gamma = c.gamma; P.q = c.q; P.q2 = c.q2;
     P.temp_optimal = c.temp_optimal; P.dt = c.dt; P.agent_gamma = c.agent_gamma;
     P.ab = c.albedo_bare; P.al = c.albedo_light; P.ad = c.albedo_dark;
-    for (int i = 0; i < 9; ++i) { P.w[i] = c.daisy_kernel[i]; P.adj[i] = c.adjacent_kernel[i]; P.mask[i] = c.obs_mask[i]; }
+    // ft_convolve is a convolution, not a correlation: the neighbour at row-major position i takes the tap turned 180 degrees
+    for (int i = 0; i < 9; ++i) { P.w[i] = c.daisy_kernel[8 - i]; P.adj[i] = c.adjacent_kernel[8 - i]; P.mask[i] = c.obs_mask[i]; }
     // Screened forward (dw_screened_cell): the fast evaluation differs from the literal one by the fast fourth root
     // (3e-12 relative, asserted in the tests) plus a few ulp. With T <= 400 K and |Topt - T| <= max(|Topt - 150|, |Topt - 400|)
     // (the kernel checks the range) and densities in [0, 1]: |d(1000 l')| <= 1000 dt 2 g |Topt - T| T 3e-12, b' twice that,

@@ -16,8 +16,8 @@ struct DevParams {
     int B, N, n_agents, pad_;
     double p, g, S, sigma, gamma, q, q2, temp_optimal, dt, agent_gamma;
     double ab, al, ad;
-    double w[9];      // daisy-spread taps, row-major
-    double adj[9];    // adjacent-albedo taps, row-major (centre tap skipped when it is 0, see nb_sum)
+    double w[9];      // daisy-spread taps by neighbour, row-major (the env's kernel turned 180 degrees, make_params_cfg)
+    double adj[9];    // adjacent-albedo taps by neighbour, likewise (centre tap skipped when it is 0, see dw_literal_cell)
     double mask[9];   // observation mask
     // screened forward (dw_screened_cell): sum of the adjacent-albedo taps, tie-filter half-widths (in units of 0.001) of
     // the covers, the bare fraction and the temperatures, accepted range of T^4; screen = 0 forces the literal path

@@ -23,7 +23,7 @@ import numpy as np
 import numpy.random as npr
 
 from . import _lib
-from ._lib import DwClock, DwConfig, DwRunResult, DW_DIAG, DW_POLICY
+from ._lib import DwClock, DwConfig, DwRunResult, DW_DIAG, DW_E_UNSUPPORTED, DW_POLICY
 
 
 def query_kwargs(key, default, **kwargs):
@@ -419,29 +419,30 @@ class RLDaisyWorld:
 
     def run_series(self, K, policy="greedy", actions=None, seed=0):
         """run() that also returns the per-step ensemble means [K, 3] = (global mean temperature of that step's forward --
-        env.temp.mean() --, mean light cover, mean dark cover): reduced inside the persistent fused kernels (64x64 worlds with at
-        most 32 agents; 8x8, 16x16 and 32x32 worlds), sampled between one-step launches for every other shape."""
+        env.temp.mean() --, mean light cover, mean dark cover): reduced inside the persistent fused kernels where the device
+        has a series mode for the shape and the constants (dw_run_series decides), sampled between one-step launches
+        otherwise."""
         B, N, n = self._shape
         colliding = self.collision_mode == 1 and n      # noise from the caller's NumPy stream every step: host-driven loop
         a8 = None
         if policy == "replay":
             a8 = np.ascontiguousarray(canonical_actions8(np.asarray(actions).reshape(-1, B, n)[:K]))
         out = np.zeros((int(K), 3))
-        in_kernel = (N == 64 and n <= 32) or (N in (8, 16, 32) and (64 // N) ** 2 * n <= 256) or \
-            (N % 4 == 0 and 20 <= N <= 156 and N not in (32, 64) and n <= 1024)
-        if not in_kernel or policy == "mlp" or colliding:
-            # other shapes: one fused step per sample, the same three means from the device-side reductions
-            for t in range(int(K)):
-                self.run(1, policy=policy, actions=None if a8 is None else a8[t:t + 1], seed=seed)
-                c = self.cover_stats()
-                out[t] = (self.diag_stats("temp")["mean"], c["mean_light"], c["mean_dark"])
-            return out
-        self._push()
-        rc = self._lib.dw_run_series(self._h, int(K), DW_POLICY[policy], _ptr(a8, C.c_int8), C.c_uint64(seed), _ptr(out, C.c_double))
-        self._check(rc, "dw_run_series")
-        self._state_changed()
-        self._pull_clock()
-        self._dead_L = None
+        if not colliding and 1 <= K <= 4096:             # dw_run_series takes up to DW_FUSED_MAX_STEPS steps per call
+            self._push()
+            rc = self._lib.dw_run_series(self._h, int(K), DW_POLICY[policy], _ptr(a8, C.c_int8), C.c_uint64(seed),
+                                         _ptr(out, C.c_double))
+            if rc != DW_E_UNSUPPORTED:                   # refused before any step has run: fall through to the loop
+                self._check(rc, "dw_run_series")
+                self._state_changed()
+                self._pull_clock()
+                self._dead_L = None
+                return out
+        # one fused step per sample, the same three means from the device-side reductions
+        for t in range(int(K)):
+            self.run(1, policy=policy, actions=None if a8 is None else a8[t:t + 1], seed=seed)
+            c = self.cover_stats()
+            out[t] = (self.diag_stats("temp")["mean"], c["mean_light"], c["mean_dark"])
         return out
 
     def run_with_series(self, K, every=16, policy="greedy", seed=0):
