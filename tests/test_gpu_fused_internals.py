@@ -45,7 +45,7 @@ def test_fast_root4_relative_error_bound():
                                           (20, 9, 3, "antigreedy"), (96, 3, 5, "greedy"), (128, 2, 6, "random"), (156, 1, 4, "greedy"),
                                           (32, 3, 70, "greedy"),
                                           # sides that are not a multiple of 4: the same kernel with padded rows and masked edge tiles
-                                          # (1, 2 and 3 columns in the last tile); 157 does not fit padded and takes the generic kernel
+                                          # (1, 2 and 3 columns in the last tile); 157 still fits with its rows padded to 160 words
                                           (13, 6, 3, "greedy"), (18, 5, 4, "random"), (61, 3, 5, "greedy"), (150, 1, 4, "antigreedy"),
                                           (157, 1, 2, "greedy")])
 def test_fused_equals_materialising_path(N, B, n, policy):

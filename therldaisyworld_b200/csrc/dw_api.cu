@@ -16,6 +16,20 @@ static thread_local std::string g_create_error;
 
 enum PreKind { PRE_NONE = 0, PRE_GRID = 1, PRE_LAT = 2, PRE_COV = 3 };
 
+// What a fused launch does besides the steps: nothing, record the per-step series (dw_run_series), or run DW_POLICY_MLP
+enum FusedMode { FUSED_PLAIN = 0, FUSED_SERIES = 1, FUSED_MLP = 2, FUSED_MODES = 3 };
+
+// One fused kernel instance: a row of the table in fused_kernel (dw_run.inl)
+struct FusedKernel {
+    void (*kern)(const FusedArgs) = nullptr;   // nullptr: no fused kernel runs this mode at this shape
+    int threads = 256;
+    size_t smem = 0;                           // dynamic shared memory per CTA
+    bool persistent = false;                   // resident CTAs share a (worlds, step chunk) queue; else one CTA per world
+    int worlds = 1;                            // worlds per work item
+    bool trim = false;                         // records alive_mask (dw_run_chunk_masked)
+    int blocks = 0;                            // resident CTAs of a persistent kernel on the handle's device (resolve_fused)
+};
+
 struct dw_handle {
     dw_config cfg{};
     dw_clock clk{};
@@ -89,7 +103,6 @@ struct dw_handle {
     int *pop_done = nullptr;                   // [members] loop ended
     int64_t *pop_steps = nullptr, *pop_frozen = nullptr;   // [members] step count at the end; [B,n] frozen (1-done) counters
     unsigned int *pop_ndone = nullptr;
-    bool fused_attr_set = false;
     unsigned char *pin = nullptr;              // pinned host staging of the single-step path: [action | obs | reward | done]
     size_t pin_cap = 0;
     bool agents_open = false;                  // between dw_agents_begin and dw_agents_collide the agent states are unclipped
@@ -100,16 +113,13 @@ struct dw_handle {
     double sc_eps = 0.0;
     dw_config sc_cfg{};
     unsigned int *persist_sync = nullptr;      // [1 + B] work queue + per-world progress of the persistent kernel
-    int persist_blocks = 0, sub64_blocks = 0;  // resident CTAs of the persistent kernels on this device
-    int sub64_blocks_series = 0;               // sub-64 kernel in series mode
+    FusedKernel fused[FUSED_MODES];            // kernel of each fused mode, resolved on the mode's first launch (resolve_fused)
+    bool fused_ready[FUSED_MODES] = {};
     // statistics-only lifespan runs (dw_run_chunk_masked / dw_trim_lifespans): per-agent "not done" bits of the last chunk
     unsigned long long *alive_mask = nullptr;
     bool mask_on = false, mask_complete = false;
     double *pop_rew = nullptr;                 // [64][B*n] per-step agent states of a fused population segment (k_pop_post)
     bool pop_rew_on = false;
-    int persist_blocks_mlp = 0;                // the same for the kernel with the in-kernel MLP policy (more shared memory)
-    int tile4_threads = 0;                     // block size chosen for k_fused_tile4
-    int tile4_blocks = 0, tile4_blocks_series = 0;    // resident CTAs of the persistent 4x4-tile kernel (plain / series mode)
     // profiling (dw_set_profiling): kernel launch count, and device time of the fused kernel via events
     dw_profile prof{};
     bool profiling = false;
