@@ -20,11 +20,12 @@
  *                     per-step species max. Parts 1 + 2 split it into edge tile rows and interior so that the
  *                     halo exchange can overlap the interior.
  *   ghost rows        toroidal wrap (dwt_halo_wrap, one rank) or the neighbours' edge rows (caller copies whole
- *                     stored rows of N + 8 words).
+ *                     stored rows of dwt_get_pitch words).
  * gain[n] and act[n] are adjacent in memory (gain first): finishing step j can be deferred until the decisions of
  * step j + 1 exist, so that ONE all-reduce per step carries both (therldaisyworld_b200/banded.py does that).
  *
- * Constraints of the tiled kernels: N % 64 == 0, rows % 64 == 0, N >= 64, D4-symmetric kernels (the defaults).
+ * Constraints of the tiled kernels: N >= 64, 8 <= rows <= N, D4-symmetric kernels (the defaults). Bands may differ in
+ * height; a side or band that is not a multiple of 64 runs a masked instance of the stencil kernel over its partial tiles.
  */
 #ifndef DAISYWORLD_B200_TILED_H
 #define DAISYWORLD_B200_TILED_H
@@ -38,13 +39,13 @@ extern "C" {
 typedef struct dwt_handle dwt_handle;
 
 /* Device pointers a multi-rank driver needs (valid until the next dwt_stencil for the halo rows, for the life of the
-   handle for the rest). Row pointers address N + 8 packed u32 words (light milli-cover | dark << 16; word 3 and word N + 4
-   are the ghost columns). */
+   handle for the rest). Row pointers address a whole stored row of dwt_get_pitch packed u32 words (light milli-cover |
+   dark << 16; words 4 .. N + 3 are the N columns, word 3 and word N + 4 the ghost columns, the rest is padding). */
 typedef struct dwt_ptrs {
     double *act;            /* [n]   action + 1 per agent (0 = not decided here); act == gain + n */
     double *gain;           /* [n]   food eaten per agent on this rank */
     int32_t *stepmax;       /* [4096, 2] per-step max milli-cover of (light, dark) over this band */
-    uint32_t *send_top;     /* band row 0 (whole stored row, N + 8 words) -> the rank above's bottom ghost */
+    uint32_t *send_top;     /* band row 0 (whole stored row)              -> the rank above's bottom ghost */
     uint32_t *send_bottom;  /* band row rows-1                            -> the rank below's top ghost */
     uint32_t *recv_top;     /* ghost row above the band */
     uint32_t *recv_bottom;  /* ghost row below the band */
@@ -80,6 +81,8 @@ int dwt_finish_agents(dwt_handle *h);
 int dwt_stencil(dwt_handle *h, int32_t part);   /* 0: whole band; 1: edge tile rows, then 2: interior tile rows */
 int dwt_halo_wrap(dwt_handle *h);      /* one rank: ghost rows from the band's own edge rows */
 int dwt_get_ptrs(dwt_handle *h, dwt_ptrs *out);
+/* words per stored row: 64 * ceil(N / 64) + 8 (N + 8 when N is a multiple of 64), a multiple of 16 bytes */
+int dwt_get_pitch(const dwt_handle *h, int32_t *pitch);
 
 /* K whole steps on one rank (rows == N): the phases above back to back on the handle's stream, no host sync. */
 int dwt_run(dwt_handle *h, int64_t K, int32_t policy, const int8_t *actions /*[K,n] or NULL*/, uint64_t seed);
@@ -116,6 +119,10 @@ int dwt_ipc_attach(dwt_handle *h, int32_t rank, int32_t n_ranks, const void *all
 /* same-process variant (several bands of one process, tests): raw device pointers [n_ranks][DWT_PEER_BUFFERS] */
 int dwt_get_peer_buffers(dwt_handle *h, void **out /* [DWT_PEER_BUFFERS] */);
 int dwt_attach_peers(dwt_handle *h, int32_t rank, int32_t n_ranks, void *const *table);
+/* rows[n_ranks]: the band height of every rank, in rank order (they add up to N). Needed before either attach call when
+   the bands differ in height: a band writes its last row into the ghost row below its upper neighbour's band. Without
+   it, attaching assumes equal bands and refuses with DW_E_STATE when rows * n_ranks != N. */
+int dwt_set_peer_rows(dwt_handle *h, int32_t n_ranks, const int32_t *rows);
 int dwt_step_p2p(dwt_handle *h, int32_t policy, const int8_t *actions /* [n] or NULL */, uint64_t seed);
 int dwt_flush_p2p(dwt_handle *h);                       /* finish the agents of the last step */
 int dwt_peer_status(dwt_handle *h, int32_t *timed_out); /* 1 if a barrier gave up waiting for a peer */

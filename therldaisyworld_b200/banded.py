@@ -1,7 +1,7 @@
 """A single giant toroidal RLDaisyWorld (BASELINE config 5), row-banded over the ranks of one node.
 
 The world is ONE batch element of the reference environment (``daisy/daisy_world_rl.py``, ``batch_size == 1``) whose
-grid does not fit in shared memory: rank r owns rows ``[r*N/R, (r+1)*N/R)`` on its GPU (a ``dwt_handle`` of
+grid does not fit in shared memory: rank r owns rows ``[floor(r*N/R), floor((r+1)*N/R))`` on its GPU (a ``dwt_handle`` of
 ``include/daisyworld_b200_tiled.h``) plus a ghost row above and below.  Agents are replicated on every rank.
 
 One env step = the phase sequence of the header, with exactly these exchanges between ranks (``torch.distributed``:
@@ -39,6 +39,14 @@ def band_rows(N, world_size, rank):
         raise ValueError(f"N={N} must be a multiple of 64*world_size={64 * world_size}")
     R = N // world_size
     return rank * R, (rank + 1) * R
+
+
+def balanced_rows(N, world_size, rank):
+    """Rows [lo, hi) of rank's band in the partition BandedDaisyWorld uses: [floor(rank*N/world_size),
+    floor((rank+1)*N/world_size)), so that bands differ by at most one row. Equals band_rows wherever that succeeds."""
+    if not 0 <= rank < world_size:
+        raise ValueError(f"rank {rank} outside 0..{world_size - 1}")
+    return rank * N // world_size, (rank + 1) * N // world_size
 
 
 class DistComm:
@@ -91,6 +99,9 @@ class DeviceBand:
             msg = self._lib.dwt_last_error(None)
             raise _lib.DaisyWorldError(f"dwt_create failed (code {rc}): {msg.decode() if msg else ''}")
         self._h = h
+        p = C.c_int32(0)
+        self._check(self._lib.dwt_get_pitch(self._h, C.byref(p)), "dwt_get_pitch")
+        self.pitch = int(p.value)          # words per stored row (whole tiles plus the ghost columns)
         self._views = {}
         self._side = None
 
@@ -184,7 +195,15 @@ class DeviceBand:
         self._check(self._lib.dwt_ipc_export(self._h, buf), "dwt_ipc_export")
         return bytes(buf.raw)
 
-    def ipc_attach(self, rank, blobs):
+    def set_peer_rows(self, rows):
+        """Band heights of all ranks in rank order (dwt_set_peer_rows); default: BandedDaisyWorld's balanced partition."""
+        if rows is None:
+            rows = [hi - lo for lo, hi in (balanced_rows(self.N, self.n_ranks, r) for r in range(self.n_ranks))]
+        arr = (C.c_int32 * len(rows))(*[int(r) for r in rows])
+        self._check(self._lib.dwt_set_peer_rows(self._h, len(rows), arr), "dwt_set_peer_rows")
+
+    def ipc_attach(self, rank, blobs, peer_rows=None):
+        self.set_peer_rows(peer_rows)
         blob = b"".join(blobs)
         self._check(self._lib.dwt_ipc_attach(self._h, int(rank), len(blobs), C.create_string_buffer(blob, len(blob))), "dwt_ipc_attach")
 
@@ -193,8 +212,9 @@ class DeviceBand:
         self._check(self._lib.dwt_get_peer_buffers(self._h, out), "dwt_get_peer_buffers")
         return [int(v or 0) for v in out]
 
-    def attach_peers(self, rank, tables):
+    def attach_peers(self, rank, tables, peer_rows=None):
         """Same-process peers: tables[r] = peer_buffers() of rank r."""
+        self.set_peer_rows(peer_rows)
         flat = (C.c_void_p * (4 * len(tables)))(*[p for t in tables for p in t])
         self._check(self._lib.dwt_attach_peers(self._h, int(rank), len(tables), flat), "dwt_attach_peers")
 
@@ -277,10 +297,10 @@ class DeviceBand:
         return self._view(p.value, (4096, 3), "<f8")[:K]
 
     def halo_tensors(self):
-        """(send_top, send_bottom, recv_top, recv_bottom): whole stored rows (N + 8 words, ghost columns included) of the
-        lattice buffer the current step writes, as int32 views."""
+        """(send_top, send_bottom, recv_top, recv_bottom): whole stored rows (pitch words, ghost columns and padding
+        included) of the lattice buffer the current step writes, as int32 views."""
         p = self._ptrs()
-        return tuple(self._view(q, (self.N + 8,), "<i4") for q in (p.send_top, p.send_bottom, p.recv_top, p.recv_bottom))
+        return tuple(self._view(q, (self.pitch,), "<i4") for q in (p.send_top, p.send_bottom, p.recv_top, p.recv_bottom))
 
     # ---- getters
     def reset_lifespans(self):
@@ -342,7 +362,7 @@ class BandedDaisyWorld:
         self.batch_size = 1
         self.rank, self.world_size, self.device = int(rank), int(world_size), int(device)
         self.comm = comm if (comm is not None or self.world_size == 1) else DistComm(rank, world_size, group)
-        self.row0, hi = band_rows(self.dim, self.world_size, self.rank)
+        self.row0, hi = balanced_rows(self.dim, self.world_size, self.rank)
         self.rows = hi - self.row0
         factory = band_factory or (lambda p, N, n, r0, R, nr: DeviceBand(p, N, n, r0, R, nr, device=self.device))
         self.band = factory(self, self.dim, self.n_agents, self.row0, self.rows, self.world_size)

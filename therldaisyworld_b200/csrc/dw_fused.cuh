@@ -133,9 +133,11 @@ __device__ __forceinline__ uint32_t dw_fast_cell(const FastCoef &F, const StepCo
 
 // Two cells in explicit lockstep: the fp64 chain of one cell is serial (8-cycle dependent latency, measured), so the
 // source interleaves two independent cells statement by statement to give the scheduler ILP without more warps.
+// DIAG: tcells = how many of the W cells (a prefix) add their temperature to *tsum (cells outside a partial tile do not).
 template <int W, bool DIAG = false>
 __device__ __forceinline__ void dw_fast_cells(const FastCoef &F, const StepCoef &C, const uint32_t (&pc)[W], const uint32_t (&E)[W],
-                                              const uint32_t (&S)[W], unsigned *tiemin, uint32_t (&out)[W], double *tsum = nullptr) {
+                                              const uint32_t (&S)[W], unsigned *tiemin, uint32_t (&out)[W], double *tsum = nullptr,
+                                              int tcells = W) {
     double kl[W], kd[W], El[W], Ed[W], Sl[W], Sd[W], Rl[W], Rd[W], rb[W], Xl[W], Xd[W];
 #pragma unroll
     for (int i = 0; i < W; ++i) { kl[i] = dw_half2d<false>(pc[i]); kd[i] = dw_half2d<true>(pc[i]); }
@@ -149,7 +151,8 @@ __device__ __forceinline__ void dw_fast_cells(const FastCoef &F, const StepCoef 
     for (int i = 0; i < W; ++i) Xd[i] = Xl[i] + F.xdd;
     if (DIAG) {              // series mode: the (unrounded) temperature of the cell itself, sqrt(g)*T, summed per thread
 #pragma unroll
-        for (int i = 0; i < W; ++i) *tsum += dw_root4_fast(__fma_rn(F.tk_l, kl[i], __fma_rn(F.tk_d, kd[i], Xl[i] + F.t0)));
+        for (int i = 0; i < W; ++i)
+            if (i < tcells) *tsum += dw_root4_fast(__fma_rn(F.tk_l, kl[i], __fma_rn(F.tk_d, kd[i], Xl[i] + F.t0)));
     }
     // seeds first: the MUFU latency (27 cycles) overlaps the rho arithmetic below
     double s1l[W], s1d[W], y0l[W], y0d[W];
@@ -486,8 +489,14 @@ __device__ __forceinline__ uint32_t dw_tile_core(const FastCoef &F, const StepCo
             const uint32_t pa[2] = {mid.p[0], mid.p[1]}, ea[2] = {E[0], E[1]}, sa[2] = {S8[0], S8[1]};
             const uint32_t pb[2] = {mid.p[2], mid.p[3]}, eb[2] = {E[2], E[3]}, sb[2] = {S8[2], S8[3]};
             uint32_t qa[2], qb[2];
-            dw_fast_cells<2, DIAG>(F, C, pa, ea, sa, tiemin, qa, tsum);
-            dw_fast_cells<2, DIAG>(F, C, pb, eb, sb, tiemin, qb, tsum);
+            if constexpr (DIAG && Store::kMasks) {       // series mode of a partial tile: only the store's cells count in tsum
+                const int v = store.cells(i);
+                dw_fast_cells<2, DIAG>(F, C, pa, ea, sa, tiemin, qa, tsum, v);
+                dw_fast_cells<2, DIAG>(F, C, pb, eb, sb, tiemin, qb, tsum, v - 2);
+            } else {
+                dw_fast_cells<2, DIAG>(F, C, pa, ea, sa, tiemin, qa, tsum);
+                dw_fast_cells<2, DIAG>(F, C, pb, eb, sb, tiemin, qb, tsum);
+            }
             q[0] = qa[0]; q[1] = qa[1]; q[2] = qb[0]; q[3] = qb[1];
         }
         if (Store::kMasks) {               // k_fused_tile4, padded sides: the store zeroes entries that lie outside the world

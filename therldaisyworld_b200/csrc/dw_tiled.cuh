@@ -1,15 +1,19 @@
 // Single large world ("giant grid", BASELINE config 5): one toroidal N x N world too large for shared memory, held as a
 // row band of `R` rows per rank (R = N on one GPU) on the packed 0.001 lattice, padded with ghost cells:
 //
-//     lat[(R + 2) x pitch],  pitch = N + 8 words
+//     lat[(64 * tiles_y + 2) x pitch],  pitch = 64 * tiles_x + 8 words,  tiles_x = ceil(N / 64), tiles_y = ceil(R / 64)
 //       row 0        ghost: the row above the band (toroidal wrap, or the neighbouring rank's last row)
 //       rows 1..R    the band
 //       row R + 1    ghost: the row below the band
 //       word 3 / words 4..N+3 / word N+4 of a row: ghost of column N-1 / the N columns / ghost of column 0
+//       words 0..2, words N+5.. and rows R+2.. are padding: never written, never read as cells (zero from the allocation)
+// (N + 8 words and R + 2 rows when N and R are multiples of 64.)
 //
 // With the ghosts in place every 64x64 output tile needs one in-bounds 66-row x 72-word box of the source, which one
 // elected thread fetches with a single TMA (cp.async.bulk.tensor.2d) into shared memory; 256 threads then run the same
 // 4x4-cells-per-thread fast path as the ensemble kernel (dw_tile_core) and write their rows straight back to HBM.
+// The padding keeps every box inside the allocation, so partial tiles (N or R not a multiple of 64) need no out-of-bounds
+// fill: the masked instance of the kernel computes them whole and keeps only the cells inside the band.
 // HBM traffic is 8 B per cell-update (4 B in, 4 B out); at the FP64-bound rate that is ~2 TB/s of the 6.5 TB/s measured,
 // so this kernel is bound by the FP64 pipe like the SMEM-resident one.
 //
@@ -474,15 +478,38 @@ struct StoreGlobalSum {
         *sum += (q[0] + q[1]) + (q[2] + q[3]);
     }
 };
+// Partial tiles: only the thread's cells inside the band (the first `rows` rows and `cols` columns of its 4x4, either may be
+// <= 0 or > 4) are stored; the others are zeroed in q, so that they count neither in the maxima nor in the cover sum.
+template <bool SUM>
+struct StoreGlobalMasked {
+    static constexpr bool kMasks = true;
+    uint32_t *o;
+    int pitch, rows, cols;
+    uint32_t *sum;          // SUM: packed sum of the stored cells (see StoreGlobalSum)
+    __device__ __forceinline__ int cells(int i) const { return i < rows ? min(max(cols, 0), 4) : 0; }
+    __device__ __forceinline__ void operator()(int i, uint32_t (&q)[4]) const {
+        if (i >= rows) { q[0] = 0u; q[1] = 0u; q[2] = 0u; q[3] = 0u; return; }     // below the band: ghost row or padding
+        uint32_t *d = o + (size_t)i * pitch;
+        if (cols >= 4) {
+            *reinterpret_cast<uint4 *>(d) = make_uint4(q[0], q[1], q[2], q[3]);
+        } else {                                         // right of column N-1: the ghost of column 0, then padding
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+                if (t < cols) d[t] = q[t];
+                else q[t] = 0u;
+            }
+        }
+        if (SUM) *sum += (q[0] + q[1]) + (q[2] + q[3]);
+    }
+};
 
 // rare path, warp-cooperative: for every lane whose 4x4 tile hit the tie filter, lanes 0..15 re-evaluate one cell of that
 // tile each from the staged tile; cells on a rounding tie are recomputed in literal order and patched in the output.
 // tile_off / out_off: each lane's offsets of its first cell inside the staged tile / the output lattice.
-// One copy per k_tiled_step instantiation (SERIES is otherwise unused): with a single caller the compiler propagates the
-// address of that kernel's shared tile into it, which the default kernel's code and shared-memory layout depend on.
-template <bool SERIES>
-__device__ __noinline__ uint32_t dwt_fix_warp(const TiledArgs *A, const uint32_t *tile, unsigned flagged, uint32_t mx, int tile_off,
-                                              long long out_off, int lane) {
+// MASK (partial tiles): rows / cols as in StoreGlobalMasked; cells outside the band are neither fixed up nor counted.
+template <bool MASK>
+__device__ __forceinline__ uint32_t dwt_fix_tiles(const TiledArgs *A, const uint32_t *tile, unsigned flagged, uint32_t mx, int tile_off,
+                                                  long long out_off, int lane, int rows, int cols) {
     uint32_t extra = 0;
     bool mine = false;
     __syncwarp();
@@ -491,8 +518,13 @@ __device__ __noinline__ uint32_t dwt_fix_warp(const TiledArgs *A, const uint32_t
         flagged &= flagged - 1;
         const int toff = __shfl_sync(0xffffffffu, tile_off, L);
         const long long ooff = __shfl_sync(0xffffffffu, out_off, L);
+        bool cell = lane < 16;
+        if (MASK) {
+            const int lr = __shfl_sync(0xffffffffu, rows, L), lc = __shfl_sync(0xffffffffu, cols, L);
+            cell = cell && (lane >> 2) < lr && (lane & 3) < lc;
+        }
         if (lane == L) mine = true;
-        if (lane < 16) {
+        if (cell) {
             const uint32_t *p = tile + toff + (lane >> 2) * DWT_TILE_PITCH + (lane & 3);
             const uint32_t *q0 = p - DWT_TILE_PITCH, *q2 = p + DWT_TILE_PITCH;
             const uint32_t E = p[-1] + p[1] + q0[0] + q2[0];
@@ -520,6 +552,18 @@ __device__ __noinline__ uint32_t dwt_fix_warp(const TiledArgs *A, const uint32_t
     __syncwarp();                                        // patches (made by helper lanes) before the owners re-read their cells
     return __vmaxu2(mine ? 0u : mx, extra);
 }
+// One copy per k_tiled_step instantiation (SERIES is otherwise unused): with a single caller the compiler propagates the
+// address of that kernel's shared tile into it, which the default kernel's code and shared-memory layout depend on.
+template <bool SERIES>
+__device__ __noinline__ uint32_t dwt_fix_warp(const TiledArgs *A, const uint32_t *tile, unsigned flagged, uint32_t mx, int tile_off,
+                                              long long out_off, int lane) {
+    return dwt_fix_tiles<false>(A, tile, flagged, mx, tile_off, out_off, lane, 0, 0);
+}
+template <bool SERIES>
+__device__ __noinline__ uint32_t dwt_fix_warp_masked(const TiledArgs *A, const uint32_t *tile, unsigned flagged, uint32_t mx, int tile_off,
+                                                     long long out_off, int lane, int rows, int cols) {
+    return dwt_fix_tiles<true>(A, tile, flagged, mx, tile_off, out_off, lane, rows, cols);
+}
 
 __device__ __forceinline__ void dwt_issue_tile(const CUtensorMap *tmap, const TiledArgs &A, int t, uint32_t smem_tile, uint32_t bar_a) {
     const int tc = t % A.tiles_x;
@@ -537,9 +581,13 @@ __device__ __forceinline__ void dwt_issue_tile(const CUtensorMap *tmap, const Ti
 // SERIES: the step also adds the sums of its produced cells to series[0..2], one atomicAdd per column and CTA:
 // {sqrt(g)*T of the forward (unrounded, from the staged pre-state), new milli-light, new milli-dark}. `series` is the last
 // parameter (not a member of TiledArgs), so that every parameter offset of the default kernel stays where it was.
-template <bool SERIES = false>
+// MASK: the instance for a side N or a band height `rows` that is not a multiple of 64. The cells of the partial tiles that
+// lie outside the band are computed from padding and dropped: not stored (the last tile row would otherwise overwrite the
+// ghost row below the band), not fixed up, and counted neither in the maxima nor in the series sums. The ghost column of
+// N-1 is copied by the thread that holds column N-1. `rows` follows `series` for the same reason as `series`.
+template <bool SERIES = false, bool MASK = false>
 __global__ void __launch_bounds__(256, 4) k_tiled_step(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ TiledArgs A,
-                                                       int n_tiles, double *series = nullptr) {
+                                                       int n_tiles, double *series = nullptr, int rows = 0) {
     constexpr int kTileWords = ((DWT_TILE_BYTES + 127) / 128) * 32;       // a TMA destination must be 128-byte aligned: 19008 -> 19072 B
     __shared__ __align__(128) uint32_t tile[kTileWords];
     __shared__ __align__(8) unsigned long long bar;
@@ -573,29 +621,56 @@ __global__ void __launch_bounds__(256, 4) k_tiled_step(const __grid_constant__ C
         const long long out_off = (long long)(tr * DWT_TILE + 1 + r0) * A.pitch + 4 + tc * DWT_TILE + 4 * tx;
         unsigned tiemin = 0xffffffffu;
         uint32_t mx, cov = 0;
-        if constexpr (SERIES)
+        // MASK: rows / columns of the thread's 4x4 cells inside the band
+        const int vr = MASK ? rows - (tr * DWT_TILE + r0) : 4, vc = MASK ? A.N - (tc * DWT_TILE + 4 * tx) : 4;
+        if constexpr (MASK)
+            mx = dw_tile_core<RowsTile72, StoreGlobalMasked<SERIES>, SERIES>(
+                A.F, A.C, RowsTile72{tile + tile_off}, StoreGlobalMasked<SERIES>{A.out + out_off, A.pitch, vr, vc, &cov}, &tiemin, &tsum);
+        else if constexpr (SERIES)
             mx = dw_tile_core<RowsTile72, StoreGlobalSum, true>(A.F, A.C, RowsTile72{tile + tile_off}, StoreGlobalSum{A.out + out_off, A.pitch, &cov},
                                                                 &tiemin, &tsum);
         else
             mx = dw_tile_core(A.F, A.C, RowsTile72{tile + tile_off}, StoreGlobal{A.out + out_off, A.pitch}, &tiemin);
         const unsigned flagged = __ballot_sync(0xffffffffu, tiemin < A.F.tie_thresh);
         if (flagged) {
-            mx = dwt_fix_warp<SERIES>(&A, tile, flagged, mx, tile_off, out_off, lane);
+            if constexpr (MASK) mx = dwt_fix_warp_masked<SERIES>(&A, tile, flagged, mx, tile_off, out_off, lane, vr, vc);
+            else mx = dwt_fix_warp<SERIES>(&A, tile, flagged, mx, tile_off, out_off, lane);
             if constexpr (SERIES) {
                 if ((flagged >> lane) & 1u) {            // literal fix-ups were patched into this lane's cells: sum them again
                     const uint32_t *o = A.out + out_off;
                     cov = 0;
+                    if constexpr (MASK) {
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const uint4 v = *reinterpret_cast<const uint4 *>(o + (size_t)i * A.pitch);
-                        cov += (v.x + v.y) + (v.z + v.w);
+                        for (int i = 0; i < 4; ++i)
+#pragma unroll
+                            for (int c = 0; c < 4; ++c)
+                                if (i < vr && c < vc) cov += o[(size_t)i * A.pitch + c];
+                    } else {
+#pragma unroll
+                        for (int i = 0; i < 4; ++i) {
+                            const uint4 v = *reinterpret_cast<const uint4 *>(o + (size_t)i * A.pitch);
+                            cov += (v.x + v.y) + (v.z + v.w);
+                        }
                     }
                 }
             }
         }
         if constexpr (SERIES) { cl += cov & 0xffffu; cd += cov >> 16; }
         // ghost columns of the produced rows: the two threads of a row group that hold column 0 / N-1 copy their (final) cells
-        if (tx == 0 && tc == 0) {
+        if constexpr (MASK) {
+            if (tx == 0 && tc == 0) {
+                uint32_t *o = A.out + out_off;
+#pragma unroll
+                for (int i = 0; i < 4; ++i)
+                    if (i < vr) o[(size_t)i * A.pitch + A.N] = o[(size_t)i * A.pitch];
+            }
+            if (tx == ((A.N - 1) & (DWT_TILE - 1)) >> 2 && tc == A.tiles_x - 1) {
+                uint32_t *o = A.out + out_off + ((A.N - 1) & 3);
+#pragma unroll
+                for (int i = 0; i < 4; ++i)
+                    if (i < vr) o[(size_t)i * A.pitch - A.N] = o[(size_t)i * A.pitch];
+            }
+        } else if (tx == 0 && tc == 0) {
             uint32_t *o = A.out + out_off;
 #pragma unroll
             for (int i = 0; i < 4; ++i) o[(size_t)i * A.pitch + A.N] = o[(size_t)i * A.pitch];

@@ -1,7 +1,14 @@
 """Time the giant-grid path in isolation on one GPU: N x N torus, n agents, K steps after the literal first step.
 
 --series: the cost of series mode (BandedDaisyWorld.run_series): the same K steps with series mode off and on, the two arms
-alternating, five repetitions each (optional argument: N, default 16384)."""
+alternating, five repetitions each (optional argument: N, default 16384).
+
+--sides N1 N2 ...: the stencil kernel alone (dwt_debug_time_stencil) and whole steps at each side, N agents, the sides
+alternating over five repetitions; the rates are reported against the first side. Sides that are not a multiple of 64 run
+the masked instance of the stencil kernel over their partial tiles.
+
+--vs-ensemble N: whole greedy steps of one N x N world as the giant world (BandedDaisyWorld.run) and as an ensemble of one
+(RLDaisyWorld, batch_size = 1, run()), 4 agents like RLDaisyWorld's default, alternating over five repetitions."""
 import sys, os, subprocess, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -66,7 +73,74 @@ def bench_series(N, n, policy, K=256, reps=5):
           f"{100.0 * (np.median(on) / np.median(off) - 1.0):+.1f} % per step", flush=True)
 
 
+def bench_sides(sides, K=64, reps=5, stencil_reps=50):
+    worlds = {}
+    for N in sides:
+        w = BandedDaisyWorld(N, N)
+        w.reset_on_device(seed=1)
+        w.run(2, "greedy")
+        worlds[N] = w
+    sten, step = {N: [] for N in sides}, {N: [] for N in sides}
+    for _ in range(reps):
+        for N in sides:
+            w = worlds[N]
+            sten[N].append(w.band.time_stencil(stencil_reps))
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda.synchronize()
+            e0.record()
+            w.band.run_local(K, "greedy")
+            e1.record()
+            torch.cuda.synchronize()
+            w._pending += K
+            w.end_chunk()
+            step[N].append(e0.elapsed_time(e1) / K * 1e3)
+    base = sides[0]
+    rate = lambda N, us: N * N / (us * 1e-6)
+    print(f"{len(sides)} sides, N agents each, {reps} alternating repetitions; stencil: {stencil_reps} launches, steps: K={K} greedy")
+    for N in sides:
+        ms, mt = np.median(sten[N]), np.median(step[N])
+        print(f"  N={N}: stencil us " + " ".join(f"{t:.1f}" for t in sten[N]) + f" | median {ms:.1f} us = {rate(N, ms):.4e} "
+              f"cell-updates/s, {rate(N, ms) / rate(base, np.median(sten[base])):.4f} of N={base}")
+        print(f"  N={N}: step    us " + " ".join(f"{t:.1f}" for t in step[N]) + f" | median {mt:.1f} us = {rate(N, mt):.4e} "
+              f"cell-updates/s, {rate(N, mt) / rate(base, np.median(step[base])):.4f} of N={base}", flush=True)
+
+
+def bench_vs_ensemble(N, K=200, reps=5):
+    from therldaisyworld_b200 import RLDaisyWorld
+    n = 4
+    giant = BandedDaisyWorld(N, n)
+    giant.reset_on_device(seed=1)
+    giant.run(2, "greedy")
+    env = RLDaisyWorld(grid_dimension=N, n_agents=n, device=0)
+    env.batch_size = 1
+    env.reset()
+    env.run(2, policy="greedy")
+    times = {"giant": [], "ensemble": []}
+    for _ in range(reps):
+        for arm in times:
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            if arm == "giant":
+                giant.run(K, "greedy", chunk=K)
+            else:
+                env.run(K, policy="greedy")
+            torch.cuda.synchronize()
+            times[arm].append((time.perf_counter() - t0) / K * 1e6)
+    print(f"N={N}, {n} agents, greedy, K={K} steps per run() call, {reps} alternating repetitions (host clock, synchronised)")
+    for arm, ts in times.items():
+        print(f"  {arm:8s} us/step: " + " ".join(f"{t:.1f}" for t in ts) + f" | median {np.median(ts):.1f}")
+    print(f"  ensemble / giant: {np.median(times['ensemble']) / np.median(times['giant']):.2f}x", flush=True)
+
+
 if __name__ == "__main__":
+    if "--sides" in sys.argv or "--vs-ensemble" in sys.argv:
+        print(f"GPU: {gpu_label()}")
+        args = [int(a) for a in sys.argv[1:] if not a.startswith("--")]
+        if "--sides" in sys.argv:
+            bench_sides(args)
+        else:
+            bench_vs_ensemble(args[0])
+        sys.exit(0)
     if "--series" in sys.argv:
         args = [a for a in sys.argv[1:] if a != "--series"]
         N = int(args[0]) if args else 16384
