@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define DW_ABI_VERSION 2
+#define DW_ABI_VERSION 3
 
 enum {
     DW_OK = 0,
@@ -36,7 +36,7 @@ enum {
     DW_E_STATE = -4         /* call not valid in the current state */
 };
 
-/* Policies executed on the device inside dw_step_policy / dw_run. */
+/* Policies executed on the device inside dw_step_packed / dw_run. */
 enum {
     DW_POLICY_NONE = 0,       /* step(None): all-zero action when n_agents>0 (daisy_world_rl.py:477-478) */
     DW_POLICY_GREEDY = 1,     /* Greedy(eps=0), argmax branch (daisy/agents/greedy.py:16-30) */
@@ -151,53 +151,48 @@ int dw_init_random(dw_handle *h, uint64_t seed, double light_proportion, double 
    T_dark of the uploaded covers at the current clock L. Called by reset() after dw_upload_state. */
 int dw_init_temperatures(dw_handle *h);
 
-/* RLDaisyWorld.step(action) (daisy_world_rl.py:475-497): update_agents -> forward -> get_obs ->
-   reward/done -> update_L, all on the device.  action: host int64 [ab,am] (ab<=B, am<=n) or NULL for step(None).
+/* RLDaisyWorld.step(action) (daisy_world_rl.py:475-497): update_agents -> forward -> get_obs -> reward/done -> update_L,
+   all on the device, with ALL of its return values brought to the host by one copy.
+   policy < 0: action is host int64 [ab,am] (ab<=B, am<=n), or NULL for step(None). Action values: ANY integer, read like
+   the reference does (a == 8 stays, else a % 4 moves, a > 4 grazes; daisy_world_rl.py:190-212). Otherwise the action is
+   chosen on the device by DW_POLICY_* (Greedy.__call__ or MLP.get_action fused in) and `action` is ignored.
    The state stays where the fused kernels keep it (packed 0.001 lattice, or the lean cover planes right after a reset)
    whenever the fast path covers the physics: one K = 1 launch of the fused kernel; the fp64 grid[B,7,N,N], the
    diagnostics and the observation windows are rebuilt on demand from the state the step started from. Partial actions
-   (ab < B or am < n) and non-D4-symmetric kernels run the materialising kernels (64 B per cell). */
-int dw_step(dw_handle *h, const int64_t *action, int32_t ab, int32_t am);
-/* dw_step followed by everything step() returns, in one call with one synchronisation: obs[B,n,7,3,3], reward and done
-   ([B,n], or [B,2] when n_agents == 0) and the advanced clock. Any output pointer may be NULL. policy < 0: explicit
-   action (or NULL = step(None)); otherwise the action is chosen on the device like dw_step_policy. */
-int dw_step_collect(dw_handle *h, const int64_t *action, int32_t ab, int32_t am, int32_t policy, uint64_t seed, double *obs,
-                    double *reward, uint8_t *done, dw_clock *clk);
-/* The same step with ALL of its return values brought to the host by one copy: `out` receives the device's output block
-   [reward f64 B*m | done u8 B*m, padded to a multiple of 8 | obs f64 B*n*63] (m = n, or 2 when n_agents == 0); byte offsets
-   from dw_step_out_layout: layout[4] = {reward, done, obs, total bytes}. want_obs == 0 stops after the reward/done part
-   (device policies do not need the observation on the host: at B = 1000, n = 4 it is 2 MB of the 2.04 MB). With `out`
-   from dw_host_alloc (page-locked) the copy is a single DMA at PCIe rate. action values: ANY integer, read like the
-   reference does (a == 8 stays, else a % 4 moves, a > 4 grazes; daisy_world_rl.py:190-212). */
+   (ab < B or am < n) and non-D4-symmetric kernels run the materialising kernels (64 B per cell).
+   `out` receives the device's output block [reward f64 B*m | done u8 B*m, padded to a multiple of 8 | obs f64 B*n*63]
+   (m = n, or 2 when n_agents == 0); byte offsets from dw_step_out_layout: layout[4] = {reward, done, obs, total bytes}.
+   want_obs == 0 stops after the reward/done part (device policies do not need the observation on the host: at B = 1000,
+   n = 4 it is 2 MB of the 2.04 MB). With `out` from dw_host_alloc (page-locked) the copy is a single DMA at PCIe rate.
+   clk (may be NULL) receives the advanced clock. */
 int dw_step_out_layout(dw_handle *h, int64_t *layout /*[4]*/);
 int dw_step_packed(dw_handle *h, const int64_t *action, int32_t ab, int32_t am, int32_t policy, uint64_t seed,
                    int32_t want_obs, void *out, dw_clock *clk);
 int dw_host_alloc(uint64_t bytes, void **out);
 int dw_host_free(void *p);
-/* Same step with the action chosen on the device by DW_POLICY_* (Greedy.__call__ fused in). */
-int dw_step_policy(dw_handle *h, int32_t policy, uint64_t seed);
 
 /* Pieces of step(), exposed because callers use them standalone:
    RLDaisyWorld.update_agents(action) (:181-244) */
 int dw_update_agents(dw_handle *h, const int64_t *action, int32_t ab, int32_t am);
 /* collision_mode == 1 (daisy_world_rl.py:220-242, default off): where several agents share a cell after the moves, the
    reference draws npr.rand(1, n, 1) from the caller's GLOBAL NumPy stream per shared cell, in (world, x, y) scan order.
-   The stream stays with the caller, so update_agents is split around the draws:
+   The stream stays with the caller, so the step is split around the draws:
      dw_agents_begin    pay agent_gamma, move, graze (no clip yet); returns the post-move agent_indices [B,n,2] so that the
                         caller can count the shared cells of every world (integer bookkeeping only) and draw.
-                        policy < 0: explicit action [ab,am] (NULL = step(None)); else DW_POLICY_NONE..EPS_GREEDY on the device.
+                        action, policy and seed as in dw_step_packed.
      dw_agents_collide  noise [cells, n] (the draws, in order), cell_offsets [B+1] (first draw of each world, [0] = 0):
                         resolves the collisions on the device (winner = resident with the largest state + 0.01 * noise,
                         gains food_chain_penalty * np.sum(other residents' states), losers keep theirs like :242) and
                         clips. Fails with DW_E_INVALID if a world's shared-cell count differs from the device's.
-     dw_step_tail_collect   the rest of step(): forward, stamp, obs, reward/done, update_L; outputs like dw_step_collect.
+     dw_step_tail_packed   the rest of step(): forward, stamp, obs, reward/done, update_L; want_obs, out and clk as in
+                        dw_step_packed.
    Every other stepping call returns DW_E_STATE between dw_agents_begin and dw_agents_collide. */
 int dw_agents_begin(dw_handle *h, const int64_t *action, int32_t ab, int32_t am, int32_t policy, uint64_t seed,
                     int64_t *agent_indices);
 int dw_agents_collide(dw_handle *h, const double *noise, const int32_t *cell_offsets, double food_chain_penalty);
-int dw_step_tail_collect(dw_handle *h, double *obs, double *reward, uint8_t *done, dw_clock *clk);
+int dw_step_tail_packed(dw_handle *h, int32_t want_obs, void *out, dw_clock *clk);
 /* same tail for multi-step loops with collisions: advances the lifespan counters of dw_run (notebook cell 2) instead of
-   collecting the observation; *worlds_alive = worlds with max(grid[:,1:3]) > 0.005 after the step */
+   collecting the outputs; *worlds_alive = worlds with max(grid[:,1:3]) > 0.005 after the step */
 int dw_step_tail_counted(dw_handle *h, int64_t *worlds_alive);
 /* RLDaisyWorld.forward(grid) (:434-461) on a caller grid (host in, host out) with the handle's agents/L;
    writes the mutated ch0 back into grid_in like the reference (:381). Does not advance the state. */
@@ -225,7 +220,6 @@ int dw_f32_stats(dw_handle *h, uint64_t *out /*[3]*/);
 int dw_debug_time_materialise(dw_handle *h, int32_t fp32, int32_t reps, double *ms_per_call);
 int dw_get_agents(dw_handle *h, int64_t *agent_indices, double *agent_states);
 int dw_get_obs(dw_handle *h, double *obs);                                /* obs of the last step / current state */
-int dw_get_reward_done(dw_handle *h, double *reward, uint8_t *done);      /* [B,n] (or [B,2] when n_agents==0) */
 int dw_get_diag(dw_handle *h, int32_t which, double *out);                /* env.temp, env.beta_l, env.growth ... */
 /* Ensemble statistics of one diagnostic field reduced on the device (what the notebooks compute with env.temp.mean(),
    notebook_helpers.py:50,145,218): out = {mean, population std, min, max} over all worlds and cells (both channels for

@@ -37,7 +37,7 @@ def test_library_exports_every_declared_symbol(lib):
     out = subprocess.check_output(["nm", "-D", "--defined-only", _lib.LIB_PATH], text=True)
     exported = set(re.findall(r"\bT (dw_[A-Za-z0-9_]+)", out))
     assert set(declared) <= exported, f"missing: {set(declared) - exported}"
-    assert lib.dw_abi_version() == 2
+    assert lib.dw_abi_version() == 3
     tiled = header_symbols(HEADER_TILED, "dwt_")
     assert tiled and sorted(_lib.TILED_SYMBOLS) == tiled, "_lib.py and daisyworld_b200_tiled.h disagree"
     exported_t = set(re.findall(r"\bT (dwt_[A-Za-z0-9_]+)", out))

@@ -274,8 +274,10 @@ def test_collision_abi_state_machine_and_count_check():
     lib, h = env._lib, env._h
     pos = np.empty((2, 20, 2), dtype=np.int64)
     assert lib.dw_agents_begin(h, None, 0, 0, -1, C.c_uint64(0), pos.ctypes.data_as(C.POINTER(C.c_int64))) == 0
-    assert lib.dw_step_policy(h, 1, C.c_uint64(0)) == -4
-    assert lib.dw_step(h, None, 0, 0) == -4
+    out = np.empty(1 << 16, dtype=np.uint8)                                   # more than the output block of 2 x 20 agents
+    out_ptr = out.ctypes.data_as(C.c_void_p)
+    assert lib.dw_step_packed(h, None, 0, 0, 1, C.c_uint64(0), 1, out_ptr, None) == -4      # device policy
+    assert lib.dw_step_packed(h, None, 0, 0, -1, C.c_uint64(0), 1, out_ptr, None) == -4     # NULL actions
     assert lib.dw_agents_begin(h, None, 0, 0, -1, C.c_uint64(0), pos.ctypes.data_as(C.POINTER(C.c_int64))) == -4
     off = np.zeros(3, dtype=np.int32)                                         # claims "no shared cells"
     assert lib.dw_agents_collide(h, None, off.ctypes.data_as(C.POINTER(C.c_int32)), 0.5) == -1

@@ -37,9 +37,9 @@ class DwRunResult(C.Structure):
 SYMBOLS = [
     "dw_abi_version", "dw_last_error", "dw_create", "dw_destroy", "dw_set_config", "dw_set_clock", "dw_get_clock", "dw_get_last_L",
     "dw_set_stream", "dw_set_epsilon", "dw_set_mlp", "dw_set_mlp_population", "dw_run_population", "dw_get_population_results",
-    "dw_upload_state", "dw_upload_covers", "dw_init_random", "dw_init_temperatures", "dw_set_profiling", "dw_get_profile", "dw_step", "dw_step_collect", "dw_step_out_layout", "dw_step_packed", "dw_host_alloc", "dw_host_free", "dw_step_policy", "dw_update_agents",
-    "dw_agents_begin", "dw_agents_collide", "dw_step_tail_collect", "dw_step_tail_counted",
-    "dw_forward", "dw_get_obs_at", "dw_get_grid", "dw_trim_supported", "dw_run_chunk_masked", "dw_trim_lifespans", "dw_get_grid_f32", "dw_get_obs_f32", "dw_f32_stats", "dw_debug_time_materialise", "dw_get_agents", "dw_get_obs", "dw_get_reward_done", "dw_get_diag", "dw_get_diag_stats", "dw_get_cover_stats",
+    "dw_upload_state", "dw_upload_covers", "dw_init_random", "dw_init_temperatures", "dw_set_profiling", "dw_get_profile", "dw_step_out_layout", "dw_step_packed", "dw_host_alloc", "dw_host_free", "dw_update_agents",
+    "dw_agents_begin", "dw_agents_collide", "dw_step_tail_packed", "dw_step_tail_counted",
+    "dw_forward", "dw_get_obs_at", "dw_get_grid", "dw_trim_supported", "dw_run_chunk_masked", "dw_trim_lifespans", "dw_get_grid_f32", "dw_get_obs_f32", "dw_f32_stats", "dw_debug_time_materialise", "dw_get_agents", "dw_get_obs", "dw_get_diag", "dw_get_diag_stats", "dw_get_cover_stats",
     "dw_run", "dw_run_chunk", "dw_run_series", "dw_reset_lifespans", "dw_get_lifespans", "dw_lifespan_stats_device",
     "dw_checkpoint_save", "dw_checkpoint_restore", "dw_synchronize", "dw_set_world_offset", "dw_debug_slow_count", "dw_debug_state",
     "dw_debug_root4", "dw_debug_markstein", "dw_debug_markstein_f32", "dw_debug_fp64_peak", "dw_debug_screen_error",
@@ -100,9 +100,6 @@ def load():
         "dw_init_temperatures": (C.c_int, [vp]),
         "dw_set_profiling": (C.c_int, [vp, i32]),
         "dw_get_profile": (C.c_int, [vp, C.POINTER(DwProfile)]),
-        "dw_step": (C.c_int, [vp, pi64, i32, i32]),
-        "dw_step_policy": (C.c_int, [vp, i32, u64]),
-        "dw_step_collect": (C.c_int, [vp, pi64, i32, i32, i32, u64, pd, pd, pu8, C.POINTER(DwClock)]),
         "dw_step_out_layout": (C.c_int, [vp, pi64]),
         "dw_step_packed": (C.c_int, [vp, pi64, i32, i32, i32, u64, i32, vp, C.POINTER(DwClock)]),
         "dw_host_alloc": (C.c_int, [u64, C.POINTER(vp)]),
@@ -110,7 +107,7 @@ def load():
         "dw_update_agents": (C.c_int, [vp, pi64, i32, i32]),
         "dw_agents_begin": (C.c_int, [vp, pi64, i32, i32, i32, u64, pi64]),
         "dw_agents_collide": (C.c_int, [vp, pd, C.POINTER(C.c_int32), C.c_double]),
-        "dw_step_tail_collect": (C.c_int, [vp, pd, pd, pu8, C.POINTER(DwClock)]),
+        "dw_step_tail_packed": (C.c_int, [vp, i32, vp, C.POINTER(DwClock)]),
         "dw_step_tail_counted": (C.c_int, [vp, C.POINTER(C.c_int64)]),
         "dw_forward": (C.c_int, [vp, pd, pd]),
         "dw_get_obs_at": (C.c_int, [vp, pi64, i32, i32, pd]),
@@ -124,7 +121,6 @@ def load():
         "dw_debug_time_materialise": (C.c_int, [vp, C.c_int32, C.c_int32, C.POINTER(C.c_double)]),
         "dw_get_agents": (C.c_int, [vp, pi64, pd]),
         "dw_get_obs": (C.c_int, [vp, pd]),
-        "dw_get_reward_done": (C.c_int, [vp, pd, pu8]),
         "dw_get_diag": (C.c_int, [vp, i32, pd]),
         "dw_get_diag_stats": (C.c_int, [vp, i32, pd]),
         "dw_get_cover_stats": (C.c_int, [vp, pd]),
@@ -197,7 +193,7 @@ def load():
         fn = getattr(lib, name)      # AttributeError if the library lacks a declared symbol
         fn.restype = res
         fn.argtypes = args
-    if lib.dw_abi_version() != 2:
+    if lib.dw_abi_version() != 3:
         raise DaisyWorldError("ABI version mismatch between _lib.py and libdaisyworld_b200.so")
     _lib = lib
     return lib

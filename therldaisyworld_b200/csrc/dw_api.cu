@@ -103,8 +103,7 @@ struct dw_handle {
     int *pop_done = nullptr;                   // [members] loop ended
     int64_t *pop_steps = nullptr, *pop_frozen = nullptr;   // [members] step count at the end; [B,n] frozen (1-done) counters
     unsigned int *pop_ndone = nullptr;
-    unsigned char *pin = nullptr;              // pinned host staging of the single-step path: [action | obs | reward | done]
-    size_t pin_cap = 0;
+    unsigned char *pin = nullptr;              // pinned host staging of a step's explicit action bytes (stage_action)
     bool agents_open = false;                  // between dw_agents_begin and dw_agents_collide the agent states are unclipped
     StepCoef *sc_dev = nullptr;                // per-step coefficient table of a fused launch
     std::vector<dw_clock> sc_clk;              // clock before each step of the table on the device (+ the one after the last)
@@ -542,14 +541,12 @@ extern "C" int dw_init_temperatures(dw_handle *h) {
     return DW_OK;
 }
 
-// Small transfers of the single-step path go through pinned staging memory: a pageable cudaMemcpyAsync blocks the host for
-// every copy, a pinned one is enqueued and the step ends with ONE synchronisation. Layout: [action count bytes | outputs].
+// A step's action bytes go through pinned staging memory: a pageable cudaMemcpyAsync blocks the host for every copy, a
+// pinned one is enqueued and the step ends with ONE synchronisation.
 #define DW_PIN_ACTION_MAX (64 * 1024)
-#define DW_PIN_OUT_MAX (512 * 1024)
 static int ensure_pinned(dw_handle *h) {
     if (h->pin) return DW_OK;
-    DW_CUDA_TRY(h, cudaMallocHost((void **)&h->pin, DW_PIN_ACTION_MAX + DW_PIN_OUT_MAX));
-    h->pin_cap = DW_PIN_ACTION_MAX + DW_PIN_OUT_MAX;
+    DW_CUDA_TRY(h, cudaMallocHost((void **)&h->pin, DW_PIN_ACTION_MAX));
     return DW_OK;
 }
 
@@ -629,27 +626,68 @@ static int launch_forward_tail(dw_handle *h, bool counters, unsigned int *alive_
     return DW_OK;
 }
 
+static int mlp_actions(dw_handle *h);
+static int run_steps_fused(dw_handle *h, int K, int policy, const int8_t *act_dev, uint64_t seed, unsigned int *alive);
+static bool dw_fused_supported(const dw_handle *h);
+
+// Between dw_agents_begin and dw_agents_collide the agent states are unclipped: every other stepping call is refused.
+static int refuse_open(dw_handle *h, const char *what) {
+    return h->agents_open ? dw_fail(h, DW_E_STATE, what, "dw_agents_begin not closed by dw_agents_collide") : DW_OK;
+}
+
+// What the agent kernels of one step run. A step's actions come from one of four sources: explicit host actions [ab<=B,
+// am<=n] (policy < 0, staged to the device), NULL (policy < 0: step(None)), the device MLP (DW_POLICY_MLP: its actions are
+// computed here from the current state, then replayed) or a device policy decided inside the kernels.
+struct StepActions {
+    const int8_t *act;   // device int8 [ab,am] of DW_POLICY_REPLAY, else NULL
+    int ab, am;
+    int policy;          // DW_POLICY_REPLAY, DW_POLICY_NONE or the device policy
+    uint64_t seed;       // the caller's for device policies, 0 for explicit actions (REPLAY and NONE do not read it)
+};
+static int resolve_actions(dw_handle *h, const char *what, const int64_t *action, int32_t ab, int32_t am, int32_t policy,
+                           uint64_t seed, StepActions *sa) {
+    int rc = refuse_open(h, what);
+    if (rc) return rc;
+    if (policy == DW_POLICY_REPLAY || policy > DW_POLICY_MLP)
+        return dw_fail(h, DW_E_INVALID, what, "policy must be < 0 (explicit action / NULL) or a device policy");
+    const int B = h->cfg.batch, n = h->cfg.n_agents;
+    if (policy < 0) {
+        *sa = StepActions{nullptr, 0, 0, DW_POLICY_NONE, 0};
+        if (!action || n == 0) return DW_OK;
+        if (ab < 0 || am < 0 || ab > B || am > n) return dw_fail(h, DW_E_INVALID, what, "action must be [ab<=B, am<=n]");
+        rc = stage_action(h, action, (size_t)ab * am);
+        if (rc) return rc;
+        *sa = StepActions{h->action_dev, ab, am, DW_POLICY_REPLAY, 0};
+        return DW_OK;
+    }
+    *sa = StepActions{nullptr, 0, 0, policy, seed};
+    if (policy != DW_POLICY_MLP) return DW_OK;
+    if (n == 0) {
+        sa->policy = DW_POLICY_NONE;
+        return DW_OK;
+    }
+    // the network's actions from the observation of the current state: before anything of this step is launched
+    rc = mlp_actions(h);
+    if (rc) return rc;
+    *sa = StepActions{h->action_dev, B, n, DW_POLICY_REPLAY, seed};
+    return DW_OK;
+}
+
 extern "C" int dw_update_agents(dw_handle *h, const int64_t *action, int32_t ab, int32_t am) {
     if (!h) return DW_E_INVALID;
     DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     if (h->cfg.n_agents == 0) return DW_OK;
-    if (!action || ab < 0 || am < 0 || ab > h->cfg.batch || am > h->cfg.n_agents)
-        return dw_fail(h, DW_E_INVALID, "dw_update_agents", "action must be [ab<=B, am<=n]");
-    if (h->agents_open) return dw_fail(h, DW_E_STATE, "dw_update_agents", "dw_agents_begin not closed by dw_agents_collide");
-    int rc = ensure_grid(h);
+    if (!action) return dw_fail(h, DW_E_INVALID, "dw_update_agents", "action must be [ab<=B, am<=n]");
+    StepActions sa;
+    int rc = resolve_actions(h, "dw_update_agents", action, ab, am, -1, 0, &sa);
+    if (!rc) rc = ensure_grid(h);
     if (rc) return rc;
-    rc = stage_action(h, action, (size_t)ab * am);
-    if (rc) return rc;
-    rc = launch_agents(h, h->action_dev, ab, am, DW_POLICY_REPLAY, 0);
+    rc = launch_agents(h, sa.act, sa.ab, sa.am, sa.policy, sa.seed);
     h->lat_valid = false;
     h->cov_valid = false;
     state_changed(h);
     return rc;
 }
-
-static int mlp_actions(dw_handle *h);
-static int run_steps_fused(dw_handle *h, int K, int policy, const int8_t *act_dev, uint64_t seed, unsigned int *alive);
-static bool dw_fused_supported(const dw_handle *h);
 
 // step() keeps the state where the fused kernels keep it (packed lattice / lean reset planes) whenever the physics is one
 // the fast path covers: one K = 1 launch of the fused kernel instead of materialising the fp64 [B,7,N,N] grid (64 B per
@@ -666,37 +704,32 @@ struct CountLifeGuard {
     ~CountLifeGuard() { h->count_life = old; }
 };
 
+// One step() with its actions from any source (resolve_actions), lean or materialising (lean_step_ok); the outputs stay in
+// the device's output block
+static int step_once(dw_handle *h, const int64_t *action, int32_t ab, int32_t am, int32_t policy, uint64_t seed) {
+    StepActions sa;
+    int rc = resolve_actions(h, "dw_step_packed", action, ab, am, policy, seed, &sa);
+    if (rc) return rc;
+    if (lean_step_ok(h, policy < 0 ? action : nullptr, ab, am)) {
+        CountLifeGuard guard(h, false);
+        return run_steps_fused(h, 1, sa.policy, sa.act, sa.seed, h->alive);
+    }
+    rc = ensure_grid(h);
+    if (!rc) rc = launch_agents(h, sa.act, sa.ab, sa.am, sa.policy, sa.seed);
+    if (rc) return rc;
+    return launch_forward_tail(h, false, nullptr);
+}
+
 // ---- collision_mode == 1 (daisy_world_rl.py:220-242): update_agents in two calls around the caller's RNG draws ----
 extern "C" int dw_agents_begin(dw_handle *h, const int64_t *action, int32_t ab, int32_t am, int32_t policy, uint64_t seed,
                                int64_t *agent_indices) {
     if (!h) return DW_E_INVALID;
     DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (h->agents_open) return dw_fail(h, DW_E_STATE, "dw_agents_begin", "previous dw_agents_begin not closed by dw_agents_collide");
     if (h->cfg.n_agents == 0) return DW_OK;
-    if (policy > DW_POLICY_MLP || policy == DW_POLICY_REPLAY)
-        return dw_fail(h, DW_E_INVALID, "dw_agents_begin", "policy must be < 0 (explicit action / NULL) or a device policy");
-    int rc = DW_OK;
-    if (policy == DW_POLICY_MLP) {                 // network actions from the observation of the current state, then replayed
-        rc = mlp_actions(h);
-        if (rc) return rc;
-    }
-    rc = ensure_grid(h);
-    if (rc) return rc;
-    if (policy == DW_POLICY_MLP) {
-        rc = launch_agents(h, h->action_dev, h->cfg.batch, h->cfg.n_agents, DW_POLICY_REPLAY, 0, false, false);
-    } else if (policy < 0) {
-        if (action) {
-            if (ab < 0 || am < 0 || ab > h->cfg.batch || am > h->cfg.n_agents)
-                return dw_fail(h, DW_E_INVALID, "dw_agents_begin", "action must be [ab<=B, am<=n]");
-            rc = stage_action(h, action, (size_t)ab * am);
-            if (rc) return rc;
-            rc = launch_agents(h, h->action_dev, ab, am, DW_POLICY_REPLAY, 0, false, false);
-        } else {
-            rc = launch_agents(h, nullptr, 0, 0, DW_POLICY_NONE, 0, false, false);
-        }
-    } else {
-        rc = launch_agents(h, nullptr, 0, 0, policy, seed, false, false);
-    }
+    StepActions sa;
+    int rc = resolve_actions(h, "dw_agents_begin", action, ab, am, policy, seed, &sa);
+    if (!rc) rc = ensure_grid(h);
+    if (!rc) rc = launch_agents(h, sa.act, sa.ab, sa.am, sa.policy, sa.seed, false, false);
     if (rc) return rc;
     h->agents_open = true;
     h->lat_valid = false;
@@ -737,25 +770,13 @@ extern "C" int dw_agents_collide(dw_handle *h, const double *noise, const int32_
     return DW_OK;
 }
 
-static int collect_step_outputs(dw_handle *h, double *obs, double *reward, uint8_t *done, dw_clock *clk);
-
-extern "C" int dw_step_tail_collect(dw_handle *h, double *obs, double *reward, uint8_t *done, dw_clock *clk) {
-    if (!h) return DW_E_INVALID;
-    DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (h->agents_open) return dw_fail(h, DW_E_STATE, "dw_step_tail_collect", "dw_agents_begin not closed by dw_agents_collide");
-    int rc = ensure_grid(h);
-    if (!rc) rc = launch_forward_tail(h, false, nullptr);
-    if (rc) return rc;
-    return collect_step_outputs(h, obs, reward, done, clk);
-}
-
 // The rest of step() after dw_agents_collide with the notebook's lifespan counters (done_at, agents_done_at) advanced like
 // dw_run does; *worlds_alive = worlds with max(grid[:,1:3]) > 0.005 after this step. Synchronises.
 extern "C" int dw_step_tail_counted(dw_handle *h, int64_t *worlds_alive) {
     if (!h) return DW_E_INVALID;
     DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (h->agents_open) return dw_fail(h, DW_E_STATE, "dw_step_tail_counted", "dw_agents_begin not closed by dw_agents_collide");
-    int rc = ensure_grid(h);
+    int rc = refuse_open(h, "dw_step_tail_counted");
+    if (!rc) rc = ensure_grid(h);
     if (rc) return rc;
     DW_CUDA_TRY(h, cudaMemsetAsync(h->alive, 0, sizeof(unsigned int), h->stream));
     rc = launch_forward_tail(h, true, h->alive);
@@ -765,37 +786,6 @@ extern "C" int dw_step_tail_counted(dw_handle *h, int64_t *worlds_alive) {
     DW_CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     if (worlds_alive) *worlds_alive = alive;
     return DW_OK;
-}
-
-extern "C" int dw_step(dw_handle *h, const int64_t *action, int32_t ab, int32_t am) {
-    if (!h) return DW_E_INVALID;
-    DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (h->agents_open) return dw_fail(h, DW_E_STATE, "dw_step", "dw_agents_begin not closed by dw_agents_collide");
-    const bool agents = h->cfg.n_agents > 0;
-    if (agents && action && (ab < 0 || am < 0 || ab > h->cfg.batch || am > h->cfg.n_agents))
-        return dw_fail(h, DW_E_INVALID, "dw_step", "action must be [ab<=B, am<=n]");
-    int rc = DW_OK;
-    if (lean_step_ok(h, action, ab, am)) {
-        if (agents && action) {
-            rc = stage_action(h, action, (size_t)ab * am);
-            if (rc) return rc;
-        }
-        CountLifeGuard guard(h, false);
-        return run_steps_fused(h, 1, (agents && action) ? DW_POLICY_REPLAY : DW_POLICY_NONE, h->action_dev, 0, h->alive);
-    }
-    rc = ensure_grid(h);
-    if (rc) return rc;
-    if (agents) {
-        if (action) {
-            rc = stage_action(h, action, (size_t)ab * am);
-            if (rc) return rc;
-            rc = launch_agents(h, h->action_dev, ab, am, DW_POLICY_REPLAY, 0);
-        } else {
-            rc = launch_agents(h, nullptr, 0, 0, DW_POLICY_NONE, 0);
-        }
-        if (rc) return rc;
-    }
-    return launch_forward_tail(h, false, nullptr);
 }
 
 static int mlp_upload(dw_handle *h, const double *params, int sets) {
@@ -869,30 +859,6 @@ static int mlp_actions(dw_handle *h) {
                                                                         h->pop_adversary);
     DW_LAUNCHED(h);
     return DW_OK;
-}
-
-extern "C" int dw_step_policy(dw_handle *h, int32_t policy, uint64_t seed) {
-    if (!h) return DW_E_INVALID;
-    DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (policy == DW_POLICY_REPLAY || policy < 0 || policy > DW_POLICY_MLP)
-        return dw_fail(h, DW_E_INVALID, "dw_step_policy", "use dw_step for explicit actions");
-    if (h->agents_open) return dw_fail(h, DW_E_STATE, "dw_step_policy", "dw_agents_begin not closed by dw_agents_collide");
-    int rc = DW_OK;
-    if (policy == DW_POLICY_MLP && h->cfg.n_agents > 0) {
-        rc = mlp_actions(h);
-        if (rc) return rc;
-    }
-    if (lean_step_ok(h, nullptr, 0, 0)) {
-        CountLifeGuard guard(h, false);
-        if (policy == DW_POLICY_MLP) return run_steps_fused(h, 1, h->cfg.n_agents ? DW_POLICY_REPLAY : DW_POLICY_NONE, h->action_dev, seed, h->alive);
-        return run_steps_fused(h, 1, policy, nullptr, seed, h->alive);
-    }
-    rc = ensure_grid(h);
-    if (rc) return rc;
-    if (policy == DW_POLICY_MLP) rc = launch_agents(h, h->action_dev, h->cfg.batch, h->cfg.n_agents, DW_POLICY_REPLAY, seed);
-    else rc = launch_agents(h, nullptr, 0, 0, policy, seed);
-    if (rc) return rc;
-    return launch_forward_tail(h, false, nullptr);
 }
 
 extern "C" int dw_forward(dw_handle *h, double *grid_in, double *grid_out) {
@@ -979,14 +945,6 @@ extern "C" int dw_get_obs(dw_handle *h, double *obs) {
     return DW_OK;
 }
 
-extern "C" int dw_step_collect(dw_handle *h, const int64_t *action, int32_t ab, int32_t am, int32_t policy, uint64_t seed, double *obs,
-                               double *reward, uint8_t *done, dw_clock *clk) {
-    if (!h) return DW_E_INVALID;
-    int rc = policy < 0 ? dw_step(h, action, ab, am) : dw_step_policy(h, policy, seed);
-    if (rc) return rc;
-    return collect_step_outputs(h, obs, reward, done, clk);
-}
-
 // ---- packed step: everything step() returns in ONE device->host copy ------------------------------------------------------
 extern "C" int dw_step_out_layout(dw_handle *h, int64_t *layout) {
     if (!h || !layout) return DW_E_INVALID;
@@ -997,20 +955,35 @@ extern "C" int dw_step_out_layout(dw_handle *h, int64_t *layout) {
     return DW_OK;
 }
 
-extern "C" int dw_step_packed(dw_handle *h, const int64_t *action, int32_t ab, int32_t am, int32_t policy, uint64_t seed,
-                              int32_t want_obs, void *out, dw_clock *clk) {
-    if (!h || !out) return DW_E_INVALID;
-    int rc = policy < 0 ? dw_step(h, action, ab, am) : dw_step_policy(h, policy, seed);
-    if (rc) return rc;
+// the output block of the step that just ran -> out (the reward | done part, or all of it with the observations), and the
+// clock after that step
+static int copy_step_outputs(dw_handle *h, int32_t want_obs, void *out, dw_clock *clk) {
     const bool obs = want_obs && h->cfg.n_agents > 0;
     if (obs) {
-        rc = compute_obs(h);
+        int rc = compute_obs(h);
         if (rc) return rc;
     }
     DW_CUDA_TRY(h, cudaMemcpyAsync(out, h->out_block, obs ? out_total(h) : out_obs_off(h), cudaMemcpyDeviceToHost, h->stream));
     DW_CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     if (clk) *clk = h->clk;
     return DW_OK;
+}
+
+extern "C" int dw_step_packed(dw_handle *h, const int64_t *action, int32_t ab, int32_t am, int32_t policy, uint64_t seed,
+                              int32_t want_obs, void *out, dw_clock *clk) {
+    if (!h || !out) return DW_E_INVALID;
+    DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    int rc = step_once(h, action, ab, am, policy, seed);
+    return rc ? rc : copy_step_outputs(h, want_obs, out, clk);
+}
+
+extern "C" int dw_step_tail_packed(dw_handle *h, int32_t want_obs, void *out, dw_clock *clk) {
+    if (!h || !out) return DW_E_INVALID;
+    DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    int rc = refuse_open(h, "dw_step_tail_packed");
+    if (!rc) rc = ensure_grid(h);
+    if (!rc) rc = launch_forward_tail(h, false, nullptr);
+    return rc ? rc : copy_step_outputs(h, want_obs, out, clk);
 }
 
 // Page-locked host memory for the packed outputs: a device->host copy into it is one DMA at PCIe rate with no staging
@@ -1024,39 +997,6 @@ extern "C" int dw_host_alloc(uint64_t bytes, void **out) {
 }
 extern "C" int dw_host_free(void *p) {
     if (p) cudaFreeHost(p);
-    return DW_OK;
-}
-
-static int collect_step_outputs(dw_handle *h, double *obs, double *reward, uint8_t *done, dw_clock *clk) {
-    int rc = DW_OK;
-    const size_t B = h->cfg.batch, n = h->cfg.n_agents;
-    const bool want_obs = obs && n;
-    if (want_obs) {
-        rc = compute_obs(h);
-        if (rc) return rc;
-    }
-    const size_t count = B * (n ? n : 2);
-    const size_t obs_bytes = want_obs ? B * n * 63 * sizeof(double) : 0, rew_bytes = reward ? count * sizeof(double) : 0,
-                 done_bytes = done ? count : 0;
-    if (obs_bytes + rew_bytes + done_bytes <= DW_PIN_OUT_MAX) {
-        // small batches (the reference's default 32 worlds): three enqueued copies into pinned staging, one synchronisation
-        rc = ensure_pinned(h);
-        if (rc) return rc;
-        unsigned char *po = h->pin + DW_PIN_ACTION_MAX, *pr = po + obs_bytes, *pd = pr + rew_bytes;
-        if (obs_bytes) DW_CUDA_TRY(h, cudaMemcpyAsync(po, h->obs, obs_bytes, cudaMemcpyDeviceToHost, h->stream));
-        if (rew_bytes) DW_CUDA_TRY(h, cudaMemcpyAsync(pr, h->reward, rew_bytes, cudaMemcpyDeviceToHost, h->stream));
-        if (done_bytes) DW_CUDA_TRY(h, cudaMemcpyAsync(pd, h->done, done_bytes, cudaMemcpyDeviceToHost, h->stream));
-        DW_CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-        if (obs_bytes) memcpy(obs, po, obs_bytes);
-        if (rew_bytes) memcpy(reward, pr, rew_bytes);
-        if (done_bytes) memcpy(done, pd, done_bytes);
-    } else {
-        if (want_obs) DW_CUDA_TRY(h, cudaMemcpyAsync(obs, h->obs, obs_bytes, cudaMemcpyDeviceToHost, h->stream));
-        if (reward) DW_CUDA_TRY(h, cudaMemcpyAsync(reward, h->reward, rew_bytes, cudaMemcpyDeviceToHost, h->stream));
-        if (done) DW_CUDA_TRY(h, cudaMemcpyAsync(done, h->done, done_bytes, cudaMemcpyDeviceToHost, h->stream));
-        DW_CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    }
-    if (clk) *clk = h->clk;
     return DW_OK;
 }
 
@@ -1273,16 +1213,6 @@ extern "C" int dw_get_agents(dw_handle *h, int64_t *agent_indices, double *agent
     if (agent_states) DW_CUDA_TRY(h, cudaMemcpyAsync(agent_states, h->agent_state, B * n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     DW_CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     if (agent_indices) for (size_t i = 0; i < xy.size(); ++i) agent_indices[i] = xy[i];
-    return DW_OK;
-}
-
-extern "C" int dw_get_reward_done(dw_handle *h, double *reward, uint8_t *done) {
-    if (!h) return DW_E_INVALID;
-    DW_CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    const size_t count = (size_t)h->cfg.batch * (h->cfg.n_agents ? h->cfg.n_agents : 2);
-    if (reward) DW_CUDA_TRY(h, cudaMemcpyAsync(reward, h->reward, count * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    if (done) DW_CUDA_TRY(h, cudaMemcpyAsync(done, h->done, count, cudaMemcpyDeviceToHost, h->stream));
-    DW_CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     return DW_OK;
 }
 

@@ -1,5 +1,5 @@
 // Materialising ("generic") kernels: one reference step on the fp64 grid[B,7,N,N], any N >= 1,
-// any (off-lattice) cover values.  Used by dw_step / dw_forward / dw_get_grid / dw_get_diag.
+// any (off-lattice) cover values.  Used by dw_step_packed / dw_forward / dw_get_grid / dw_get_diag.
 // Roofline: writes 6 live channels + reads 2 => 64 B per cell-update (SURVEY 8(d)); in literal
 // arithmetic (6 fp64 sqrt pairs, 7 fp64 divides per cell) it is fp64-pipe bound at about the same rate.
 #pragma once

@@ -653,14 +653,9 @@ class RLDaisyWorld:
         self._dead_L = self.L
         clk = DwClock()
         if self.collision_mode == 1 and n:
-            obs = np.empty((B, n, self.ch, 3, 3))
-            reward = np.empty((B, n, 1))
-            done = np.empty((B, n, 1), dtype=np.uint8)
             self._update_agents_colliding(a, policy, seed)
-            rc = self._lib.dw_step_tail_collect(self._h, _ptr(obs, C.c_double), _ptr(reward, C.c_double), _ptr(done, C.c_uint8),
-                                                C.byref(clk))
-            self._check(rc, "dw_step_tail_collect")
-            done = done.astype(bool)
+            ptr, obs, reward, done = self._out_views(True)       # the collision step returns the observation even without want_obs
+            self._check(self._lib.dw_step_tail_packed(self._h, 1, ptr, C.byref(clk)), "dw_step_tail_packed")
         else:
             ptr, obs, reward, done = self._out_views(want_obs)
             rc = self._lib.dw_step_packed(self._h, None if a is None else _ptr(a, C.c_int64), 0 if a is None else a.shape[0],
