@@ -24,6 +24,17 @@
  * gain[n] and act[n] are adjacent in memory (gain first): finishing step j can be deferred until the decisions of
  * step j + 1 exist, so that ONE all-reduce per step carries both (therldaisyworld_b200/banded.py does that).
  *
+ * Observations and DW_POLICY_MLP: once a step's agents are finished, dwt_observe writes the band's PARTIAL observation of
+ * the current state, obs[n, 7, 3, 3] -- step()'s obs[0] (daisy_world_rl.py:494) for the window cells in rows this band
+ * owns, 0 elsewhere -- into a device buffer (dwt_get_obs_ptr).  With several ranks the caller sums it across ranks (one
+ * non-zero term per element, like act); with one rank it is already the whole observation.  dwt_decide(DW_POLICY_MLP)
+ * then maps that buffer to every agent's action on every rank, so an MLP step needs no act exchange:
+ *
+ *   dwt_finish_agents (step j - 1) -> dwt_observe [ranks > 1: all-reduce SUM of obs] -> dwt_decide(DW_POLICY_MLP)
+ *   -> dwt_move_graze -> dwt_stencil ...
+ *
+ * Peer-memory mode (dwt_step_p2p) refuses DW_POLICY_MLP; dwt_observe works there after dwt_flush_p2p.
+ *
  * Constraints of the tiled kernels: N >= 64, 8 <= rows <= N, D4-symmetric kernels (the defaults). Bands may differ in
  * height; a side or band that is not a multiple of 64 runs a masked instance of the stencil kernel over its partial tiles.
  */
@@ -74,7 +85,9 @@ int dwt_upload_agents(dwt_handle *h, const int64_t *agent_indices, const double 
 int dwt_init_random(dwt_handle *h, uint64_t seed, double light_proportion, double dark_proportion, double initial_al,
                     double initial_ad);
 
-/* phases of one step (see the header comment). actions: host int8 [n] for DW_POLICY_REPLAY, else NULL. */
+/* phases of one step (see the header comment). actions: host int8 [n] for DW_POLICY_REPLAY, else NULL.
+   DW_POLICY_MLP reads the observation buffer: it needs dwt_set_mlp (else DW_E_STATE) and a dwt_observe since the last
+   change of state -- step phase, upload, reset, dwt_set_config (else DW_E_STATE). */
 int dwt_decide(dwt_handle *h, int32_t policy, const int8_t *actions, uint64_t seed);
 int dwt_move_graze(dwt_handle *h);
 int dwt_finish_agents(dwt_handle *h);
@@ -84,7 +97,21 @@ int dwt_get_ptrs(dwt_handle *h, dwt_ptrs *out);
 /* words per stored row: 64 * ceil(N / 64) + 8 (N + 8 when N is a multiple of 64), a multiple of 16 bytes */
 int dwt_get_pitch(const dwt_handle *h, int32_t *pitch);
 
-/* K whole steps on one rank (rows == N): the phases above back to back on the handle's stream, no host sync. */
+/* ---- observations and the MLP policy (see the header comment) ---------------------------------------------------------
+ * dwt_observe: the band's partial observation obs[n, 7, 3, 3] of the current state -> the device buffer, on the handle's
+ * stream. The window is the 3x3 around each agent's current position, all 7 channels (ch4: the state of the highest-index
+ * agent on the cell, dead agents included, after the step), times dw_config.obs_mask. Right after a reset, before any
+ * step, it shows initialize_grid's unrounded fields at the current L with no agent stamp. DW_E_STATE before any state
+ * exists, after dwt_debug_time_stencil (until the next step), and while a step's agents are not finished (between
+ * dwt_move_graze and dwt_finish_agents; in peer-memory mode until dwt_flush_p2p). The buffer is allocated on first use. */
+int dwt_observe(dwt_handle *h);
+int dwt_get_obs_ptr(dwt_handle *h, double **obs /* device [n, 7, 3, 3] */);
+int dwt_get_obs(dwt_handle *h, double *out /* host [n, 7, 3, 3] */);         /* synchronises */
+/* MLP.set_parameters (daisy/agents/mlp.py:130-147) for DW_POLICY_MLP: host double[DW_MLP_PARAMS], as dw_set_mlp */
+int dwt_set_mlp(dwt_handle *h, const double *parameters, int32_t n_parameters);
+
+/* K whole steps on one rank (rows == N): the phases above back to back on the handle's stream, no host sync.
+   DW_POLICY_MLP runs dwt_observe before each decision. */
 int dwt_run(dwt_handle *h, int64_t K, int32_t policy, const int8_t *actions /*[K,n] or NULL*/, uint64_t seed);
 /* Close a chunk of `K` steps whose per-step maxima sit in stepmax (all-reduced MAX over ranks by the caller when there
    are several): done_at += #steps whose max(light, dark) > 5 (notebook cell 2: grid_done = max <= 0.005);
@@ -123,6 +150,7 @@ int dwt_attach_peers(dwt_handle *h, int32_t rank, int32_t n_ranks, void *const *
    the bands differ in height: a band writes its last row into the ghost row below its upper neighbour's band. Without
    it, attaching assumes equal bands and refuses with DW_E_STATE when rows * n_ranks != N. */
 int dwt_set_peer_rows(dwt_handle *h, int32_t n_ranks, const int32_t *rows);
+/* DW_POLICY_MLP: DW_E_UNSUPPORTED, before anything is launched */
 int dwt_step_p2p(dwt_handle *h, int32_t policy, const int8_t *actions /* [n] or NULL */, uint64_t seed);
 int dwt_flush_p2p(dwt_handle *h);                       /* finish the agents of the last step */
 int dwt_peer_status(dwt_handle *h, int32_t *timed_out); /* 1 if a barrier gave up waiting for a peer */

@@ -53,6 +53,7 @@ TILED_SYMBOLS = [
     "dwt_reset_lifespans", "dwt_get_lifespans", "dwt_get_agents", "dwt_get_reward_done", "dwt_get_covers", "dwt_get_grid",
     "dwt_debug_slow_count", "dwt_debug_time_stencil", "dwt_cover_checksum", "dwt_ipc_export", "dwt_ipc_attach", "dwt_get_peer_buffers", "dwt_attach_peers", "dwt_step_p2p",
     "dwt_flush_p2p", "dwt_peer_status", "dwt_set_series", "dwt_get_series_ptr", "dwt_get_series", "dwt_get_pitch", "dwt_set_peer_rows",
+    "dwt_observe", "dwt_get_obs_ptr", "dwt_get_obs", "dwt_set_mlp",
 ]
 
 
@@ -186,6 +187,10 @@ def load():
         "dwt_get_series": (C.c_int, [vp, i32, pd]),
         "dwt_get_pitch": (C.c_int, [vp, pi32]),
         "dwt_set_peer_rows": (C.c_int, [vp, i32, pi32]),
+        "dwt_observe": (C.c_int, [vp]),
+        "dwt_get_obs_ptr": (C.c_int, [vp, C.POINTER(vp)]),
+        "dwt_get_obs": (C.c_int, [vp, pd]),
+        "dwt_set_mlp": (C.c_int, [vp, pd, i32]),
     }
     assert set(tsig) == set(TILED_SYMBOLS)
     sig.update(tsig)

@@ -13,7 +13,10 @@ NCCL over NVLink on GPUs, gloo in the CPU tests -- plumbing only, the data path 
   * after the edge tile rows of the stencil: the band's first/last row goes to the upper/lower neighbour's ghost row
     (ring, toroidal) on a side stream while the interior tile rows are still being computed;
   * per chunk of steps: MAX all-reduce of the per-step cover maxima (lifespan bookkeeping, ``grid_done``), and in
-    ``run_series`` a SUM all-reduce of the per-step temperature and cover sums next to it.
+    ``run_series`` a SUM all-reduce of the per-step temperature and cover sums next to it;
+  * ``observe()`` and every ``policy="mlp"`` step: a SUM all-reduce of the bands' partial observations ``[n, 7, 3, 3]``
+    (the band that owns a window cell's row evaluates it, every other band contributes 0). An MLP step then decides on
+    every rank from the same observation and needs no act exchange: two collectives per step (gain, obs).
 
 ``world_size == 1`` needs none of them (``dwt_halo_wrap`` closes the torus locally).
 
@@ -161,6 +164,25 @@ class DeviceBand:
 
     def move_graze(self):
         self._check(self._lib.dwt_move_graze(self._h), "dwt_move_graze")
+
+    def observe(self):
+        """The band's partial observation of the current state into the device buffer (dwt_observe)."""
+        self._check(self._lib.dwt_observe(self._h), "dwt_observe")
+
+    def obs_tensor(self):
+        """The device observation buffer [n, 7, 3, 3] as a torch view (summed over the ranks in place by the caller)."""
+        p = C.c_void_p()
+        self._check(self._lib.dwt_get_obs_ptr(self._h, C.byref(p)), "dwt_get_obs_ptr")
+        return self._view(p.value, (max(self.n, 1), 7, 3, 3), "<f8")[:self.n]
+
+    def get_obs(self):
+        out = np.zeros((self.n, 7, 3, 3))
+        self._check(self._lib.dwt_get_obs(self._h, out.ctypes.data_as(C.POINTER(C.c_double))), "dwt_get_obs")
+        return out
+
+    def set_mlp(self, params):
+        p = np.ascontiguousarray(params, dtype=np.float64).ravel()
+        self._check(self._lib.dwt_set_mlp(self._h, p.ctypes.data_as(C.POINTER(C.c_double)), int(p.size)), "dwt_set_mlp")
 
     def finish_agents(self):
         self._check(self._lib.dwt_finish_agents(self._h), "dwt_finish_agents")
@@ -405,14 +427,22 @@ class BandedDaisyWorld:
         self._reset_clock()
         self.band.init_random(seed, self)
 
+    def set_mlp(self, params):
+        """MLP.set_parameters (daisy/agents/mlp.py) for policy="mlp": 1808 weights, flat layout of MLP.get_parameters."""
+        self.band.set_mlp(params)
+
     # ---- stepping
     def step(self, policy="greedy", actions_step=None, seed=0):
+        """One env step with a device policy ("greedy", "antigreedy", "eps_greedy", "random", "none", "mlp") or "replay"
+        of actions_step [n]. "mlp" is not available in p2p mode (raises before the step)."""
         b, comm = self.band, self.comm
         if self.mode == "p2p":
             b.step_p2p(policy, actions_step, seed)
             self._gain_pending = bool(self.n_agents)
             self._pending += 1
             return
+        if policy == "mlp":
+            self._observe_device()                   # finishes step j-1 first; every rank then decides on the same obs
         b.decide(policy, actions_step, seed)
         if comm is None:
             b.move_graze()
@@ -452,6 +482,51 @@ class BandedDaisyWorld:
                 self.comm.all_reduce_sum(self.band.exch_tensor(gain=True, act=False))
                 self.band.finish_agents()
             self._gain_pending = False
+
+    def _observe_device(self):
+        """The whole observation of the current state in the band's device buffer, on every rank: the agents' states must
+        be final (the stamp of ch4), then the partial observations are summed over the ranks."""
+        self._flush()
+        self.band.observe()
+        if self.comm is not None:
+            # p2p mode: the pre-state's ghost rows read here are overwritten by the neighbours' halo push of the NEXT step;
+            # this all-reduce completes on every rank only after every rank's observation, and before any of them can
+            # issue that step
+            self.comm.all_reduce_sum(self.band.obs_tensor())
+
+    def observe(self):
+        """obs[1, n, 7, 3, 3] of the current state: what the reference's step() returned for it (the 3x3 windows around
+        the agents, all channels, times the neighbourhood mask), or after a reset its observation of the reset state.
+        Every rank returns the same array."""
+        if not self.n_agents:
+            return np.zeros((1, 0, 7, 3, 3))
+        self._observe_device()
+        obs = self.band.get_obs()[None]
+        self._check_peers()
+        return obs
+
+    def env_step(self, action=None):
+        """The reference's step(action) for batch 1: (obs [1, n, 7, 3, 3], reward, done, {}). action: n integers 0..8 as
+        [n], [1, n] or [1, n, 1]; None is the reference's all-zero action. reward / done are [1, n, 1] (the agents' states,
+        state < 0.1), or with no agents [1, 2] (any light / dark cover left, and its negation)."""
+        n = self.n_agents
+        if action is not None:
+            a = np.asarray(action)
+            if a.shape not in ((n,), (1, n), (1, n, 1)) or (a.size and not np.issubdtype(a.dtype, np.integer)):
+                raise ValueError(f"action must be n={n} integers as [n], [1, n] or [1, n, 1]; got shape {a.shape}, dtype {a.dtype}")
+            if a.size and (a.min() < 0 or a.max() > 8):
+                raise ValueError("actions must be in 0..8")
+            self.step("replay", a.reshape(n))
+        else:
+            self.step("none")
+        obs = self.observe()
+        if n:
+            reward = self.band.agents()[1].reshape(1, n, 1).copy()
+            reward = reward * (reward > 0)
+        else:
+            cs = self.cover_checksum()
+            reward = np.array([[cs[0] > 0, cs[1] > 0]])
+        return obs, reward, reward < 0.1, {}
 
     def end_chunk(self):
         """Fold the per-step cover maxima of the steps since the last call into the lifespan counter."""

@@ -856,6 +856,57 @@ __global__ void __launch_bounds__(256) k_band_stamp_write(BandGeom G, const int3
     else claim[c] = 0x7fffffff;
 }
 
+// ---- observations (step()'s obs[0], daisy_world_rl.py:246-263, 494) ----------------------------------------------------
+// The band's PARTIAL observation obs[n, 7, 3, 3]: one thread per (agent, window cell). A window cell whose row this band
+// owns is evaluated whole, as k_obs_from_pre does it (screened, literal next to ties: what forward stored there), from the
+// post-graze pre-state at SL = S * L_last; every other cell is 0. A ghost-row cell would need a pre-state row two away from
+// the band, which is stored nowhere, so the owner always evaluates: the partial observations of all bands add up to the
+// whole one with exactly one non-zero term per element (a caller with several bands sums them, like act).
+// ch4 carries the agent stamp (highest index on the cell, dead agents included) from `claim`, filled by k_band_stamp_claim
+// (n - 1 - i, smallest wins); a value >= n is idle.
+// init != 0: the state right after a reset -- `pre` holds the reset covers themselves, SL = S * L, and the window shows
+// initialize_grid's unrounded fields (no stamp; daisy_world_rl.py:304-324), like the init branch of k_obs_from_pre.
+template <class Pre>
+__global__ void __launch_bounds__(256) k_band_obs(DevParams P, double SL, BandGeom G, Pre pre, const int32_t *__restrict__ xy,
+                                                  const double *__restrict__ st, int n, const int *__restrict__ claim,
+                                                  double *__restrict__ obs, int init) {
+    const size_t total = (size_t)n * 9;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t ag = i / 9;
+        const int w = (int)(i - ag * 9);
+        double *o = obs + ag * 63 + w;
+        int x = xy[2 * ag] + w / 3 - 1, y = xy[2 * ag + 1] + w % 3 - 1;
+        x = x < 0 ? x + G.N : (x >= G.N ? x - G.N : x);
+        y = y < 0 ? y + G.N : (y >= G.N ? y - G.N : y);
+        const int lr = band_owned_row(G, x);
+        if (lr < 0) {
+#pragma unroll
+            for (int ch = 0; ch < 7; ++ch) o[9 * ch] = 0.0;
+            continue;
+        }
+        const double mk = P.mask[w];
+        double l9[9], d9[9];
+        pre.load9(G, lr - 1, y, l9, d9);
+        if (init) {
+            const LitCell c = dw_literal_cell(P, SL, l9, d9);
+            o[0] = c.b0 * mk; o[9] = l9[4] * mk; o[18] = d9[4] * mk; o[27] = c.T * mk; o[36] = c.Tl * mk; o[45] = c.Td * mk;
+            o[54] = 0.0 * mk;
+            continue;
+        }
+        ScrCell c;
+        if (!(P.screen && dw_screened_cell(P, SL / P.sigma, l9, d9, c))) dw_literal_rounded(P, SL, l9, d9, c);
+        const int s = claim[(size_t)lr * G.N + y];
+        const double ch4 = (s >= 0 && s < n) ? st[n - 1 - s] : dw_k2v(c.k[4]);
+        o[0] = dw_k2v(c.k[0]) * mk;
+        o[9] = dw_k2v(c.k[1]) * mk;
+        o[18] = dw_k2v(c.k[2]) * mk;
+        o[27] = dw_k2v(c.k[3]) * mk;
+        o[36] = ch4 * mk;
+        o[45] = dw_k2v(c.k[5]) * mk;
+        o[54] = 0.0 * mk;
+    }
+}
+
 // device-side synthetic reset of the band (+ its ghost rows) and of the replicated agents: same distribution as
 // initialize_grid / initialize_agents (daisy_world_rl.py:285-302, 173-179), counter RNG keyed by the GLOBAL cell index,
 // so any banding of the same world draws the same state.

@@ -7,6 +7,11 @@ alternating, five repetitions each (optional argument: N, default 16384).
 alternating over five repetitions; the rates are reported against the first side. Sides that are not a multiple of 64 run
 the masked instance of the stencil kernel over their partial tiles.
 
+--policy mlp [N]: the MLP policy on the giant world (default N = 16384, N agents, golden weights): whole steps with greedy and
+with mlp decisions (dwt_run; an mlp step also observes), alternating over five repetitions; the latency of observe() (host
+clock, download included) and of the device observation alone (CUDA events); and the mean time per launch of each kernel
+of an mlp step from torch.profiler (k_band_obs, k_mlp_act, ...), in a separate profiled run.
+
 --vs-ensemble N: whole greedy steps of one N x N world as the giant world (BandedDaisyWorld.run) and as an ensemble of one
 (RLDaisyWorld, batch_size = 1, run()), 4 agents like RLDaisyWorld's default, alternating over five repetitions."""
 import sys, os, subprocess, time
@@ -105,6 +110,63 @@ def bench_sides(sides, K=64, reps=5, stencil_reps=50):
               f"cell-updates/s, {rate(N, mt) / rate(base, np.median(step[base])):.4f} of N={base}", flush=True)
 
 
+def bench_mlp(N, K=64, reps=5):
+    from torch.profiler import ProfilerActivity, profile
+    params = np.load(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden",
+                                  "mlp_n16_b4_mixed_150.npz"))["mlp_params"]
+    w = BandedDaisyWorld(N, N)
+    w.set_mlp(params)
+    w.reset_on_device(seed=1)
+    w.run(2, "mlp")
+    w.run(2, "greedy")
+
+    def timed(fn):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        torch.cuda.synchronize()
+        e0.record()
+        fn()
+        e1.record()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) * 1e3
+
+    steps = {"greedy": [], "mlp": []}
+    for _ in range(reps):
+        for pol in steps:
+            steps[pol].append(timed(lambda: w.band.run_local(K, pol)) / K)
+            w._pending += K
+            w.end_chunk()
+    obs_host, obs_dev, decide = [], [], []
+    for _ in range(reps):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        o = w.observe()
+        obs_host.append((time.perf_counter() - t0) * 1e6)
+        obs_dev.append(timed(lambda: [w.band.observe() for _ in range(20)]) / 20)
+        decide.append(timed(lambda: [w.band.decide("mlp") for _ in range(20)]) / 20)
+    assert o.shape == (1, N, 7, 3, 3)
+    print(f"N={N}, {N} agents, K={K} steps per arm (dwt_run), {reps} alternating repetitions, golden MLP weights")
+    for pol, ts in steps.items():
+        print(f"  {pol:6s} us/step: " + " ".join(f"{t:.1f}" for t in ts) + f" | median {np.median(ts):.1f}")
+    print(f"  mlp - greedy: {np.median(steps['mlp']) - np.median(steps['greedy']):+.1f} us/step "
+          f"({100.0 * (np.median(steps['mlp']) / np.median(steps['greedy']) - 1.0):+.2f} %)")
+    print("  observe() us (host clock, obs download included): " + " ".join(f"{t:.0f}" for t in obs_host) +
+          f" | median {np.median(obs_host):.0f}")
+    print("  dwt_observe us (events, stamp claim + k_band_obs + claim reset): " + " ".join(f"{t:.1f}" for t in obs_dev) +
+          f" | median {np.median(obs_dev):.1f}")
+    print("  dwt_decide(mlp) us (events, k_mlp_act + k_band_decide): " + " ".join(f"{t:.1f}" for t in decide) +
+          f" | median {np.median(decide):.1f}")
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        w.band.run_local(16, "mlp")
+        torch.cuda.synchronize()
+    w._pending += 16
+    w.end_chunk()
+    print("  kernels of 16 mlp steps (torch.profiler, separate run): mean us per launch x launches")
+    for ev in sorted(prof.key_averages(), key=lambda e: -e.device_time_total):
+        if ev.device_time_total > 0 and ev.count > 0:
+            print(f"    {ev.key[:60]:60s} {ev.device_time_total / ev.count:9.1f} x {ev.count}")
+    sys.stdout.flush()
+
+
 def bench_vs_ensemble(N, K=200, reps=5):
     from therldaisyworld_b200 import RLDaisyWorld
     n = 4
@@ -140,6 +202,12 @@ if __name__ == "__main__":
             bench_sides(args)
         else:
             bench_vs_ensemble(args[0])
+        sys.exit(0)
+    if "--policy" in sys.argv:
+        args = [a for a in sys.argv[1:] if not a.startswith("--")]
+        assert args and args[0] == "mlp", "--policy mlp [N]"
+        print(f"GPU: {gpu_label()}")
+        bench_mlp(int(args[1]) if len(args) > 1 else 16384)
         sys.exit(0)
     if "--series" in sys.argv:
         args = [a for a in sys.argv[1:] if a != "--series"]
