@@ -15,7 +15,8 @@
  *                     [ranks > 1 and greedy/antigreedy: all-reduce SUM of act]
  *   dwt_move_graze    update_agents (:181-216): pay agent_gamma, move, graze in agent-index order -> gain[n]
  *                     [ranks > 1: all-reduce SUM of gain]
- *   dwt_finish_agents state += gain, clip (:244), reward/done (:486-492), agents_done_at += !done
+ *   dwt_finish_agents state += gain, clip (:244), agents_done_at += !done; reward and done (:486-492) follow from
+ *                     the states (dwt_get_agents)
  *   dwt_stencil       forward (:434-452) on the band -> new covers (ghost columns included); update_L (:463-473);
  *                     per-step species max. Parts 1 + 2 split it into edge tile rows and interior so that the
  *                     halo exchange can overlap the interior.
@@ -157,7 +158,6 @@ int dwt_peer_status(dwt_handle *h, int32_t *timed_out); /* 1 if a barrier gave u
 
 /* getters (synchronise) */
 int dwt_get_agents(dwt_handle *h, int64_t *agent_indices, double *agent_states);
-int dwt_get_reward_done(dwt_handle *h, double *reward, uint8_t *done);          /* [n] */
 int dwt_get_covers(dwt_handle *h, double *light, double *dark);                 /* band rows, [rows, N] each */
 /* env.grid of the band: [7, rows, N] (channels as in the reference; ch4 carries the agent stamp), materialised by a
    literal forward from the post-graze state the last step started from. Needs at least one step. */

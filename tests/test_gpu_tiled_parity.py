@@ -80,13 +80,15 @@ def test_bands_on_one_gpu_match_oracle(bands, policy):
 
 
 @pytest.mark.parametrize("bands,policy,n", [(2, "greedy", 200), (4, "antigreedy", 200), (4, "replay", 200), (2, "none", 200),
-                                            (2, "greedy", 900), (4, "antigreedy", 1500)])
+                                            (2, "greedy", 900), (4, "antigreedy", 1500), (2, "greedy", "sms+1")])
 def test_peer_memory_mode_bands_on_one_gpu(bands, policy, n):
     """dwt_step_p2p: owners publish decisions / gains into every band's exchange vector, edge rows are pushed into the
     neighbours' ghost rows, bands meet at device-side flag barriers. Here the 'peers' are bands of one process on one GPU,
     each on its own stream (the IPC variant of the same code path runs in tools/banded_nccl_check.py)."""
     import torch
     N, steps = 256, 30               # n > 256: several blocks in the agent kernels (grid barrier of k_band_fmc_graze)
+    if n == "sms+1":                 # one block more than there are SMs: move/claim and graze as two launches on the lattice
+        n = 256 * torch.cuda.get_device_properties(0).multi_processor_count + 1
     light, dark, ai, st = make_state(N, n, seed=17, clustered=True)
     ai[n // 2:, 0] = (ai[n // 2:, 0] + N // bands) % N
     shared = ThreadComm.Shared(bands)

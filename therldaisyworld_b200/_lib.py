@@ -50,7 +50,7 @@ TILED_SYMBOLS = [
     "dwt_last_error", "dwt_create", "dwt_destroy", "dwt_set_config", "dwt_set_clock", "dwt_get_clock", "dwt_set_stream", "dwt_set_epsilon",
     "dwt_synchronize", "dwt_upload_covers", "dwt_upload_agents", "dwt_init_random", "dwt_decide", "dwt_move_graze",
     "dwt_finish_agents", "dwt_stencil", "dwt_halo_wrap", "dwt_get_ptrs", "dwt_run", "dwt_end_chunk",
-    "dwt_reset_lifespans", "dwt_get_lifespans", "dwt_get_agents", "dwt_get_reward_done", "dwt_get_covers", "dwt_get_grid",
+    "dwt_reset_lifespans", "dwt_get_lifespans", "dwt_get_agents", "dwt_get_covers", "dwt_get_grid",
     "dwt_debug_slow_count", "dwt_debug_time_stencil", "dwt_cover_checksum", "dwt_ipc_export", "dwt_ipc_attach", "dwt_get_peer_buffers", "dwt_attach_peers", "dwt_step_p2p",
     "dwt_flush_p2p", "dwt_peer_status", "dwt_set_series", "dwt_get_series_ptr", "dwt_get_series", "dwt_get_pitch", "dwt_set_peer_rows",
     "dwt_observe", "dwt_get_obs_ptr", "dwt_get_obs", "dwt_set_mlp",
@@ -169,7 +169,6 @@ def load():
         "dwt_reset_lifespans": (C.c_int, [vp]),
         "dwt_get_lifespans": (C.c_int, [vp, pi64, pi64]),
         "dwt_get_agents": (C.c_int, [vp, pi64, pd]),
-        "dwt_get_reward_done": (C.c_int, [vp, pd, pu8]),
         "dwt_get_covers": (C.c_int, [vp, pd, pd]),
         "dwt_get_grid": (C.c_int, [vp, pd]),
         "dwt_debug_slow_count": (C.c_int, [vp, C.POINTER(u64)]),

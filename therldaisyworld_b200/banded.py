@@ -9,7 +9,7 @@ NCCL over NVLink on GPUs, gloo in the CPU tests -- plumbing only, the data path 
 
   * ONE SUM all-reduce per step over ``[gain(j-1) | act(j)]``: only the owner band of a cell knows what was eaten there,
     only the owner band of an agent sees its neighbourhood (greedy / anti-greedy).  Finishing step j-1 (state += gain,
-    clip, reward/done) is deferred until the decisions of step j exist, so both vectors travel together;
+    clip, lifespan counter) is deferred until the decisions of step j exist, so both vectors travel together;
   * after the edge tile rows of the stencil: the band's first/last row goes to the upper/lower neighbour's ghost row
     (ring, toroidal) on a side stream while the interior tile rows are still being computed;
   * per chunk of steps: MAX all-reduce of the per-step cover maxima (lifespan bookkeeping, ``grid_done``), and in
@@ -155,12 +155,21 @@ class DeviceBand:
         self._views = {}
 
     # ---- phases
+    def _replay_ptr(self, policy, actions, K=None):
+        """The host int8 actions of a replay as dwt_decide / dwt_step_p2p ([n]) or dwt_run (K steps: [K, n]) take them;
+        None for every other policy."""
+        if policy != "replay":
+            return None
+        if K is None:
+            a = np.asarray(actions).reshape(self.n)
+        else:
+            a = np.asarray(actions).reshape(-1, self.n)[:K]
+            assert a.shape[0] == K
+        return np.ascontiguousarray(a, dtype=np.int8).ctypes.data_as(C.POINTER(C.c_int8))
+
     def decide(self, policy, actions_step=None, seed=0):
-        a = None
-        if policy == "replay":
-            a = np.ascontiguousarray(np.asarray(actions_step).reshape(self.n), dtype=np.int8)
-        self._check(self._lib.dwt_decide(self._h, DW_POLICY[policy], None if a is None else a.ctypes.data_as(C.POINTER(C.c_int8)),
-                                         C.c_uint64(seed)), "dwt_decide")
+        self._check(self._lib.dwt_decide(self._h, DW_POLICY[policy], self._replay_ptr(policy, actions_step), C.c_uint64(seed)),
+                    "dwt_decide")
 
     def move_graze(self):
         self._check(self._lib.dwt_move_graze(self._h), "dwt_move_graze")
@@ -241,11 +250,8 @@ class DeviceBand:
         self._check(self._lib.dwt_attach_peers(self._h, int(rank), len(tables), flat), "dwt_attach_peers")
 
     def step_p2p(self, policy, actions_step=None, seed=0):
-        a = None
-        if policy == "replay":
-            a = np.ascontiguousarray(np.asarray(actions_step).reshape(self.n), dtype=np.int8)
-        self._check(self._lib.dwt_step_p2p(self._h, DW_POLICY[policy], None if a is None else a.ctypes.data_as(C.POINTER(C.c_int8)),
-                                           C.c_uint64(seed)), "dwt_step_p2p")
+        self._check(self._lib.dwt_step_p2p(self._h, DW_POLICY[policy], self._replay_ptr(policy, actions_step), C.c_uint64(seed)),
+                    "dwt_step_p2p")
 
     def flush_p2p(self):
         self._check(self._lib.dwt_flush_p2p(self._h), "dwt_flush_p2p")
@@ -267,12 +273,8 @@ class DeviceBand:
 
     def run_local(self, K, policy, actions=None, seed=0):
         """K steps without any exchange (a band that is the whole torus)."""
-        a = None
-        if policy == "replay":
-            a = np.ascontiguousarray(np.asarray(actions).reshape(-1, self.n)[:K], dtype=np.int8)
-            assert a.shape[0] == K
-        self._check(self._lib.dwt_run(self._h, int(K), DW_POLICY[policy], None if a is None else a.ctypes.data_as(C.POINTER(C.c_int8)),
-                                      C.c_uint64(seed)), "dwt_run")
+        self._check(self._lib.dwt_run(self._h, int(K), DW_POLICY[policy], self._replay_ptr(policy, actions, K), C.c_uint64(seed)),
+                    "dwt_run")
 
     def set_series(self, on):
         """Series mode: every step also sums sqrt(g)*T and the new milli-covers of the band's cells (dwt_set_series)."""
@@ -341,14 +343,6 @@ class DeviceBand:
             self._check(self._lib.dwt_get_agents(self._h, ai.ctypes.data_as(C.POINTER(C.c_int64)), st.ctypes.data_as(C.POINTER(C.c_double))),
                         "dwt_get_agents")
         return ai, st
-
-    def reward_done(self):
-        r = np.zeros((self.n,), dtype=np.float64)
-        d = np.zeros((self.n,), dtype=np.uint8)
-        if self.n:
-            self._check(self._lib.dwt_get_reward_done(self._h, r.ctypes.data_as(C.POINTER(C.c_double)), d.ctypes.data_as(C.POINTER(C.c_uint8))),
-                        "dwt_get_reward_done")
-        return r, d.astype(bool)
 
     def covers(self):
         out = np.empty((2, self.rows, self.N))

@@ -61,15 +61,37 @@ __device__ __forceinline__ int band_owned_row(const BandGeom &G, int x) {
 }
 
 // ---- cell accessors: packed lattice (steady state) or fp64 cover planes (the off-lattice state right after reset) ----
+// load9: the covers of the 3x3 window around band row r (stored rows r .. r+2), column y
 struct LatCells {
     uint32_t *p;
     __device__ __forceinline__ double food(size_t i) const { return dw_food(p[i]); }
     __device__ __forceinline__ void zero(size_t i) const { p[i] = 0u; }
+    __device__ __forceinline__ void load9(const BandGeom &G, int r, int y, double (&l9)[9], double (&d9)[9]) const {
+#pragma unroll
+        for (int a = 0; a < 3; ++a)
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const uint32_t w = p[(size_t)(r + a) * G.pitch + G.c0 + y + c - 1];
+                l9[a * 3 + c] = dw_milli(w & 0xffffu);
+                d9[a * 3 + c] = dw_milli(w >> 16);
+            }
+    }
 };
 struct PlaneCells {
     double *l, *d;
     __device__ __forceinline__ double food(size_t i) const { return l[i] + d[i]; }
     __device__ __forceinline__ void zero(size_t i) const { l[i] = 0.0; d[i] = 0.0; }
+    __device__ __forceinline__ void load9(const BandGeom &G, int r, int y, double (&l9)[9], double (&d9)[9]) const {
+        const int ys[3] = {y == 0 ? G.N - 1 : y - 1, y, y == G.N - 1 ? 0 : y + 1};
+#pragma unroll
+        for (int a = 0; a < 3; ++a)
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const size_t k = (size_t)(r + a) * G.pitch + ys[c];
+                l9[a * 3 + c] = l[k];
+                d9[a * 3 + c] = d[k];
+            }
+    }
 };
 // column index with toroidal wrap for planes without column ghosts
 __device__ __forceinline__ int band_col(const BandGeom &G, int y) {
@@ -180,16 +202,13 @@ __global__ void __launch_bounds__(256) k_band_decide(BandGeom G, Cells C, const 
     if (epoch) dw_last_block_barrier(PT, epoch, timed_out, ticket);     // peer-memory mode, world-reading policies
 }
 
-// Phase 2 (replicated on every rank): pay agent_gamma, move the living, and file the graze claims of cells this band owns.
-// gz[i] = 1 if agent i grazes this step.
-__global__ void __launch_bounds__(256) k_band_move_claim(BandGeom G, double agent_gamma, int32_t *xy, double *st, int n,
-                                                         const double *__restrict__ act, int *claim, uint8_t *gz) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+// Phase 2 of agent i with state s at (x, y) (replicated on every rank): pay agent_gamma, move if still alive, and file the
+// graze claim of a cell this band owns. x, y become the new position; gz[i] = 1 (returned) if the agent grazes this step.
+__device__ __forceinline__ uint8_t dwt_move_claim_agent(const BandGeom &G, double agent_gamma, int32_t *xy, double *st, double s, int &x,
+                                                        int &y, const double *__restrict__ act, int *claim, uint8_t *gz, int i) {
     const int a = (int)act[i] - 1;
-    const double s = st[i] - agent_gamma;
+    s = s - agent_gamma;
     st[i] = s;
-    int x = xy[2 * i], y = xy[2 * i + 1];
     uint8_t g = 0;
     if (s > 0.0) {
         if (a != 8) {
@@ -206,55 +225,60 @@ __global__ void __launch_bounds__(256) k_band_move_claim(BandGeom G, double agen
         }
     }
     gz[i] = g;
+    return g;
 }
 
-// Peer-memory mode: phase 4 of step j-1 and phase 2 of step j in one launch (the finish is deferred until the gains are
-// known to be complete, i.e. after the closing barrier of step j-1). The two steps use different claim arrays (step
-// parity), so returning step j-1's claims to "idle" cannot collide with step j's atomicMin on the same cell.
-__global__ void __launch_bounds__(256) k_band_finish_move_claim(BandGeom G, double agent_gamma, int32_t *xy, double *st, int n,
-                                                                const double *__restrict__ act, int *claim_new, uint8_t *gz, int do_finish,
-                                                                double *gain_prev, int *claim_prev, double *reward, uint8_t *done,
-                                                                int64_t *agents_done_at) {
+// Phase 3 of grazing agent i at (x, y): the claim winner of an owned cell eats it and clears every stored copy; a graze that
+// lands in a ghost row only clears the ghost copy (the owner rank does the eating). claim_at(k) loads claim[k] the way the
+// caller needs it. The winner sets won and got = the food it eats on THIS rank; both are left alone otherwise.
+template <class Cells, class ClaimAt>
+__device__ __forceinline__ void dwt_graze_agent(const BandGeom &G, const Cells &C, int x, int y, ClaimAt claim_at, int i, double &got,
+                                                bool &won) {
+    const int lr = band_owned_row(G, x);
+    bool clear = true;
+    if (lr >= 0) {
+        if (claim_at((size_t)lr * G.N + y) == i) { got = C.food((size_t)lr * G.pitch + G.c0 + y); won = true; }
+        else clear = false;                              // a lower-index agent eats here; it also does the clearing
+    }
+    if (clear)
+        band_row_images(G, x, [&](int r) { band_col_images(G, y, [&](int cc) { C.zero((size_t)r * G.pitch + cc); }); });
+}
+
+// Phase 4 of agent i with state s at (x, y), the cell it grazed (replicated, after the gains were summed over ranks):
+// state += gain if it grazed, its claim back to "idle", clip, lifespan counter. Returns the new state.
+// zero_gain: peer-memory mode, where only the winners write the gain vector, so it is re-armed here.
+__device__ __forceinline__ double dwt_finish_agent(const BandGeom &G, int x, int y, double s, double *gain, bool zero_gain,
+                                                   const uint8_t *gz, int *claim, int64_t *agents_done_at, int i) {
+    const double g = gain[i];
+    if (zero_gain) gain[i] = 0.0;
+    if (gz[i]) {
+        s = s + g;
+        const int lr = band_owned_row(G, x);
+        if (lr >= 0) claim[(size_t)lr * G.N + y] = 0x7fffffff;
+    }
+    s = dw_clip01(s);
+    agents_done_at[i] += (s < 0.1) ? 0 : 1;
+    return s;
+}
+
+// Phase 2 (replicated on every rank), in peer-memory mode preceded by phase 4 of the previous step (do_finish: its gains
+// are complete since its closing barrier). The two steps use different claim arrays there (step parity), so returning
+// step j-1's claims to "idle" cannot collide with step j's atomicMin on the same cell. Phase-by-phase and NCCL mode have
+// one claim array and finish with k_band_finish instead (do_finish = 0): merged, the return of step j-1's claims would race
+// with step j's claims in the same launch.
+__global__ void __launch_bounds__(256) k_band_move_claim(BandGeom G, double agent_gamma, int32_t *xy, double *st, int n,
+                                                         const double *__restrict__ act, int *claim, uint8_t *gz, int do_finish,
+                                                         double *gain_prev, int *claim_prev, int64_t *agents_done_at) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     double s = st[i];
     int x = xy[2 * i], y = xy[2 * i + 1];
-    if (do_finish) {
-        const double g = gain_prev[i];
-        gain_prev[i] = 0.0;
-        if (gz[i]) {
-            s = s + g;
-            const int lr = band_owned_row(G, x);
-            if (lr >= 0) claim_prev[(size_t)lr * G.N + y] = 0x7fffffff;
-        }
-        s = dw_clip01(s);
-        reward[i] = s;
-        done[i] = s < 0.1;
-        agents_done_at[i] += (s < 0.1) ? 0 : 1;
-    }
-    const int a = (int)act[i] - 1;
-    s = s - agent_gamma;
-    st[i] = s;
-    uint8_t g = 0;
-    if (s > 0.0) {
-        if (a != 8) {
-            const int d = (a & 2) ? 1 : -1;
-            if (((a + 1) & 2) == 0) { y += d; y = y < 0 ? y + G.N : (y >= G.N ? y - G.N : y); }
-            else { x += d; x = x < 0 ? x + G.N : (x >= G.N ? x - G.N : x); }
-            xy[2 * i] = x;
-            xy[2 * i + 1] = y;
-        }
-        if (a > 4) {
-            g = 1;
-            const int lr = band_owned_row(G, x);
-            if (lr >= 0) atomicMin(claim_new + (size_t)lr * G.N + y, i);
-        }
-    }
-    gz[i] = g;
+    if (do_finish) s = dwt_finish_agent(G, x, y, s, gain_prev, true, gz, claim_prev, agents_done_at, i);
+    dwt_move_claim_agent(G, agent_gamma, xy, st, s, x, y, act, claim, gz, i);
 }
 
-// Phase 3: the claim winner of an owned cell eats it and clears every stored copy; grazes that land in a ghost row only
-// clear the ghost copy (the owner rank does the eating). gain[i] = food eaten by agent i on THIS rank (0 elsewhere).
+// Phase 3. gain[i] = food eaten by agent i on THIS rank (0 elsewhere); in peer-memory mode the winner publishes it to every
+// rank instead, at exch + gain_off.
 template <class Cells>
 __global__ void __launch_bounds__(256) k_band_graze(BandGeom G, Cells C, const int32_t *__restrict__ xy, int n,
                                                     const uint8_t *__restrict__ gz, const int *__restrict__ claim, double *__restrict__ gain,
@@ -263,34 +287,23 @@ __global__ void __launch_bounds__(256) k_band_graze(BandGeom G, Cells C, const i
     if (i >= n) return;
     double got = 0.0;
     bool won = false;
-    if (gz[i]) {
-        const int x = xy[2 * i], y = xy[2 * i + 1];
-        const int lr = band_owned_row(G, x);
-        bool clear = true;
-        if (lr >= 0) {
-            if (claim[(size_t)lr * G.N + y] == i) { got = C.food((size_t)lr * G.pitch + G.c0 + y); won = true; }
-            else clear = false;                          // a lower-index agent eats here; it also does the clearing
-        }
-        if (clear)
-            band_row_images(G, x, [&](int r) { band_col_images(G, y, [&](int cc) { C.zero((size_t)r * G.pitch + cc); }); });
-    }
-    if (PT.on) {                                         // the winner publishes to every rank; the vectors were zeroed by k_band_finish
+    if (gz[i]) dwt_graze_agent(G, C, xy[2 * i], xy[2 * i + 1], [&](size_t k) { return claim[k]; }, i, got, won);
+    if (PT.on) {                                         // the vectors were zeroed by the finish of the step that last used them
         if (won) for (int p = 0; p < PT.R; ++p) PT.exch[p][(size_t)gain_off + i] = got;
         return;
     }
     gain[i] = got;
 }
 
-// Peer-memory mode, lattice state: k_band_finish_move_claim and k_band_graze in ONE launch. The graze needs every claim of
-// the step filed, so the two halves are separated by a grid-wide barrier (monotonic counter in global memory: the host passes
-// the value it has after this launch's blocks have all arrived). Only launched when the grid is at most one block per SM
+// Peer-memory mode, lattice state: k_band_move_claim and k_band_graze in ONE launch. The graze needs every claim of the step
+// filed, so the two halves are separated by a grid-wide barrier (monotonic counter in global memory: the host passes the
+// value it has after this launch's blocks have all arrived). Only launched when the grid is at most one block per SM
 // (n <= 256 * SMs), so every block is resident and the spin cannot deadlock. Saves one kernel boundary per step on the
 // critical path of a step (the two agent kernels are what is left there besides the stencil).
 __global__ void __launch_bounds__(256) k_band_fmc_graze(BandGeom G, double agent_gamma, int32_t *xy, double *st, int n,
                                                         const double *__restrict__ act, int *claim_new, uint8_t *gz, int do_finish,
-                                                        double *gain_prev, int *claim_prev, double *reward, uint8_t *done,
-                                                        int64_t *agents_done_at, LatCells C, PeerTable PT, int gain_off,
-                                                        unsigned int *bar, unsigned int target) {
+                                                        double *gain_prev, int *claim_prev, int64_t *agents_done_at, LatCells C,
+                                                        PeerTable PT, int gain_off, unsigned int *bar, unsigned int target) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const bool active = i < n;
     int x = 0, y = 0;
@@ -298,37 +311,8 @@ __global__ void __launch_bounds__(256) k_band_fmc_graze(BandGeom G, double agent
     if (active) {
         double s = st[i];
         x = xy[2 * i]; y = xy[2 * i + 1];
-        if (do_finish) {
-            const double gp = gain_prev[i];
-            gain_prev[i] = 0.0;
-            if (gz[i]) {
-                s = s + gp;
-                const int lr = band_owned_row(G, x);
-                if (lr >= 0) claim_prev[(size_t)lr * G.N + y] = 0x7fffffff;
-            }
-            s = dw_clip01(s);
-            reward[i] = s;
-            done[i] = s < 0.1;
-            agents_done_at[i] += (s < 0.1) ? 0 : 1;
-        }
-        const int a = (int)act[i] - 1;
-        s = s - agent_gamma;
-        st[i] = s;
-        if (s > 0.0) {
-            if (a != 8) {
-                const int d = (a & 2) ? 1 : -1;
-                if (((a + 1) & 2) == 0) { y += d; y = y < 0 ? y + G.N : (y >= G.N ? y - G.N : y); }
-                else { x += d; x = x < 0 ? x + G.N : (x >= G.N ? x - G.N : x); }
-                xy[2 * i] = x;
-                xy[2 * i + 1] = y;
-            }
-            if (a > 4) {
-                g = 1;
-                const int lr = band_owned_row(G, x);
-                if (lr >= 0) atomicMin(claim_new + (size_t)lr * G.N + y, i);
-            }
-        }
-        gz[i] = g;
+        if (do_finish) s = dwt_finish_agent(G, x, y, s, gain_prev, true, gz, claim_prev, agents_done_at, i);
+        g = dwt_move_claim_agent(G, agent_gamma, xy, st, s, x, y, act, claim_new, gz, i);
     }
     // every claim of the step is filed once all blocks have passed here
     __syncthreads();
@@ -341,37 +325,18 @@ __global__ void __launch_bounds__(256) k_band_fmc_graze(BandGeom G, double agent
     __syncthreads();
     if (!active || !g) return;
     double got = 0.0;
-    bool won = false, clear = true;
-    const int lr = band_owned_row(G, x);
-    if (lr >= 0) {
-        if (__ldcg(claim_new + (size_t)lr * G.N + y) == i) { got = C.food((size_t)lr * G.pitch + G.c0 + y); won = true; }
-        else clear = false;
-    }
-    if (clear)
-        band_row_images(G, x, [&](int r) { band_col_images(G, y, [&](int cc) { C.zero((size_t)r * G.pitch + cc); }); });
+    bool won = false;                                    // claims of other blocks of this launch: read past L1
+    dwt_graze_agent(G, C, x, y, [&](size_t k) { return __ldcg(claim_new + k); }, i, got, won);
     if (won) for (int p = 0; p < PT.R; ++p) PT.exch[p][(size_t)gain_off + i] = got;
 }
 
-// Phase 4 (replicated, after the gains were summed over ranks): state += gain, clip, reward/done, lifespan counter;
-// also returns the graze claims of this step to "idle".
+// Phase 4 (replicated, after the gains were summed over ranks) of phase-by-phase and NCCL mode, and of the last step in
+// peer-memory mode (dwt_flush_p2p).
 __global__ void __launch_bounds__(256) k_band_finish(BandGeom G, const int32_t *__restrict__ xy, int *claim, double *st, int n,
-                                                     double *gain, int zero_gain, const uint8_t *__restrict__ gz, double *reward,
-                                                     uint8_t *done, int64_t *agents_done_at) {
+                                                     double *gain, int zero_gain, const uint8_t *__restrict__ gz, int64_t *agents_done_at) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    double s = st[i];
-    const double g = gain[i];
-    if (zero_gain) gain[i] = 0.0;                        // peer-memory mode: only winners write, so the vector is re-armed here
-    if (gz[i]) {
-        s = s + g;
-        const int lr = band_owned_row(G, xy[2 * i]);
-        if (lr >= 0) claim[(size_t)lr * G.N + xy[2 * i + 1]] = 0x7fffffff;
-    }
-    s = dw_clip01(s);
-    st[i] = s;
-    reward[i] = s;
-    done[i] = s < 0.1;
-    agents_done_at[i] += (s < 0.1) ? 0 : 1;
+    st[i] = dwt_finish_agent(G, xy[2 * i], xy[2 * i + 1], st[i], gain, zero_gain, gz, claim, agents_done_at, i);
 }
 
 // ---- ghost maintenance ---------------------------------------------------------------------------------------------
@@ -387,24 +352,16 @@ __global__ void __launch_bounds__(256) k_band_ghost_rows_wrap(BandGeom G, uint32
 // ---- first step: literal forward from the off-lattice fp64 cover planes [(R+2) x N] onto the padded lattice ---------
 // SERIES: also adds {sum sqrt(g)*T, sum milli-light, sum milli-dark} of the band's cells to series[0..2] (see k_tiled_step)
 template <bool SERIES = false>
-__global__ void __launch_bounds__(256) k_band_first_step(DevParams P, double SL, BandGeom Gp, const double *__restrict__ l,
-                                                         const double *__restrict__ d, BandGeom Gl, uint32_t *__restrict__ lat_out,
-                                                         int *stepmax, double sqrt_g = 0.0, double *series = nullptr) {
+__global__ void __launch_bounds__(256) k_band_first_step(DevParams P, double SL, BandGeom Gp, PlaneCells pre, BandGeom Gl,
+                                                         uint32_t *__restrict__ lat_out, int *stepmax, double sqrt_g = 0.0,
+                                                         double *series = nullptr) {
     const size_t total = (size_t)Gp.R * Gp.N;
     uint32_t mx = 0;
     double ser[3] = {0.0, 0.0, 0.0};     // series mode; the cover sums are integers below 2^53, so exact in fp64
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const int r = (int)(i / Gp.N), y = (int)(i - (size_t)r * Gp.N);
-        const int ys[3] = {y == 0 ? Gp.N - 1 : y - 1, y, y == Gp.N - 1 ? 0 : y + 1};
         double l9[9], d9[9];
-#pragma unroll
-        for (int a = 0; a < 3; ++a)
-#pragma unroll
-            for (int c = 0; c < 3; ++c) {
-                const size_t k = (size_t)(r + a) * Gp.pitch + ys[c];     // stored rows r .. r+2 = band rows r-1 .. r+1
-                l9[a * 3 + c] = l[k];
-                d9[a * 3 + c] = d[k];
-            }
+        pre.load9(Gp, r, y, l9, d9);
         const LitCell o = dw_literal_cell(P, SL, l9, d9);
         const uint32_t q = dw_pack((int)rint(o.nl * 1000.0), (int)rint(o.nd * 1000.0));
         uint32_t *orow = lat_out + (size_t)(r + 1) * Gl.pitch;
@@ -766,33 +723,6 @@ __global__ void __launch_bounds__(256) k_band_lookahead_decide(BandGeom G, const
 // ---- materialisation / synthetic reset -------------------------------------------------------------------------------
 // full reference grid [7, R, N] of the band, materialised by a literal forward from the post-graze state the last step
 // started from: the other lattice buffer, or the fp64 planes when that step was the first one after a reset
-struct PreLattice {
-    const uint32_t *p;
-    __device__ __forceinline__ void load9(const BandGeom &G, int r, int y, double (&l9)[9], double (&d9)[9]) const {
-#pragma unroll
-        for (int a = 0; a < 3; ++a)
-#pragma unroll
-            for (int c = 0; c < 3; ++c) {
-                const uint32_t w = p[(size_t)(r + a) * G.pitch + G.c0 + y + c - 1];
-                l9[a * 3 + c] = dw_milli(w & 0xffffu);
-                d9[a * 3 + c] = dw_milli(w >> 16);
-            }
-    }
-};
-struct PrePlanes {
-    const double *l, *d;
-    __device__ __forceinline__ void load9(const BandGeom &G, int r, int y, double (&l9)[9], double (&d9)[9]) const {
-        const int ys[3] = {y == 0 ? G.N - 1 : y - 1, y, y == G.N - 1 ? 0 : y + 1};
-#pragma unroll
-        for (int a = 0; a < 3; ++a)
-#pragma unroll
-            for (int c = 0; c < 3; ++c) {
-                const size_t k = (size_t)(r + a) * G.pitch + ys[c];
-                l9[a * 3 + c] = l[k];
-                d9[a * 3 + c] = d[k];
-            }
-    }
-};
 template <class Pre>
 __global__ void __launch_bounds__(256) k_band_materialise(DevParams P, double SL, BandGeom G, Pre pre, double *__restrict__ out) {
     const size_t RN = (size_t)G.R * G.N;
