@@ -36,6 +36,9 @@
  *
  * Peer-memory mode (dwt_step_p2p) refuses DW_POLICY_MLP; dwt_observe works there after dwt_flush_p2p.
  *
+ * Diagnostics (dwt_get_diag, dwt_get_diag_stats, dwt_get_cover_stats, dwt_pool): the unrounded fields of the last step's
+ * forward, their statistics and block sums for images, reduced on the device per band; see the section below.
+ *
  * Constraints of the tiled kernels: N >= 64, 8 <= rows <= N, D4-symmetric kernels (the defaults). Bands may differ in
  * height; a side or band that is not a multiple of 64 runs a masked instance of the stencil kernel over its partial tiles.
  */
@@ -173,6 +176,43 @@ int dwt_debug_slow_count(dwt_handle *h, uint64_t *count);
    agent overhead. Overwrites the recorded pre-state (dwt_get_grid needs a new step afterwards). Always times the kernel
    with series mode off and records nothing into the series rows. */
 int dwt_debug_time_stencil(dwt_handle *h, int32_t reps, double *us_per_launch);
+
+/* ---- diagnostics and plot feed (what the reference's notebook helpers read: env.temp.mean(), the covers, images) ---------
+ * The fields are the unrounded side effects of the last step's forward, as dw_get_diag defines them (DW_DIAG_* selectors),
+ * evaluated like dwt_get_grid: a literal forward of the post-graze pre-state that step started from, at S * L of that step.
+ * Nothing but the requested result is allocated: statistics and images are reduced on the device while the field is
+ * evaluated (per-CTA partials, then one block, in a fixed order: the same banding returns the same bits on every call).
+ * The results are the band's own part; a multi-rank caller merges them (banded.py: one SUM all-reduce per call).
+ * DW_E_STATE without a pre-state (before the first step after an upload / reset, after dwt_debug_time_stencil) and while a
+ * step's agents are not finished (as dwt_observe); DW_E_INVALID for a bad selector or block size.
+ * Reading the pre-state races with the next step's halo push in peer-memory mode: a caller meets every rank (any
+ * collective) after these calls and before the next dwt_step_p2p. */
+/* dwt_pool field selectors: DW_DIAG_TEMP .. DW_DIAG_BETA_D, the two planes of DW_DIAG_GROWTH, and the grid channels
+   0, 1, 2, 3, 5 of dwt_get_grid (rounded b', light, dark, rounded T, rounded T_d) */
+enum {
+    DWT_FIELD_TEMP = 0, DWT_FIELD_TEMP_LIGHT = 1, DWT_FIELD_TEMP_DARK = 2, DWT_FIELD_TEMP_EFFECTIVE = 3,
+    DWT_FIELD_BETA = 4, DWT_FIELD_BETA_L = 5, DWT_FIELD_BETA_D = 6, DWT_FIELD_GROWTH_L = 7, DWT_FIELD_GROWTH_D = 8,
+    DWT_FIELD_GRID_BARE = 9, DWT_FIELD_GRID_LIGHT = 10, DWT_FIELD_GRID_DARK = 11, DWT_FIELD_GRID_TEMP = 12,
+    DWT_FIELD_GRID_TEMP_DARK = 13
+};
+/* the band's field [rows, N] (DW_DIAG_GROWTH: [2, rows, N], dl then dd) -> host; uses the dwt_get_grid scratch. Synchronises. */
+int dwt_get_diag(dwt_handle *h, int32_t which, double *out);
+/* out[5] = {count, mean, m2, min, max} of a DW_DIAG_* field over the band's own cells (growth: both planes, 2 * rows * N
+   values), m2 = sum (x - mean)^2 about the band's mean. Synchronises. */
+int dwt_get_diag_stats(dwt_handle *h, int32_t which, double *out);
+/* out[4] = {sum light, sum dark, max light, max dark} over the band's own cells of the CURRENT state (also right after a
+   reset); exact on the lattice (integer milli-covers). Synchronises. */
+int dwt_get_cover_stats(dwt_handle *h, double *out);
+/* Block sums of a DWT_FIELD_* field over the cells this band owns -> device buffer [H, H], H = ceil(N / block), 1 <= block
+   <= N: entry (i, j) sums global rows and columns [i * block, min((i + 1) * block, N)) x [j * block, ...); every entry is
+   written (0 where the band owns nothing), so the SUM over the ranks is the whole world's block sums. Dividing by the
+   cells of each block (fewer at the edges when block does not divide N) gives the block-averaged image. On the handle's
+   stream; the buffer is allocated on first use and grows with H. */
+int dwt_pool(dwt_handle *h, int32_t field, int32_t block);
+int dwt_get_pool_ptr(dwt_handle *h, double **pool /* device [H, H] */, int32_t *H);
+int dwt_get_pool(dwt_handle *h, double *out /* host [H, H] */);               /* synchronises */
+/* L of the last step's forward (the L of the reset before any step), for the bare-planet temperature; as dw_get_last_L */
+int dwt_get_last_L(dwt_handle *h, double *L);
 
 #ifdef __cplusplus
 }

@@ -10,6 +10,10 @@ DW_POLICY = {"none": 0, "greedy": 1, "antigreedy": 2, "replay": 3, "random": 4, 
 DW_E_UNSUPPORTED = -3       # include/daisyworld_b200.h: configuration outside what the kernels implement
 DW_DIAG = {"temp": 0, "temp_light": 1, "temp_dark": 2, "temp_effective": 3, "beta": 4, "beta_l": 5, "beta_d": 6,
            "growth": 7}
+# dwt_pool field selectors (include/daisyworld_b200_tiled.h): the diagnostics, the growth planes and grid channels 0-3, 5
+DWT_FIELD = {"temp": 0, "temp_light": 1, "temp_dark": 2, "temp_effective": 3, "beta": 4, "beta_l": 5, "beta_d": 6,
+             "growth_l": 7, "growth_d": 8, "grid_bare": 9, "grid_light": 10, "grid_dark": 11, "grid_temp": 12,
+             "grid_temp_dark": 13}
 
 
 class DwConfig(C.Structure):
@@ -54,6 +58,7 @@ TILED_SYMBOLS = [
     "dwt_debug_slow_count", "dwt_debug_time_stencil", "dwt_cover_checksum", "dwt_ipc_export", "dwt_ipc_attach", "dwt_get_peer_buffers", "dwt_attach_peers", "dwt_step_p2p",
     "dwt_flush_p2p", "dwt_peer_status", "dwt_set_series", "dwt_get_series_ptr", "dwt_get_series", "dwt_get_pitch", "dwt_set_peer_rows",
     "dwt_observe", "dwt_get_obs_ptr", "dwt_get_obs", "dwt_set_mlp",
+    "dwt_get_diag", "dwt_get_diag_stats", "dwt_get_cover_stats", "dwt_pool", "dwt_get_pool_ptr", "dwt_get_pool", "dwt_get_last_L",
 ]
 
 
@@ -190,6 +195,13 @@ def load():
         "dwt_get_obs_ptr": (C.c_int, [vp, C.POINTER(vp)]),
         "dwt_get_obs": (C.c_int, [vp, pd]),
         "dwt_set_mlp": (C.c_int, [vp, pd, i32]),
+        "dwt_get_diag": (C.c_int, [vp, i32, pd]),
+        "dwt_get_diag_stats": (C.c_int, [vp, i32, pd]),
+        "dwt_get_cover_stats": (C.c_int, [vp, pd]),
+        "dwt_pool": (C.c_int, [vp, i32, i32]),
+        "dwt_get_pool_ptr": (C.c_int, [vp, C.POINTER(vp), pi32]),
+        "dwt_get_pool": (C.c_int, [vp, pd]),
+        "dwt_get_last_L": (C.c_int, [vp, pd]),
     }
     assert set(tsig) == set(TILED_SYMBOLS)
     sig.update(tsig)

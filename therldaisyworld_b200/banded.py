@@ -16,7 +16,9 @@ NCCL over NVLink on GPUs, gloo in the CPU tests -- plumbing only, the data path 
     ``run_series`` a SUM all-reduce of the per-step temperature and cover sums next to it;
   * ``observe()`` and every ``policy="mlp"`` step: a SUM all-reduce of the bands' partial observations ``[n, 7, 3, 3]``
     (the band that owns a window cell's row evaluates it, every other band contributes 0). An MLP step then decides on
-    every rank from the same observation and needs no act exchange: two collectives per step (gain, obs).
+    every rank from the same observation and needs no act exchange: two collectives per step (gain, obs);
+  * the diagnostics (``diag_stats``, ``cover_stats``, ``image``): one SUM all-reduce per call of the bands' device-reduced
+    parts, so every rank returns the same value.
 
 ``world_size == 1`` needs none of them (``dwt_halo_wrap`` closes the torus locally).
 
@@ -30,7 +32,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import DwClock, DwtPtrs, DW_POLICY
+from ._lib import DwClock, DwtPtrs, DW_DIAG, DW_POLICY, DWT_FIELD
 from .env import make_clock_struct, make_config_struct, set_default_attributes, set_default_kernels
 
 _WORLD_POLICIES = ("greedy", "antigreedy", "eps_greedy")      # decisions that (may) read the grid: need the act exchange
@@ -355,6 +357,46 @@ class DeviceBand:
         self._check(self._lib.dwt_get_grid(self._h, out.ctypes.data_as(C.POINTER(C.c_double))), "dwt_get_grid")
         return out
 
+    # ---- diagnostics and plot feed (the unrounded fields of the last forward; dwt_get_diag .. dwt_pool)
+    def diag(self, name):
+        """The band's field `name` (a DW_DIAG key) of the last forward: [rows, N], growth [2, rows, N] (dl, dd)."""
+        out = np.empty((2, self.rows, self.N) if name == "growth" else (self.rows, self.N))
+        self._check(self._lib.dwt_get_diag(self._h, DW_DIAG[name], out.ctypes.data_as(C.POINTER(C.c_double))), "dwt_get_diag")
+        return out
+
+    def diag_stats(self, name):
+        """[count, mean, m2, min, max] of the field over the band's own cells, m2 about the band's mean."""
+        out = np.zeros(5)
+        self._check(self._lib.dwt_get_diag_stats(self._h, DW_DIAG[name], out.ctypes.data_as(C.POINTER(C.c_double))),
+                    "dwt_get_diag_stats")
+        return out
+
+    def cover_stats(self):
+        """[sum light, sum dark, max light, max dark] over the band's own cells of the current state."""
+        out = np.zeros(4)
+        self._check(self._lib.dwt_get_cover_stats(self._h, out.ctypes.data_as(C.POINTER(C.c_double))), "dwt_get_cover_stats")
+        return out
+
+    def pool(self, field, block):
+        """Launch the block sums [H, H] of a DWT_FIELD field over the band's own cells (dwt_pool) and return the device
+        buffer as a torch view (summed over the ranks in place by the caller)."""
+        self._check(self._lib.dwt_pool(self._h, DWT_FIELD[field], int(block)), "dwt_pool")
+        p, H = C.c_void_p(), C.c_int32(0)
+        self._check(self._lib.dwt_get_pool_ptr(self._h, C.byref(p), C.byref(H)), "dwt_get_pool_ptr")
+        return self._view(p.value, (H.value, H.value), "<f8")
+
+    def get_pool(self):
+        p, H = C.c_void_p(), C.c_int32(0)
+        self._check(self._lib.dwt_get_pool_ptr(self._h, C.byref(p), C.byref(H)), "dwt_get_pool_ptr")
+        out = np.zeros((H.value, H.value))
+        self._check(self._lib.dwt_get_pool(self._h, out.ctypes.data_as(C.POINTER(C.c_double))), "dwt_get_pool")
+        return out
+
+    def last_L(self):
+        L = C.c_double(0.0)
+        self._check(self._lib.dwt_get_last_L(self._h, C.byref(L)), "dwt_get_last_L")
+        return L.value
+
     def slow_count(self):
         c = C.c_uint64(0)
         self._check(self._lib.dwt_debug_slow_count(self._h, C.byref(c)), "dwt_debug_slow_count")
@@ -610,3 +652,104 @@ class BandedDaisyWorld:
         """[7, rows, N]: env.grid[0] restricted to this rank's rows."""
         self._flush()
         return self.band.grid()
+
+    # ---- diagnostics and plot feed (DESIGN.md §0 row (f) N3): what the reference's notebook helpers read from
+    # RLDaisyWorld (notebook_helpers.py:45-57,139-150,210-223), reduced on the device per band and merged over the ranks.
+    # The fields are the unrounded side effects of the last step's forward, like RLDaisyWorld.temp / .growth.
+    # Every call is collective when world_size > 1 (every rank calls it) and returns the same value on every rank.
+    def _table(self, row):
+        """Every rank's row of a [world_size, k] table, in rank order: one SUM all-reduce of a table in which each rank
+        fills its own row (x + 0 is exact, so every rank gets every row's bits). In peer-memory mode it is also what keeps
+        the next step's halo push off the pre-state until every rank has read it (see _observe_device)."""
+        row = np.asarray(row, dtype=np.float64)
+        if self.comm is None:
+            return row[None]
+        t = self.band.exch_tensor(gain=True, act=False).new_zeros((self.world_size, row.size))
+        t[self.rank] = t.new_tensor(row)
+        self.comm.all_reduce_sum(t)
+        return t.cpu().numpy()
+
+    @staticmethod
+    def _merge_stats(rows):
+        """Chan's pairwise merge of [count, mean, m2, min, max] rows, in row order -> (count, mean, m2, min, max)."""
+        n, mean, m2 = rows[0, :3]
+        for c, mu, q in rows[1:, :3]:
+            tot = n + c
+            d = mu - mean
+            mean = mean + d * (c / tot)
+            m2 = m2 + q + d * d * (n * c / tot)
+            n = tot
+        return n, mean, m2, rows[:, 3].min(), rows[:, 4].max()
+
+    def local_diag(self, name):
+        """[rows, N] ([2, rows, N] for growth): this rank's rows of the unrounded field `name` (temp, temp_light, temp_dark,
+        temp_effective, beta, beta_l, beta_d, growth) of the last step's forward. In peer-memory mode every rank must call it."""
+        if name not in DW_DIAG:
+            raise ValueError(f"unknown diagnostic field {name!r}; one of {sorted(DW_DIAG)}")
+        self._flush()
+        out = self.band.diag(name)
+        if self.mode == "p2p":
+            self._table([0.0])                       # fence: no rank's next step before every rank has read its pre-state
+        self._check_peers()
+        return out
+
+    def diag_stats(self, name):
+        """{mean, std, min, max} of a diagnostic field over the whole world (growth: both planes), std the population std
+        like np.std -- RLDaisyWorld.diag_stats for the giant world."""
+        if name not in DW_DIAG:
+            raise ValueError(f"unknown diagnostic field {name!r}; one of {sorted(DW_DIAG)}")
+        self._flush()
+        n, mean, m2, mn, mx = self._merge_stats(self._table(self.band.diag_stats(name)))
+        self._check_peers()
+        return dict(mean=mean, std=float(np.sqrt(m2 / n)), min=mn, max=mx)
+
+    def cover_stats(self):
+        """Mean and max light / dark cover of the current state over the whole world (RLDaisyWorld.cover_stats)."""
+        self._flush()
+        rows = self._table(self.band.cover_stats())
+        self._check_peers()
+        cells = float(self.dim) * self.dim
+        return dict(mean_light=rows[:, 0].sum() / cells, mean_dark=rows[:, 1].sum() / cells, max_light=rows[:, 2].max(),
+                    max_dark=rows[:, 3].max())
+
+    def image(self, field, block=16):
+        """[H, H] block means of a field over the whole world, H = ceil(N / block): block (i, j) averages rows and columns
+        [i*block, min((i+1)*block, N)) x [j*block, ...) (edge blocks are smaller when block does not divide N). field: a
+        diagnostic (growth gives [2, H, H]; growth_l / growth_d one plane) or a grid channel as local_grid() holds it --
+        grid_bare, grid_light, grid_dark, grid_temp, grid_temp_dark (channels 0, 1, 2, 3, 5). Only the image leaves the
+        device."""
+        if field == "growth":
+            return np.stack([self.image("growth_l", block), self.image("growth_d", block)])
+        if field not in DWT_FIELD:
+            raise ValueError(f"unknown image field {field!r}; one of {sorted(DWT_FIELD) + ['growth']}")
+        self._flush()
+        t = self.band.pool(field, block)
+        self.band.synchronize()                      # the block sums exist (and the pre-state is read) before any exchange
+        if self.comm is not None:
+            self.comm.all_reduce_sum(t)
+        sums = t.cpu().numpy()
+        self._check_peers()
+        H = sums.shape[0]
+        edge = np.minimum(np.arange(1, H + 1) * int(block), self.dim) - np.arange(H) * int(block)
+        return sums / np.outer(edge, edge)
+
+    @property
+    def dead_temp(self):
+        """reference :406-407,416 -- bare-planet temperature at the L of the last forward, as RLDaisyWorld.dead_temp."""
+        L = self.band.last_L()
+        return np.array([((self.S * L * (1 - self.albedo_bare)) / self.sigma) ** (1 / 4)])
+
+    def run_with_series(self, K, every=16, policy="greedy", seed=0, images=(), block=16):
+        """K steps in chunks of `every`, recording after each chunk what the reference's plot helpers read
+        (notebook_helpers.py:45-57), as RLDaisyWorld.run_with_series: step, L, temp_mean, temp_std, dead_temp, light,
+        dark; plus images = {field: image(field, block)} for the requested fields."""
+        series = []
+        done = 0
+        while done < K:
+            k = min(every, K - done)
+            self.run(k, policy=policy, seed=seed)
+            done += k
+            t, c = self.diag_stats("temp"), self.cover_stats()
+            series.append(dict(step=self.step_count, L=self.L, temp_mean=t["mean"], temp_std=t["std"], dead_temp=float(self.dead_temp[0]),
+                               light=c["mean_light"], dark=c["mean_dark"], images={f: self.image(f, block) for f in images}))
+        return series

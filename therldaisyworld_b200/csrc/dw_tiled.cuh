@@ -857,3 +857,138 @@ __global__ void __launch_bounds__(256) k_band_init_random(BandGeom Gp, uint64_t 
         agent_state[i] = 1.0;
     }
 }
+
+// ---- diagnostics and plot feed (the unrounded fields of the last forward, their statistics, block-averaged images) ------
+// Every field is evaluated like k_band_materialise: dw_literal_cell on the post-graze pre-state at SL = S * L_last. Field
+// selectors are those of dwt_pool (include/daisyworld_b200_tiled.h): 0..6 equal DW_DIAG_TEMP..DW_DIAG_BETA_D, then the two
+// growth planes and the grid channels 0, 1, 2, 3, 5 as dwt_get_grid holds them. The one mapping all field kernels share:
+__device__ __forceinline__ double dwt_field_value(const LitCell &o, int field) {
+    switch (field) {
+        case DWT_FIELD_TEMP: return o.T;
+        case DWT_FIELD_TEMP_LIGHT: return o.Tl;
+        case DWT_FIELD_TEMP_DARK: return o.Td;
+        case DWT_FIELD_TEMP_EFFECTIVE: return o.Te;
+        case DWT_FIELD_BETA: return o.beta;
+        case DWT_FIELD_BETA_L: return o.beta_l;
+        case DWT_FIELD_BETA_D: return o.beta_d;
+        case DWT_FIELD_GROWTH_L: return o.dl;
+        case DWT_FIELD_GROWTH_D: return o.dd;
+        case DWT_FIELD_GRID_BARE: return dw_round3(o.nb);
+        case DWT_FIELD_GRID_LIGHT: return dw_round3(o.nl);
+        case DWT_FIELD_GRID_DARK: return dw_round3(o.nd);
+        case DWT_FIELD_GRID_TEMP: return dw_round3(o.T);
+        default: return dw_round3(o.Td);                 // DWT_FIELD_GRID_TEMP_DARK
+    }
+}
+// the cell (r, y) of the band (band row r, 0-based), evaluated from the pre-state
+template <class Pre>
+__device__ __forceinline__ LitCell dwt_band_cell(const DevParams &P, double SL, const BandGeom &G, const Pre &pre, int r, int y) {
+    double l9[9], d9[9];
+    pre.load9(G, r, y, l9, d9);
+    return dw_literal_cell(P, SL, l9, d9);
+}
+
+// One DW_DIAG_* field of the band [R, N] (DW_DIAG_GROWTH: [2, R, N], dl then dd), as k_diag computes it.
+template <class Pre>
+__global__ void __launch_bounds__(256) k_band_diag(DevParams P, double SL, BandGeom G, Pre pre, int which, double *__restrict__ out) {
+    const size_t RN = (size_t)G.R * G.N;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < RN; i += (size_t)gridDim.x * blockDim.x) {
+        const int r = (int)(i / G.N), y = (int)(i - (size_t)r * G.N);
+        const LitCell o = dwt_band_cell(P, SL, G, pre, r, y);
+        if (which == DW_DIAG_GROWTH) {
+            out[i] = dwt_field_value(o, DWT_FIELD_GROWTH_L);
+            out[RN + i] = dwt_field_value(o, DWT_FIELD_GROWTH_D);
+        } else {
+            out[i] = dwt_field_value(o, which);
+        }
+    }
+}
+
+// Statistics of one DW_DIAG_* field over the band's own cells, evaluated and reduced without storing the field: per thread
+// {sum, sum of squares} of (x - shift), min and max, then dw_stats_block_reduce -> partial[4 * blockIdx.x]. The shift is the
+// field at the band's first cell (dl there for growth, whose two planes are reduced together); block 0 stores it at
+// partial[4 * gridDim.x + 4], behind the 4 results of k_band_partials_final. A fixed grid gives a fixed summation order.
+template <class Pre>
+__global__ void __launch_bounds__(256) k_band_field_stats(DevParams P, double SL, BandGeom G, Pre pre, int which, double *__restrict__ partial) {
+    const bool growth = which == DW_DIAG_GROWTH;
+    const int f0 = growth ? DWT_FIELD_GROWTH_L : which;
+    const double shift = dwt_field_value(dwt_band_cell(P, SL, G, pre, 0, 0), f0);
+    double s = 0.0, q = 0.0, mn = 1e300, mx = -1e300;
+    const size_t RN = (size_t)G.R * G.N;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < RN; i += (size_t)gridDim.x * blockDim.x) {
+        const int r = (int)(i / G.N), y = (int)(i - (size_t)r * G.N);
+        const LitCell o = dwt_band_cell(P, SL, G, pre, r, y);
+        for (int k = 0; k < (growth ? 2 : 1); ++k) {
+            const double v = dwt_field_value(o, f0 + k), d = v - shift;
+            s += d; q += d * d; mn = fmin(mn, v); mx = fmax(mx, v);
+        }
+    }
+    dw_stats_block_reduce(s, q, mn, mx, partial + 4 * blockIdx.x);
+    if (blockIdx.x == 0 && threadIdx.x == 0) partial[4 * gridDim.x + 4] = shift;
+}
+
+// Covers of the band's own cells in the current state: per block {sum light, sum dark, min(-light), max dark} (the min slot
+// of dw_stats_block_reduce carries the light maximum negated). On the lattice the values are the integer milli-covers, so
+// every sum is exact (below 2^53) and independent of the order; on the fp64 planes of a reset the fixed grid fixes it.
+__device__ __forceinline__ void dwt_cell_covers(const LatCells &C, size_t i, double &l, double &d) {
+    const uint32_t w = C.p[i];
+    l = (double)(w & 0xffffu);
+    d = (double)(w >> 16);
+}
+__device__ __forceinline__ void dwt_cell_covers(const PlaneCells &C, size_t i, double &l, double &d) { l = C.l[i]; d = C.d[i]; }
+template <class Cells>
+__global__ void __launch_bounds__(256) k_band_cover_stats(BandGeom G, Cells C, double *__restrict__ partial) {
+    double sl = 0.0, sd = 0.0, nml = 1e300, md = -1e300;
+    const size_t RN = (size_t)G.R * G.N;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < RN; i += (size_t)gridDim.x * blockDim.x) {
+        const int r = (int)(i / G.N), y = (int)(i - (size_t)r * G.N);
+        double l, d;
+        dwt_cell_covers(C, (size_t)(r + 1) * G.pitch + G.c0 + y, l, d);
+        sl += l; sd += d; nml = fmin(nml, -l); md = fmax(md, d);
+    }
+    dw_stats_block_reduce(sl, sd, nml, md, partial + 4 * blockIdx.x);
+}
+
+// Second stage of both: the `blocks` partials in a fixed order -> out[0..3] = {sum, sum, min, max}.
+__global__ void __launch_bounds__(256) k_band_partials_final(const double *__restrict__ partial, int blocks, double *__restrict__ out) {
+    double s = 0.0, q = 0.0, mn = 1e300, mx = -1e300;
+    for (int i = threadIdx.x; i < blocks; i += blockDim.x) {
+        s += partial[4 * i]; q += partial[4 * i + 1]; mn = fmin(mn, partial[4 * i + 2]); mx = fmax(mx, partial[4 * i + 3]);
+    }
+    dw_stats_block_reduce(s, q, mn, mx, out);
+}
+
+// Block sums of a field for a block-averaged image: output block (i, j) covers global rows and columns [i*b, min((i+1)*b, N))
+// x [j*b, min((j+1)*b, N)); only the cells this band owns count, so the sum over the ranks is the whole world's. Work unit u =
+// (output block, slice s of `slices`) -- the slice takes every slices-th row of the block -- is reduced by one warp in a
+// fixed order (lane-strided, then a shuffle tree); out[u] is written for every unit, 0 where the band owns nothing.
+// slices == 1: out is the [H, H] image; else [H * H, slices] partials for k_band_pool_final.
+template <class Pre>
+__global__ void __launch_bounds__(256) k_band_pool(DevParams P, double SL, BandGeom G, Pre pre, int field, int b, int H, int slices,
+                                                   double *__restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    const long long units = (long long)H * H * slices;
+    for (long long u = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5; u < units; u += ((long long)gridDim.x * blockDim.x) >> 5) {
+        const long long blk = u / slices;
+        const int s = (int)(u - blk * slices);
+        const int bi = (int)(blk / H), bj = (int)(blk - (long long)bi * H);
+        const int x0 = bi * b, y0 = bj * b;
+        const int bh = min(b, G.N - x0), bw = min(b, G.N - y0);
+        const int sh = bh > s ? (bh - s + slices - 1) / slices : 0;    // rows s, s + slices, ... of the block
+        double acc = 0.0;
+        for (int k = lane; k < sh * bw; k += 32) {
+            const int rr = k / bw, y = y0 + (k - rr * bw);
+            const int lr = band_owned_row(G, x0 + s + rr * slices);
+            if (lr >= 0) acc += dwt_field_value(dwt_band_cell(P, SL, G, pre, lr - 1, y), field);
+        }
+        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+        if (lane == 0) out[u] = acc;
+    }
+}
+__global__ void __launch_bounds__(256) k_band_pool_final(const double *__restrict__ partial, int slices, long long hh, double *__restrict__ out) {
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < hh; i += (long long)gridDim.x * blockDim.x) {
+        double acc = 0.0;
+        for (int s = 0; s < slices; ++s) acc += partial[i * slices + s];
+        out[i] = acc;
+    }
+}

@@ -13,7 +13,11 @@ clock, download included) and of the device observation alone (CUDA events); and
 of an mlp step from torch.profiler (k_band_obs, k_mlp_act, ...), in a separate profiled run.
 
 --vs-ensemble N: whole greedy steps of one N x N world as the giant world (BandedDaisyWorld.run) and as an ensemble of one
-(RLDaisyWorld, batch_size = 1, run()), 4 agents like RLDaisyWorld's default, alternating over five repetitions."""
+(RLDaisyWorld, batch_size = 1, run()), 4 agents like RLDaisyWorld's default, alternating over five repetitions.
+
+--diag [N]: the diagnostics and plot feed (default N = 16384, N agents): diag_stats("temp"), image("temp", 16),
+image("grid_light", 16), cover_stats() and the device part of image() alone (dwt_pool), each timed with CUDA events around
+the whole call (download included), next to a greedy step, alternating over five repetitions."""
 import sys, os, subprocess, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -167,6 +171,44 @@ def bench_mlp(N, K=64, reps=5):
     sys.stdout.flush()
 
 
+def bench_diag(N, K=32, reps=5):
+    w = BandedDaisyWorld(N, N)
+    w.reset_on_device(seed=1)
+    w.run(2, "greedy")
+
+    def timed(fn):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        torch.cuda.synchronize()
+        e0.record()
+        fn()
+        e1.record()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) * 1e3
+
+    def step():
+        w.band.run_local(K, "greedy")
+        w._pending += K
+        w.end_chunk()
+
+    calls = {"greedy step": lambda: timed(step) / K,
+             'diag_stats("temp")': lambda: timed(lambda: w.diag_stats("temp")),
+             'image("temp", 16)': lambda: timed(lambda: w.image("temp", 16)),
+             'image("grid_light", 16)': lambda: timed(lambda: w.image("grid_light", 16)),
+             "cover_stats()": lambda: timed(w.cover_stats),
+             'dwt_pool("temp", 16) alone': lambda: timed(lambda: w.band.pool("temp", 16))}
+    for fn in calls.values():                    # warm-up: module loading, lazy buffers
+        fn()
+    times = {k: [] for k in calls}
+    for _ in range(reps):
+        for k, fn in calls.items():
+            times[k].append(fn())
+    print(f"N={N}, {N} agents, greedy, {reps} alternating repetitions (CUDA events around each call, download included)")
+    for k, ts in times.items():
+        print(f"  {k:26s} us: " + " ".join(f"{t:.0f}" for t in ts) + f" | median {np.median(ts):.0f}")
+    t, img = w.diag_stats("temp"), w.image("temp", 16)
+    print(f"  check: temp mean {t['mean']:.6f} K, std {t['std']:.6f}; mean of the 16-block image {img.mean():.6f}", flush=True)
+
+
 def bench_vs_ensemble(N, K=200, reps=5):
     from therldaisyworld_b200 import RLDaisyWorld
     n = 4
@@ -208,6 +250,11 @@ if __name__ == "__main__":
         assert args and args[0] == "mlp", "--policy mlp [N]"
         print(f"GPU: {gpu_label()}")
         bench_mlp(int(args[1]) if len(args) > 1 else 16384)
+        sys.exit(0)
+    if "--diag" in sys.argv:
+        args = [a for a in sys.argv[1:] if a != "--diag"]
+        print(f"GPU: {gpu_label()}")
+        bench_diag(int(args[0]) if args else 16384)
         sys.exit(0)
     if "--series" in sys.argv:
         args = [a for a in sys.argv[1:] if a != "--series"]
