@@ -39,6 +39,10 @@
  * Diagnostics (dwt_get_diag, dwt_get_diag_stats, dwt_get_cover_stats, dwt_pool): the unrounded fields of the last step's
  * forward, their statistics and block sums for images, reduced on the device per band; see the section below.
  *
+ * Snapshots (dwt_save_state, dwt_restore_state): a band's whole state out to the host and back, exactly, between steps; a
+ * snapshot of one banding restores on any other, because the state is the same integer lattice whatever the banding. See
+ * the section below.
+ *
  * Constraints of the tiled kernels: N >= 64, 8 <= rows <= N, D4-symmetric kernels (the defaults). Bands may differ in
  * height; a side or band that is not a multiple of 64 runs a masked instance of the stencil kernel over its partial tiles.
  */
@@ -150,6 +154,8 @@ int dwt_ipc_attach(dwt_handle *h, int32_t rank, int32_t n_ranks, const void *all
 /* same-process variant (several bands of one process, tests): raw device pointers [n_ranks][DWT_PEER_BUFFERS] */
 int dwt_get_peer_buffers(dwt_handle *h, void **out /* [DWT_PEER_BUFFERS] */);
 int dwt_attach_peers(dwt_handle *h, int32_t rank, int32_t n_ranks, void *const *table);
+/* Both attach calls also allocate the fp64 reset planes (otherwise allocated by the first dwt_upload_covers /
+   dwt_init_random), so that no band of a peer-memory world allocates device memory once any band may be stepping. */
 /* rows[n_ranks]: the band height of every rank, in rank order (they add up to N). Needed before either attach call when
    the bands differ in height: a band writes its last row into the ghost row below its upper neighbour's band. Without
    it, attaching assumes equal bands and refuses with DW_E_STATE when rows * n_ranks != N. */
@@ -213,6 +219,46 @@ int dwt_get_pool_ptr(dwt_handle *h, double **pool /* device [H, H] */, int32_t *
 int dwt_get_pool(dwt_handle *h, double *out /* host [H, H] */);               /* synchronises */
 /* L of the last step's forward (the L of the reset before any step), for the bare-planet temperature; as dw_get_last_L */
 int dwt_get_last_L(dwt_handle *h, double *L);
+
+/* ---- snapshots: a band's state out of and back into a handle, exactly --------------------------------------------------
+ * A band's state is its current state, the pre-state the last step started from (observations, DW_POLICY_MLP and the
+ * diagnostics read it), L_last, done_at and agents_done_at; the agents and the clock have their own getters and setters.
+ * Each of the two states is held in one representation:
+ *   DWT_REP_LATTICE  packed u32 words (light milli-cover | dark << 16), row by row, N words per row, no padding;
+ *   DWT_REP_PLANES   fp64 covers [2][rows][N] (light plane, then dark): the off-lattice state of a reset or upload;
+ *   DWT_REP_NONE     absent (the pre-state right after a reset or upload, and after dwt_debug_time_stencil).
+ * The current state is planes until the first step and the lattice after it; the pre-state is none, then the planes after
+ * the first step, then the lattice. None of it depends on the banding, so a snapshot taken on one partition of the world
+ * can be restored on any other. */
+enum { DWT_REP_NONE = 0, DWT_REP_PLANES = 1, DWT_REP_LATTICE = 2 };
+typedef struct dwt_band_state {
+    int32_t cur_rep, pre_rep;   /* DWT_REP_* of the current state and of the pre-state */
+    double L_last;              /* dwt_get_last_L */
+    int64_t done_at;            /* dwt_get_lifespans */
+    uint64_t cur_bytes;         /* bytes of cur_rows of dwt_save_state (the band's own rows); 0 for DWT_REP_NONE */
+    uint64_t pre_bytes;         /* bytes of pre_rows of dwt_save_state */
+} dwt_band_state;
+/* The band's state -> host. meta always receives the representations, L_last, done_at and the byte sizes, so a first call
+   with NULL rows sizes the buffers. cur_rows / pre_rows (when not NULL) receive the band's OWN rows [rows][N] in their
+   representation, agents_done_at (when not NULL) n counters. Staged through a page-locked buffer of the handle (about
+   (rows + 2) * N * 4 bytes, allocated on first use). DW_E_STATE while the snapshot would not be a whole step: between
+   dwt_move_graze and dwt_finish_agents, in peer-memory mode before dwt_flush_p2p, and while a chunk is open (call
+   dwt_end_chunk first). Synchronises. */
+int dwt_save_state(dwt_handle *h, dwt_band_state *meta, void *cur_rows, void *pre_rows, int64_t *agents_done_at);
+/* Replaces the band's state. cur_rows / pre_rows hold the band's rows WITH both ghost rows, global rows row0 - 1 .. row0 +
+   rows (toroidal), i.e. rows + 2 rows in the representation meta names (pre_rows is ignored for DWT_REP_NONE); the ghost
+   columns are written on the device, so no exchange between bands is needed. Sets L_last, done_at and agents_done_at[n]
+   (NULL: zero), drops any look-ahead decisions and observation, returns the claim arrays to idle and clears the per-step
+   maxima and series rows. Keeps the lattice buffer parity (every rank of a peer-memory world must keep the same one).
+   Allocates the fp64 planes when the snapshot holds planes. DW_E_INVALID for an unknown representation or a pair that
+   cannot occur (the pre-state is at most one step behind); DW_E_STATE while a step's agents are not finished (as
+   dwt_save_state). In peer-memory mode every rank meets every other (any collective) before and after this call. If it fails
+   after its checks (a copy or an allocation), the band's old state is partly overwritten: every call that reads the state
+   then fails with DW_E_STATE until dwt_upload_covers, dwt_init_random or a successful dwt_restore_state. Synchronises. */
+int dwt_restore_state(dwt_handle *h, const dwt_band_state *meta, const void *cur_rows, const void *pre_rows,
+                      const int64_t *agents_done_at);
+/* dwt_cover_checksum of the pre-state when it is on the lattice (DW_E_STATE otherwise) */
+int dwt_pre_checksum(dwt_handle *h, uint64_t *out /*[4]*/);
 
 #ifdef __cplusplus
 }

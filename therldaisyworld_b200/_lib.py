@@ -59,7 +59,17 @@ TILED_SYMBOLS = [
     "dwt_flush_p2p", "dwt_peer_status", "dwt_set_series", "dwt_get_series_ptr", "dwt_get_series", "dwt_get_pitch", "dwt_set_peer_rows",
     "dwt_observe", "dwt_get_obs_ptr", "dwt_get_obs", "dwt_set_mlp",
     "dwt_get_diag", "dwt_get_diag_stats", "dwt_get_cover_stats", "dwt_pool", "dwt_get_pool_ptr", "dwt_get_pool", "dwt_get_last_L",
+    "dwt_save_state", "dwt_restore_state", "dwt_pre_checksum",
 ]
+
+
+# representations of a band's state in a snapshot (dwt_band_state)
+DWT_REP = {"none": 0, "planes": 1, "lattice": 2}
+
+
+class DwtBandState(C.Structure):
+    _fields_ = [("cur_rep", C.c_int32), ("pre_rep", C.c_int32), ("L_last", C.c_double), ("done_at", C.c_int64),
+                ("cur_bytes", C.c_uint64), ("pre_bytes", C.c_uint64)]
 
 
 class DwtPtrs(C.Structure):
@@ -202,6 +212,9 @@ def load():
         "dwt_get_pool_ptr": (C.c_int, [vp, C.POINTER(vp), pi32]),
         "dwt_get_pool": (C.c_int, [vp, pd]),
         "dwt_get_last_L": (C.c_int, [vp, pd]),
+        "dwt_save_state": (C.c_int, [vp, C.POINTER(DwtBandState), vp, vp, pi64]),
+        "dwt_restore_state": (C.c_int, [vp, C.POINTER(DwtBandState), vp, vp, pi64]),
+        "dwt_pre_checksum": (C.c_int, [vp, C.POINTER(u64)]),
     }
     assert set(tsig) == set(TILED_SYMBOLS)
     sig.update(tsig)

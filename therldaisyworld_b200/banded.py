@@ -28,12 +28,14 @@ an agent / the winner of a graze stores straight into every rank's exchange vect
 into the neighbours' ghost rows, ranks meet at device-side flag barriers.  Only the per-chunk MAX all-reduce remains.
 """
 import ctypes as C
+import json
+import os
 
 import numpy as np
 
 from . import _lib
-from ._lib import DwClock, DwtPtrs, DW_DIAG, DW_POLICY, DWT_FIELD
-from .env import make_clock_struct, make_config_struct, set_default_attributes, set_default_kernels
+from ._lib import DwClock, DwtPtrs, DW_DIAG, DW_POLICY, DWT_FIELD, DWT_REP
+from .env import RLDaisyWorld, make_clock_struct, make_config_struct, set_default_attributes, set_default_kernels
 
 _WORLD_POLICIES = ("greedy", "antigreedy", "eps_greedy")      # decisions that (may) read the grid: need the act exchange
 
@@ -52,6 +54,45 @@ def balanced_rows(N, world_size, rank):
     if not 0 <= rank < world_size:
         raise ValueError(f"rank {rank} outside 0..{world_size - 1}")
     return rank * N // world_size, (rank + 1) * N // world_size
+
+
+# ---- snapshots (BandedDaisyWorld.save / restore)
+SNAPSHOT_FORMAT = 1
+_REP_NAME = {v: k for k, v in DWT_REP.items()}
+# the constants a snapshot carries: RLDaisyWorld's configuration plus the other dw_config scalars, and the arrays
+_SNAPSHOT_CONSTANTS = RLDaisyWorld._CONFIG_KEYS + ("q", "q2", "dt", "ddL", "ramp_up_down")
+_SNAPSHOT_ARRAYS = ("daisy_kernel", "local_albedo_kernel", "adjacent_albedo_kernel", "neighborhood")
+_CLOCK_KEYS = ("L", "dL", "min_L", "max_L", "ddL", "step_count", "ramp_period", "ramp_up_down")
+
+
+def _rep_layout(rep, rows, N):
+    """(shape, dtype) of `rows` rows of a state in representation rep (a DWT_REP value); (None, None) for none."""
+    if rep == DWT_REP["lattice"]:
+        return (rows, N), np.uint32
+    if rep == DWT_REP["planes"]:
+        return (2, rows, N), np.float64
+    return None, None
+
+
+def shard_name(which, lo, hi):
+    """File of a snapshot shard: the rows [lo, hi) of the current state ("cur") or pre-state ("pre")."""
+    return f"{which}.rows-{lo:07d}-{hi:07d}.npy"
+
+
+def shard_pieces(ranges, N, first, count):
+    """[(k, a, b)]: world rows first .. first + count - 1 (toroidal), in order, as row slices [a, b) of the shards whose
+    global rows are ranges[k] = (lo, hi). The ranges must tile [0, N)."""
+    cover = sorted(ranges)
+    if not cover or cover[0][0] != 0 or cover[-1][1] != N or any(p[1] != q[0] for p, q in zip(cover, cover[1:])):
+        raise ValueError(f"the shards {cover} do not tile the rows 0..{N - 1}")
+    out, g, left = [], first % N, count
+    while left:
+        k = next(k for k, (lo, hi) in enumerate(ranges) if lo <= g < hi)
+        lo, hi = ranges[k]
+        take = min(hi - g, left)
+        out.append((k, g - lo, g - lo + take))
+        g, left = (g + take) % N, left - take
+    return out
 
 
 class DistComm:
@@ -155,6 +196,59 @@ class DeviceBand:
         self._check(self._lib.dwt_init_random(self._h, C.c_uint64(seed), params.light_proportion, params.dark_proportion,
                                               params.initial_al, params.initial_ad), "dwt_init_random")
         self._views = {}
+
+    def set_agents(self, agent_indices, agent_states):
+        """all n agents, global coordinates (dwt_upload_agents); the covers are left alone"""
+        if self.n:
+            ai = np.ascontiguousarray(agent_indices, dtype=np.int64).reshape(self.n, 2)
+            st = np.ascontiguousarray(agent_states, dtype=np.float64).reshape(self.n)
+            self._check(self._lib.dwt_upload_agents(self._h, ai.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                    st.ctypes.data_as(C.POINTER(C.c_double))), "dwt_upload_agents")
+
+    # ---- snapshots (dwt_save_state / dwt_restore_state)
+    def save_state(self, alloc=None):
+        """(meta, cur, pre, agents_done_at): the band's own rows of its current state and of its pre-state in their
+        representation -- lattice: uint32 [rows, N] packed words, planes: float64 [2, rows, N] --, pre None when there is
+        no pre-state; meta {cur_rep, pre_rep, L_last, done_at} with DWT_REP names. alloc(which, shape, dtype) ("cur" /
+        "pre") supplies the arrays to fill, e.g. memory maps of the files they go to; default np.empty."""
+        alloc = alloc or (lambda which, shape, dtype: np.empty(shape, dtype=dtype))
+        m = _lib.DwtBandState()
+        self._check(self._lib.dwt_save_state(self._h, C.byref(m), None, None, None), "dwt_save_state")
+        arrays = {}
+        for which, rep in (("cur", m.cur_rep), ("pre", m.pre_rep)):
+            shape, dtype = _rep_layout(rep, self.rows, self.N)
+            arrays[which] = alloc(which, shape, dtype) if shape else None
+        ada = np.zeros(max(self.n, 1), dtype=np.int64)
+        ptr = lambda a: None if a is None else a.ctypes.data
+        self._check(self._lib.dwt_save_state(self._h, C.byref(m), ptr(arrays["cur"]), ptr(arrays["pre"]),
+                                             ada.ctypes.data_as(C.POINTER(C.c_int64))), "dwt_save_state")
+        meta = dict(cur_rep=_REP_NAME[m.cur_rep], pre_rep=_REP_NAME[m.pre_rep], L_last=m.L_last, done_at=int(m.done_at))
+        return meta, arrays["cur"], arrays["pre"], ada[:self.n]
+
+    def restore_state(self, meta, cur_rows, pre_rows, agents_done_at):
+        """Replace the band's state (dwt_restore_state): cur_rows / pre_rows hold the band's rows WITH both ghost rows
+        (rows + 2), in the layout save_state returns; meta as save_state returns it."""
+        m = _lib.DwtBandState(cur_rep=DWT_REP[meta["cur_rep"]], pre_rep=DWT_REP[meta["pre_rep"]], L_last=float(meta["L_last"]),
+                              done_at=int(meta["done_at"]))
+        keep = []
+
+        def ptr(a, rep):
+            shape, dtype = _rep_layout(DWT_REP.get(rep, -1), self.rows + 2, self.N)
+            if a is None or not shape:
+                return None
+            a = np.ascontiguousarray(a, dtype=dtype)
+            assert a.shape == shape, (a.shape, shape)
+            keep.append(a)
+            return a.ctypes.data
+
+        ada = np.ascontiguousarray(agents_done_at, dtype=np.int64).reshape(self.n) if self.n else np.zeros(1, dtype=np.int64)
+        self._check(self._lib.dwt_restore_state(self._h, C.byref(m), ptr(cur_rows, meta["cur_rep"]), ptr(pre_rows, meta["pre_rep"]),
+                                                ada.ctypes.data_as(C.POINTER(C.c_int64))), "dwt_restore_state")
+
+    def pre_checksum(self):
+        out = (C.c_uint64 * 4)()
+        self._check(self._lib.dwt_pre_checksum(self._h, out), "dwt_pre_checksum")
+        return [int(v) for v in out]
 
     # ---- phases
     def _replay_ptr(self, policy, actions, K=None):
@@ -466,6 +560,115 @@ class BandedDaisyWorld:
     def set_mlp(self, params):
         """MLP.set_parameters (daisy/agents/mlp.py) for policy="mlp": 1808 weights, flat layout of MLP.get_parameters."""
         self.band.set_mlp(params)
+
+    # ---- snapshots: the whole world's state to a directory and back, exactly, on any banding
+    def _sum_u64(self, words):
+        """The sum over the ranks of each 64-bit word, mod 2^64, on every rank: one _table of 16-bit limbs (exact in fp64)."""
+        limbs = [(int(w) >> (16 * j)) & 0xffff for w in words for j in range(4)]
+        tot = self._table(limbs).sum(axis=0)
+        return [sum(int(tot[4 * i + j]) << (16 * j) for j in range(4)) & ((1 << 64) - 1) for i in range(len(words))]
+
+    def _band_checksums(self, cur_rep, pre_rep):
+        """this band's dwt_cover_checksum of the current state and of the pre-state (zeros where not on the lattice)"""
+        cur = self.band.cover_checksum() if cur_rep == "lattice" else [0] * 4
+        pre = self.band.pre_checksum() if pre_rep == "lattice" else [0] * 4
+        return cur + pre
+
+    def save(self, path):
+        """Write the world's state to the directory `path`, exactly: every rank its own rows of the current state and the
+        pre-state (cur.rows-<lo>-<hi>.npy, pre.rows-...), rank 0 world.json (clock, counters, constants, checksums) and
+        agents.npz. Collective when world_size > 1: every rank calls it. MLP weights and eps_greedy's epsilon are policy
+        parameters, not world state, and are not saved. restore() takes the snapshot back on any banding of a world with the
+        same N and n."""
+        self.end_chunk()                             # pending gains applied, lifespans folded: the state of a whole step
+        b = self.band
+        lo, hi = self.row0, self.row0 + self.rows
+        os.makedirs(path, exist_ok=True)
+        meta, cur, pre, ada = b.save_state()
+        # np.save of an array in memory: writing through a memory map of the file was measured slower (tools/tiled_bench.py)
+        for which, a in (("cur", cur), ("pre", pre)):
+            if a is not None:
+                np.save(os.path.join(path, shard_name(which, lo, hi)), a)
+        sums = self._sum_u64(self._band_checksums(meta["cur_rep"], meta["pre_rep"]))
+        # (peer-memory mode: that collective also keeps the next step's halo push off the pre-state until every rank read it)
+        if self.rank == 0:
+            ai, st = b.agents()
+            np.savez(os.path.join(path, "agents.npz"), indices=ai, states=st, agents_done_at=ada)
+            clk = b.get_clock()
+            world = dict(format=SNAPSHOT_FORMAT, N=self.dim, n_agents=self.n_agents,
+                         writer=dict(world_size=self.world_size, mode=self.mode,
+                                     rows=[list(balanced_rows(self.dim, self.world_size, r)) for r in range(self.world_size)]),
+                         cur_rep=meta["cur_rep"], pre_rep=meta["pre_rep"], clock={k: getattr(clk, k) for k in _CLOCK_KEYS},
+                         step_count=self.step_count, first_done_step=self.first_done_step, L_last=meta["L_last"],
+                         done_at=meta["done_at"], cover_checksum=sums[:4] if meta["cur_rep"] == "lattice" else None,
+                         pre_checksum=sums[4:] if meta["pre_rep"] == "lattice" else None,
+                         constants={k: np.asarray(getattr(self, k)).item() for k in _SNAPSHOT_CONSTANTS},
+                         arrays={k: np.asarray(getattr(self, k)).tolist() for k in _SNAPSHOT_ARRAYS})
+            with open(os.path.join(path, "world.json"), "w") as f:
+                json.dump(world, f, indent=1)
+        if self.comm is not None:
+            self._table([0.0])                       # the snapshot is whole on disk once save() returns on any rank
+
+    @staticmethod
+    def read_snapshot_meta(path):
+        with open(os.path.join(path, "world.json")) as f:
+            return json.load(f)
+
+    def _snapshot_rows(self, path, world, which):
+        """This band's rows with both ghost rows (rows + 2, toroidal) of the snapshot's current state or pre-state, gathered
+        from whichever shards hold them; None when the snapshot has no such state."""
+        rep = world[f"{which}_rep"]
+        if rep == "none":
+            return None
+        ranges = [tuple(r) for r in world["writer"]["rows"]]
+        shards = [np.load(os.path.join(path, shard_name(which, lo, hi)), mmap_mode="r") for lo, hi in ranges]
+        shape, _ = _rep_layout(DWT_REP[rep], None, self.dim)
+        for (lo, hi), s in zip(ranges, shards):
+            want = tuple(hi - lo if d is None else d for d in shape)
+            if s.shape != want:
+                raise ValueError(f"snapshot shard {shard_name(which, lo, hi)} has shape {s.shape}, expected {want}")
+        axis = 0 if rep == "lattice" else 1
+        parts = [shards[k][a:b] if axis == 0 else shards[k][:, a:b]
+                 for k, a, b in shard_pieces(ranges, self.dim, self.row0 - 1, self.rows + 2)]
+        return np.concatenate(parts, axis=axis)
+
+    def restore(self, path):
+        """Replace the world's whole state by the snapshot in `path` (save()): covers, pre-state, agents, clock, lifespan
+        counters and constants. Works on any world_size and mode with the same N and n; refuses another N, n or format
+        before touching the device. Nothing of the world's earlier history remains, so one snapshot can be restored many
+        times into the same world (branching). Verifies the whole-world checksums of the lattice states and raises
+        DaisyWorldError on a mismatch (a corrupted shard, or shards of two saves). Collective when world_size > 1."""
+        world = self.read_snapshot_meta(path)
+        if world.get("format") != SNAPSHOT_FORMAT:
+            raise ValueError(f"snapshot format {world.get('format')!r}, this version reads {SNAPSHOT_FORMAT}")
+        if (world["N"], world["n_agents"]) != (self.dim, self.n_agents):
+            raise ValueError(f"snapshot of N={world['N']}, n={world['n_agents']} does not fit this world (N={self.dim}, "
+                             f"n={self.n_agents})")
+        cur, pre = self._snapshot_rows(path, world, "cur"), self._snapshot_rows(path, world, "pre")
+        with np.load(os.path.join(path, "agents.npz")) as z:
+            ai, st, ada = z["indices"], z["states"], z["agents_done_at"]
+        self._flush()
+        if self.mode == "p2p":
+            self._table([0.0])                       # no neighbour's last halo push may still land in this band's ghost rows
+        for k, v in world["constants"].items():
+            setattr(self, k, v)
+        for k, v in world["arrays"].items():
+            setattr(self, k, np.array(v, dtype=np.float64))
+        self.band.set_params(self)
+        self.band.restore_state(dict(cur_rep=world["cur_rep"], pre_rep=world["pre_rep"], L_last=world["L_last"],
+                                     done_at=world["done_at"]), cur, pre, ada)
+        self.band.set_agents(ai, st)
+        for k, v in world["clock"].items():
+            setattr(self, k, v)
+        self.band.set_clock(make_clock_struct(self))
+        self.step_count, self.first_done_step = world["step_count"], world["first_done_step"]
+        self._pending, self._gain_pending = 0, False
+        # also the closing collective: no rank steps while a neighbour still writes its rows
+        sums = self._sum_u64(self._band_checksums(world["cur_rep"], world["pre_rep"]))
+        for name, got in (("cover_checksum", sums[:4]), ("pre_checksum", sums[4:])):
+            if world[name] is not None and got != world[name]:
+                raise _lib.DaisyWorldError(f"restore({path!r}): the {name} of the restored world {got} differs from the snapshot's "
+                                           f"{world[name]} (a corrupted shard, or shards of two saves); restore or reset again")
 
     # ---- stepping
     def step(self, policy="greedy", actions_step=None, seed=0):

@@ -348,6 +348,15 @@ __global__ void __launch_bounds__(256) k_band_ghost_rows_wrap(BandGeom G, uint32
     lat[c] = lat[(size_t)G.R * G.pitch + c];
     lat[(size_t)(G.R + 1) * G.pitch + c] = lat[(size_t)G.pitch + c];
 }
+// Ghost COLUMNS of stored rows 0 .. rows - 1 from the row's own columns (toroidal): word c0 - 1 <- column N - 1, word c0 + N
+// <- column 0. dwt_restore_state uploads the R + 2 rows of a snapshot without them; the padding words stay untouched.
+__global__ void __launch_bounds__(256) k_band_ghost_cols(BandGeom G, uint32_t *lat, int rows) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= rows) return;
+    uint32_t *row = lat + (size_t)r * G.pitch;
+    row[G.c0 - 1] = row[G.c0 + G.N - 1];
+    row[G.c0 + G.N] = row[G.c0];
+}
 
 // ---- first step: literal forward from the off-lattice fp64 cover planes [(R+2) x N] onto the padded lattice ---------
 // SERIES: also adds {sum sqrt(g)*T, sum milli-light, sum milli-dark} of the band's cells to series[0..2] (see k_tiled_step)

@@ -17,7 +17,14 @@ of an mlp step from torch.profiler (k_band_obs, k_mlp_act, ...), in a separate p
 
 --diag [N]: the diagnostics and plot feed (default N = 16384, N agents): diag_stats("temp"), image("temp", 16),
 image("grid_light", 16), cover_stats() and the device part of image() alone (dwt_pool), each timed with CUDA events around
-the whole call (download included), next to a greedy step, alternating over five repetitions."""
+the whole call (download included), next to a greedy step, alternating over five repetitions.
+
+--snapshot [N]: save() and restore() of the giant world (default N = 16384, N agents, after 3 greedy steps: lattice state and
+lattice pre-state, 4 B per cell each), split into the band's copies between device and host memory (dwt_save_state /
+dwt_restore_state with in-memory arrays: DMA through the page-locked staging buffer, host copies, ghost-column kernel),
+the file I/O of the .npy shards (to a temporary directory), the checksums, and the whole calls; next to the raw PCIe rate
+of one pinned device -> host / host -> device copy of the same size. Host clock around synchronising calls, three
+repetitions after a warm-up."""
 import sys, os, subprocess, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -209,6 +216,55 @@ def bench_diag(N, K=32, reps=5):
     print(f"  check: temp mean {t['mean']:.6f} K, std {t['std']:.6f}; mean of the 16-block image {img.mean():.6f}", flush=True)
 
 
+def bench_snapshot(N, reps=3):
+    import shutil, tempfile
+    w = BandedDaisyWorld(N, N)
+    w.reset_on_device(seed=1)
+    w.run(3, "greedy")
+    b = w.band
+    tmp = tempfile.mkdtemp(prefix="dw_snapshot_bench_")
+    path = os.path.join(tmp, "snap")
+
+    def clock(fn):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        r = fn()
+        torch.cuda.synchronize()
+        return (time.perf_counter() - t0) * 1e3, r
+
+    nbytes = N * N * 4
+    dev = torch.empty(nbytes // 4, dtype=torch.int32, device="cuda")
+    pin = torch.empty(nbytes // 4, dtype=torch.int32, pin_memory=True)
+    meta, cur, pre, ada = b.save_state()                # warm-up: staging buffer, page faults of the arrays
+    rows = np.concatenate([cur[-1:], cur, cur[:1]])        # the band's rows with both ghost rows (one band: the torus wrap)
+    prows = np.concatenate([pre[-1:], pre, pre[:1]])
+    b.restore_state(meta, rows, prows, ada)
+    w.save(path)
+    w.restore(path)
+    cs = w.cover_checksum()
+    times = {k: [] for k in ("pcie d2h (pinned, 1 copy)", "pcie h2d (pinned, 1 copy)", "save_state -> RAM (cur + pre)",
+                             "np.save of both shards", "save() whole", "read both shards (np.load)",
+                             "restore_state <- RAM (cur + pre)", "checksums (cur + pre)", "restore() whole")}
+    for _ in range(reps):
+        times["pcie d2h (pinned, 1 copy)"].append(clock(lambda: pin.copy_(dev))[0])
+        times["pcie h2d (pinned, 1 copy)"].append(clock(lambda: dev.copy_(pin))[0])
+        times["save_state -> RAM (cur + pre)"].append(clock(lambda: b.save_state(lambda which, shape, dtype: cur if which == "cur" else pre))[0])
+        times["np.save of both shards"].append(clock(lambda: [np.save(os.path.join(tmp, f"{k}.npy"), a) for k, a in (("c", cur), ("p", pre))])[0])
+        times["save() whole"].append(clock(lambda: w.save(path))[0])
+        times["read both shards (np.load)"].append(clock(lambda: [np.array(np.load(os.path.join(tmp, f"{k}.npy"), mmap_mode="r")) for k in "cp"])[0])
+        times["restore_state <- RAM (cur + pre)"].append(clock(lambda: b.restore_state(meta, rows, prows, ada))[0])
+        times["checksums (cur + pre)"].append(clock(lambda: (b.cover_checksum(), b.pre_checksum()))[0])
+        times["restore() whole"].append(clock(lambda: w.restore(path))[0])
+    assert w.cover_checksum() == cs
+    shutil.rmtree(tmp)
+    print(f"N={N}, {N} agents, after 3 greedy steps (lattice + lattice pre-state, {nbytes / 2**30:.2f} GiB per state and band); "
+          f"{reps} repetitions, host clock around synchronising calls (ms)")
+    for k, ts in times.items():
+        print(f"  {k:36s} ms: " + " ".join(f"{t:.1f}" for t in ts) + f" | median {np.median(ts):.1f}")
+    print(f"  pcie floor of one state: {nbytes / np.median(times['pcie d2h (pinned, 1 copy)']) / 1e6:.1f} GB/s d2h, "
+          f"{nbytes / np.median(times['pcie h2d (pinned, 1 copy)']) / 1e6:.1f} GB/s h2d", flush=True)
+
+
 def bench_vs_ensemble(N, K=200, reps=5):
     from therldaisyworld_b200 import RLDaisyWorld
     n = 4
@@ -255,6 +311,11 @@ if __name__ == "__main__":
         args = [a for a in sys.argv[1:] if a != "--diag"]
         print(f"GPU: {gpu_label()}")
         bench_diag(int(args[0]) if args else 16384)
+        sys.exit(0)
+    if "--snapshot" in sys.argv:
+        args = [a for a in sys.argv[1:] if a != "--snapshot"]
+        print(f"GPU: {gpu_label()}")
+        bench_snapshot(int(args[0]) if args else 16384)
         sys.exit(0)
     if "--series" in sys.argv:
         args = [a for a in sys.argv[1:] if a != "--series"]
