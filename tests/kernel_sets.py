@@ -108,3 +108,137 @@ def apply_draw(env, attrs):
             setattr(env, k, v)
     env.q = 0.2 * env.S / env.sigma
     env.set_use_microclimate(attrs["use_microclimate"])
+
+
+# (N, B, n) -> kernel family of the fused path (csrc/dw_run.inl::fused_kernel)
+SHAPES = {
+    (64, 6, 4): "64x64 persistent", (16, 9, 4): "sub-64", (8, 70, 3): "sub-64, partial CTA group", (20, 5, 3): "4x4 tile",
+    (13, 4, 3): "padded tile", (33, 3, 5): "padded tile, odd N", (5, 3, 2): "generic", (2, 2, 1): "degenerate wrap",
+    (1, 2, 1): "degenerate wrap",
+}
+
+
+# Shocks that move a cover by thousands of milli-covers in one step. The low word of the lattice kernels' rounding sum holds
+# x + 0.5 (x = 1000 (l + dt dl), milli-cover) with only 12 integer bits, exact for x + 0.5 in [-2048, 2048); the kernels take
+# the value from both words (csrc/dw_fused.cuh, DESIGN.md section 2). Far from T_opt, beta = 1 - g (T_opt - T)^2 is strongly
+# negative. Every scenario leaves the 12-bit window and stays inside the tile loops' 16-bit one (window_crossings counts
+# both). Every scenario is reached through plain attributes:
+#   ctor    constructor keywords          attrs   attributes set before reset()
+#   grow    steps before the shocked one  shock   attributes set right before the shocked step, put back after it
+#   settle  steps after it                crosses whether the shocked step leaves the window (window_crossings proves it)
+# A luminosity shock is not put back: the clock carries on from it (update_L clamps it into [min_L, max_L]).
+# heat_step needs no shock: ramp_period=1 puts L at max_L after the literal first step, so step 2, the first step of the fast
+# path, runs at max_L.
+SCENARIOS = {
+    "heat_step": dict(ctor=dict(ramp_period=1), attrs=dict(max_L=2.5), grow=1, shock={}, settle=20, crosses=True),
+    "heat_graze": dict(ctor=dict(ramp_period=1), attrs=dict(max_L=2.0), grow=1, shock={}, settle=20, crosses=True),
+    "heat_pulse": dict(ctor={}, attrs={}, grow=40, shock=dict(L=2.5), settle=20, crosses=True),
+    "cold_pulse": dict(ctor={}, attrs={}, grow=40, shock=dict(L=0.1), settle=20, crosses=True),
+    "upper_edge": dict(ctor={}, attrs={}, grow=40, shock=dict(dt=12.0, gamma=0.0), settle=20, crosses=True),
+}
+WINDOW = 2048.0          # |x + 0.5| bound of the fast path's low rounding word alone (12 integer bits), milli-cover
+WIDE_WINDOW = 32768.0    # |x + 0.5| bound of the tile loops' rounding (funnel shift of both words, 16 bits)
+
+
+def make_env(cls, name, N, B, n, seed):
+    """An env of class `cls` (product or NumPy oracle) reset into scenario `name`'s starting state."""
+    sc = SCENARIOS[name]
+    np.random.seed(seed)
+    env = cls(grid_dimension=N, n_agents=n, **sc["ctor"])
+    env.batch_size = B
+    for k, v in sc["attrs"].items():
+        setattr(env, k, v)
+    env.reset()
+    return env
+
+
+def apply_shock(name, *envs):
+    """Set scenario `name`'s shock on every env (product, oracle or COracleWorld); returns the values to put back."""
+    saved = []
+    for env in envs:
+        old = {}
+        for k, v in SCENARIOS[name]["shock"].items():
+            if hasattr(env, "clk") and hasattr(env, "P"):            # oracle.daisy_c.COracleWorld: clock and parameter structs
+                target = env.clk if k == "L" else env.P
+            else:
+                target = env
+            old[k] = getattr(target, k)
+            setattr(target, k, v)
+        saved.append(old)
+    return saved
+
+
+def undo_shock(name, saved, *envs):
+    """Put back what apply_shock changed, except the luminosity, which the clock has moved on from."""
+    for env, old in zip(envs, saved):
+        for k, v in old.items():
+            if k == "L":
+                continue
+            setattr(env.P if hasattr(env, "clk") and hasattr(env, "P") else env, k, v)
+
+
+def window_crossings(name, N=64, B=4, n=4, seed=1, actions=None, state=None):
+    """Run scenario `name` on the NumPy oracle up to its shocked step and
+    return (below, above, wide, finite): how many cover updates of that step have 1000 (l + dt dl) + 0.5 below -WINDOW, at or
+    above +WINDOW, and outside [-WIDE_WINDOW, WIDE_WINDOW), and whether every field of the step is finite. Counted from the
+    unrounded fields(), so it holds whatever the kernels do. Agents: greedy, or actions[t] ([K, B, n] replay), or
+    actions(obs) (a policy); state = (light, dark, agent_indices, agent_states) of one world replaces the reset state.
+    """
+    from oracle.daisy_numpy import OracleDaisyWorld, OracleGreedy
+    sc = SCENARIOS[name]
+    env = make_env(OracleDaisyWorld, name, N, B, n, seed)
+    if state is not None:
+        light, dark, ai, st = state
+        env.batch_size = 1
+        env.grid = np.zeros((1, 7, N, N))
+        env.grid[0, 1], env.grid[0, 2] = light, dark
+        env.agent_indices, env.agent_states = np.array(ai)[None].copy(), np.array(st, dtype=float)[None, :, None].copy()
+    agent = OracleGreedy()
+    obs = env.get_obs(env.agent_indices)
+
+    def act(t, obs):
+        if actions is None:
+            return agent(obs)
+        return actions(obs) if callable(actions) else np.asarray(actions[t]).reshape(env.batch_size, -1, 1)
+
+    for t in range(sc["grow"]):
+        obs, _, _, _ = env.step(act(t, obs))
+    saved = apply_shock(name, env)
+    seen = {}
+    forward = env.forward
+
+    def spy(grid):
+        seen["f"] = env.fields(grid[:, 1].copy(), grid[:, 2].copy())
+        seen["l"], seen["d"] = grid[:, 1].copy(), grid[:, 2].copy()
+        return forward(grid)
+
+    env.forward = spy
+    try:
+        env.step(act(sc["grow"], obs))
+    finally:
+        del env.forward
+    f = seen["f"]
+    x = np.stack([1000.0 * (seen["l"] + env.dt * f["dl"]), 1000.0 * (seen["d"] + env.dt * f["dd"])]) + 0.5
+    undo_shock(name, saved, env)
+    finite = all(np.isfinite(v).all() for v in f.values())
+    return int((x < -WINDOW).sum()), int((x >= WINDOW).sum()), int(((x < -WIDE_WINDOW) | (x >= WIDE_WINDOW)).sum()), finite
+
+
+def update_bound(L, dt=1.0, gamma=0.25, g=0.003265, S=1000.0, sigma=5.67e-8, p=1.0, ab=0.5, al=0.75, ad=0.25, Topt=295.5,
+                 microclimate=True):
+    """Upper bound of |x - k| (milli-cover) over every lattice state, for one step at luminosity L with the reference's kernels:
+    rho (milli) <= 1000, |rho_b| <= dt max(p, 2 - p), and beta >= 1 - g (T_opt - T)^2 over the temperatures the fast path's
+    linear form of T^4 reaches with covers in [0, 1000] and neighbour sums in [0, 8000]. inf when T^4 can reach 0."""
+    q = 0.2 * S / sigma
+    q2 = q / 8.0 if microclimate else 0.0
+    a, cl, cd, cL = 0.125, (al - ab) / 1000.0, (ad - ab) / 1000.0, S * L / sigma
+    x0 = cL + (q - cL) * ab * p * 8 * a + (q2 - q) * ab * p - q2 * al
+    terms = ((q2 - q) * cl * 1000, (q2 - q) * cd * 1000, (q - cL) * a * cl * 8000, (q - cL) * a * cd * 8000)
+    lo, hi = x0 + sum(min(0.0, t) for t in terms), x0 + sum(max(0.0, t) for t in terms)
+    xdd = q2 * (al - ad)
+    lo, hi = min(lo, lo + xdd), max(hi, hi + xdd)
+    if lo <= 0:
+        return np.inf
+    dev = max(abs(Topt - lo ** 0.25), abs(Topt - hi ** 0.25))
+    beta = max(1.0, g * dev * dev - 1.0)
+    return 1000.0 * (abs(dt) * max(p, 2 - p) * beta + abs(dt * gamma))

@@ -6,16 +6,10 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from kernel_sets import ASYMMETRIC, DRAWS, KERNEL_SETS, apply_draw, set_kernels
+from kernel_sets import ASYMMETRIC, DRAWS, KERNEL_SETS, SHAPES, apply_draw, set_kernels  # noqa: F401 (SHAPES: the families)
 
 pytestmark = pytest.mark.gpu
 
-# (N, B, n) -> kernel family of the fused path (csrc/dw_run.inl::fused_kernel)
-SHAPES = {
-    (64, 6, 4): "64x64 persistent", (16, 9, 4): "sub-64", (8, 70, 3): "sub-64, partial CTA group", (20, 5, 3): "4x4 tile",
-    (13, 4, 3): "padded tile", (33, 3, 5): "padded tile, odd N", (5, 3, 2): "generic", (2, 2, 1): "degenerate wrap",
-    (1, 2, 1): "degenerate wrap",
-}
 MAIN = [(64, 6, 4), (16, 9, 4), (20, 5, 3), (33, 3, 5), (5, 3, 2)]
 
 

@@ -98,11 +98,29 @@ template <bool HI>
 __device__ __forceinline__ double dw_half2d(uint32_t p) {
     return HI ? (double)(unsigned short)(p >> 16) : (double)(unsigned short)(p & 0xffffu);
 }
-// Rounding of x (milli units) to the lattice with the tie filter folded into ONE add: f = low word of
-// x + (1.5*2^32 + 0.5 + EPS*2^-FIX) = round((x + 0.5) * 2^FIX) + EPS as a signed fixed-point number.
-//   floor(x + .5) = f >> FIX   unless frac(x + .5) is within EPS*2^-FIX below 1 -- but then the cell is flagged anyway;
-//   tie flag: frac(x + .5) * 2^FIX + EPS (mod 2^FIX) < 2 EPS   <=>   (unsigned)(f << (32-FIX)) < F.tie_thresh.
+// Rounding of x (milli units) to the lattice with the tie filter folded into ONE add: v = x + (1.5*2^32 + 0.5 + EPS*2^-FIX)
+// has the ulp 2^-FIX, and its mantissa holds round((x + 0.5) * 2^FIX) + EPS as a signed fixed-point number F offset by 2^51
+// (|x| < 2^31). f = low word of v, h = high word:
+//   tie flag: frac(x + .5) * 2^FIX + EPS (mod 2^FIX) < 2 EPS   <=>   (unsigned)(f << (32-FIX)) < F.tie_thresh;
+//   floor(x + .5) = F >> FIX   unless frac(x + .5) is within EPS*2^-FIX below 1 -- but then the cell is flagged anyway.
+// The low word alone holds only 12 integer bits of F >> FIX and wraps modulo 4096 outside x + .5 in [-2048, 2048): a cell that
+// dies by 2100 milli-cover in one step would come back at 1000. So the value is taken with ONE funnel shift of both words,
+// (h:f) >> FIX, whose low 16 bits are F >> FIX exactly for x + .5 in [-32768, 32768) (DW_WIDE_WINDOW) -- the same instruction
+// count as a shift of f alone. The s16x2 clamp to [0, 1000] then saturates like the reference's clip (which comes before its
+// rounding). dw_fast_cell saturates any x; the tile loops' dw_fast_cells stay exact inside the 16-bit window, which holds
+// every cell update whose bound |x - k| <= rho_max (rho_b,max |beta|_max + dt gamma) is below 31768 (DESIGN.md section 2).
 // EPS is chosen per handle on the host (F.magic, F.tie_thresh).
+#define DW_WIDE_WINDOW 32768
+#define DW_MAGIC_HI 0x41F80000      // high word of v for x + .5 in [0, 4096): (h - DW_MAGIC_HI) = F >> 32
+
+// floor(x + .5) clamped to [0, 1000] from the words of v, for any x. Inf and NaN sums (X' <= 0: NaN temperatures, where the
+// reference's grid is NaN too) keep what the low word always gave them, (f >> FIX) clamped.
+__device__ __forceinline__ unsigned dw_round_any(int h, int f) {
+    if ((h & 0x7ff00000) == 0x7ff00000) return (unsigned)min(max(f >> DW_FIX_BITS, 0), 1000);
+    if (h < 0x41F00000 || h > 0x41FFFFFF) return h > DW_MAGIC_HI ? 1000u : 0u;    // |x| >= 2^31 (signed: v < 0 is below)
+    const long long F = ((long long)(h - DW_MAGIC_HI) << 32) + (long long)(unsigned)f;
+    return (unsigned)min(max(F >> DW_FIX_BITS, 0ll), 1000ll);
+}
 
 // One cell of the fast path. pc: packed centre, E: packed sum of the 4 edge neighbours, S: packed sum of all 8.
 // Returns the packed new cell; *tiemin is lowered below F.tie_thresh when either species sits within the filter of
@@ -124,10 +142,14 @@ __device__ __forceinline__ uint32_t dw_fast_cell(const FastCoef &F, const StepCo
     const double bd = __fma_rn(-dTd, dTd, 1.0);
     const double xl = __fma_rn(Rl, __fma_rn(rb, bl, -F.dtg), kl);             // l + dt*dl in milli units
     const double xd = __fma_rn(Rd, __fma_rn(rb, bd, -F.dtg), kd);
-    const int fl = __double2loint(xl + F.magic), fd = __double2loint(xd + F.magic);
+    const double vl = xl + F.magic, vd = xd + F.magic;
+    const int fl = __double2loint(vl), fd = __double2loint(vd), hl = __double2hiint(vl), hd = __double2hiint(vd);
     *tiemin = __vimin3_u32(*tiemin, (unsigned)fl << (32 - DW_FIX_BITS), (unsigned)fd << (32 - DW_FIX_BITS));
+    // outside the 16-bit window of the tile loops' rounding (rare): saturate
+    if ((unsigned)(hl - (DW_MAGIC_HI - 8)) >= 16u || (unsigned)(hd - (DW_MAGIC_HI - 8)) >= 16u)
+        return dw_round_any(hl, fl) | (dw_round_any(hd, fd) << 16);
     // floor(x + .5) of both species packed as s16x2, clamped to [0,1000] by one VIMNMX.S16x2.RELU
-    const unsigned packed = __byte_perm((unsigned)(fl >> DW_FIX_BITS), (unsigned)(fd >> DW_FIX_BITS), 0x5410);
+    const unsigned packed = __byte_perm(__funnelshift_r(fl, hl, DW_FIX_BITS), __funnelshift_r(fd, hd, DW_FIX_BITS), 0x5410);
     return __vimin_s16x2_relu(packed, 1000u | (1000u << 16));
 }
 
@@ -194,9 +216,12 @@ __device__ __forceinline__ void dw_fast_cells(const FastCoef &F, const StepCoef 
     for (int i = 0; i < W; ++i) { zl[i] = __fma_rn(Rl[i], zl[i], kl[i]); zd[i] = __fma_rn(Rd[i], zd[i], kd[i]); }     // l + dt*dl (milli)
 #pragma unroll
     for (int i = 0; i < W; ++i) {
-        const int fl = __double2loint(zl[i] + F.magic), fd = __double2loint(zd[i] + F.magic);
+        const double vl = zl[i] + F.magic, vd = zd[i] + F.magic;
+        const int fl = __double2loint(vl), fd = __double2loint(vd);
         *tiemin = __vimin3_u32(*tiemin, (unsigned)fl << (32 - DW_FIX_BITS), (unsigned)fd << (32 - DW_FIX_BITS));
-        const unsigned packed = __byte_perm((unsigned)(fl >> DW_FIX_BITS), (unsigned)(fd >> DW_FIX_BITS), 0x5410);
+        // funnel shift of both words: exact inside DW_WIDE_WINDOW (see the rounding note)
+        const unsigned packed = __byte_perm(__funnelshift_r(fl, __double2hiint(vl), DW_FIX_BITS),
+                                            __funnelshift_r(fd, __double2hiint(vd), DW_FIX_BITS), 0x5410);
         out[i] = __vimin_s16x2_relu(packed, 1000u | (1000u << 16));
     }
 }
