@@ -220,6 +220,32 @@ int dwt_get_pool(dwt_handle *h, double *out /* host [H, H] */);               /*
 /* L of the last step's forward (the L of the reset before any step), for the bare-planet temperature; as dw_get_last_L */
 int dwt_get_last_L(dwt_handle *h, double *L);
 
+/* ---- fp32 mode: the band's grid as float32, evaluated with fp32 arithmetic from the lattice ------------------------------
+ * The grid of dwt_get_grid, [7, rows, N] float32 (ch4: the agent stamp), the giant world's counterpart of dw_get_grid_f32:
+ * the temperatures (channels 3..5) are evaluated in binary32 from the post-graze pre-state at S * L of the last step (within
+ * 1e-5 relative of the fp64 grid), the bare fraction is screened against a proven fp32 error bound and otherwise finished by
+ * the fp64 fast path and the literal cell, so channels 0, 1, 2 and 6 are the exact binary32 roundings of dwt_get_grid's.
+ * 36 bytes of device memory traffic per cell against 64 or more for the fp64 grid, and no fp64 scratch. Right after the
+ * first step of a reset or upload (the pre-state is the fp64 planes) the fp64 grid is converted, exactly
+ * dwt_get_grid's values rounded to float32; those cells do not count in dwt_f32_stats.
+ * DW_E_STATE without a pre-state (before the first step after an upload / reset / restore of a snapshot without one, after
+ * dwt_debug_time_stencil), while a step's agents are not finished (between dwt_move_graze and dwt_finish_agents; in
+ * peer-memory mode until dwt_flush_p2p) and after a failed dwt_restore_state; DW_E_INVALID for NULL pointers.
+ * Reading the pre-state races with the next step's halo push in peer-memory mode: a caller meets every rank (any
+ * collective) after these calls and before the next dwt_step_p2p. */
+/* materialise into the device buffer float [7, rows, N] (allocated on first use, 28 bytes per band cell) on the handle's
+   stream, without synchronising; the buffer is overwritten by the next call */
+int dwt_grid_f32(dwt_handle *h);
+int dwt_get_grid_f32_ptr(dwt_handle *h, float **grid /* device [7, rows, N] */);
+int dwt_get_grid_f32(dwt_handle *h, float *out /* host [7, rows, N] */);     /* dwt_grid_f32 + download; synchronises */
+/* out[3] = {cells evaluated with fp32 arithmetic, cells whose bare fraction went on to the fp64 tier, cells that needed the
+   literal cell}, cumulative over the handle's life. Synchronises. */
+int dwt_f32_stats(dwt_handle *h, uint64_t *out /*[3]*/);
+/* Measurement hook: average device time (microseconds, CUDA events) of `reps` back-to-back materialisations after one
+   warm-up: fp32 != 0 the work of dwt_grid_f32, fp32 == 0 that of dwt_get_grid without its download. Refuses like
+   dwt_grid_f32. */
+int dwt_debug_time_materialise(dwt_handle *h, int32_t fp32, int32_t reps, double *us_per_call);
+
 /* ---- snapshots: a band's state out of and back into a handle, exactly --------------------------------------------------
  * A band's state is its current state, the pre-state the last step started from (observations, DW_POLICY_MLP and the
  * diagnostics read it), L_last, done_at and agents_done_at; the agents and the clock have their own getters and setters.

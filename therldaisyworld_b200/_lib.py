@@ -60,6 +60,7 @@ TILED_SYMBOLS = [
     "dwt_observe", "dwt_get_obs_ptr", "dwt_get_obs", "dwt_set_mlp",
     "dwt_get_diag", "dwt_get_diag_stats", "dwt_get_cover_stats", "dwt_pool", "dwt_get_pool_ptr", "dwt_get_pool", "dwt_get_last_L",
     "dwt_save_state", "dwt_restore_state", "dwt_pre_checksum",
+    "dwt_grid_f32", "dwt_get_grid_f32_ptr", "dwt_get_grid_f32", "dwt_f32_stats", "dwt_debug_time_materialise",
 ]
 
 
@@ -215,6 +216,11 @@ def load():
         "dwt_save_state": (C.c_int, [vp, C.POINTER(DwtBandState), vp, vp, pi64]),
         "dwt_restore_state": (C.c_int, [vp, C.POINTER(DwtBandState), vp, vp, pi64]),
         "dwt_pre_checksum": (C.c_int, [vp, C.POINTER(u64)]),
+        "dwt_grid_f32": (C.c_int, [vp]),
+        "dwt_get_grid_f32_ptr": (C.c_int, [vp, C.POINTER(vp)]),
+        "dwt_get_grid_f32": (C.c_int, [vp, C.POINTER(C.c_float)]),
+        "dwt_f32_stats": (C.c_int, [vp, C.POINTER(u64)]),
+        "dwt_debug_time_materialise": (C.c_int, [vp, i32, i32, pd]),
     }
     assert set(tsig) == set(TILED_SYMBOLS)
     sig.update(tsig)

@@ -451,6 +451,37 @@ class DeviceBand:
         self._check(self._lib.dwt_get_grid(self._h, out.ctypes.data_as(C.POINTER(C.c_double))), "dwt_get_grid")
         return out
 
+    # ---- fp32 mode (dwt_grid_f32 .. dwt_f32_stats)
+    def grid_f32(self):
+        """The band's grid [7, rows, N] as float32 (dwt_get_grid_f32): channels 0, 1, 2, 6 and the agent stamp the binary32
+        roundings of grid()'s, temperatures evaluated with fp32 arithmetic (within 1e-5 relative)."""
+        out = np.empty((7, self.rows, self.N), dtype=np.float32)
+        self._check(self._lib.dwt_get_grid_f32(self._h, out.ctypes.data_as(C.POINTER(C.c_float))), "dwt_get_grid_f32")
+        return out
+
+    def grid_f32_tensor(self):
+        """Launch the fp32 materialisation (dwt_grid_f32, on the handle's stream) and return the device buffer [7, rows, N]
+        as a torch view; the next call overwrites it."""
+        self._check(self._lib.dwt_grid_f32(self._h), "dwt_grid_f32")
+        p = C.c_void_p()
+        self._check(self._lib.dwt_get_grid_f32_ptr(self._h, C.byref(p)), "dwt_get_grid_f32_ptr")
+        return self._view(p.value, (7, self.rows, self.N), "<f4")
+
+    def f32_stats(self):
+        """Tier counters of the fp32 materialisation: cells evaluated with fp32 arithmetic, cells whose bare fraction went on
+        to the fp64 tier, cells that needed the literal cell (cumulative)."""
+        out = (C.c_uint64 * 3)()
+        self._check(self._lib.dwt_f32_stats(self._h, out), "dwt_f32_stats")
+        return {"cells": int(out[0]), "fp64_tier": int(out[1]), "literal": int(out[2])}
+
+    def time_materialise(self, fp32, reps=10):
+        """Device microseconds per materialisation (dwt_debug_time_materialise): fp32 mode, or the fp64 grid without its
+        download."""
+        us = C.c_double(0.0)
+        self._check(self._lib.dwt_debug_time_materialise(self._h, 1 if fp32 else 0, int(reps), C.byref(us)),
+                    "dwt_debug_time_materialise")
+        return us.value
+
     # ---- diagnostics and plot feed (the unrounded fields of the last forward; dwt_get_diag .. dwt_pool)
     def diag(self, name):
         """The band's field `name` (a DW_DIAG key) of the last forward: [rows, N], growth [2, rows, N] (dl, dd)."""
@@ -855,6 +886,43 @@ class BandedDaisyWorld:
         """[7, rows, N]: env.grid[0] restricted to this rank's rows."""
         self._flush()
         return self.band.grid()
+
+    # ---- fp32 mode: the grid of local_grid() as float32, evaluated with fp32 arithmetic from the lattice
+    def _fenced(self, fn):
+        """fn() on the band after the last step's agents are finished; in peer-memory mode followed by the fence that keeps
+        every rank's next step (its halo push into the pre-state this reads) behind every rank's call, as local_diag."""
+        self._flush()
+        out = fn()
+        if self.mode == "p2p":
+            self.band.synchronize()                  # the pre-state is read before this rank meets the others
+            self._table([0.0])
+        self._check_peers()
+        return out
+
+    def local_grid_f32(self):
+        """[7, rows, N] float32: local_grid() in fp32 mode. Channels 0, 1, 2, 6 and the agent stamp on channel 4 equal
+        local_grid().astype(np.float32); the temperatures are evaluated with fp32 arithmetic, within 1e-5 relative. Half the
+        download of local_grid() and no fp64 scratch on the device. In peer-memory mode every rank must call it."""
+        return self._fenced(self.band.grid_f32)
+
+    def local_grid_f32_tensor(self):
+        """local_grid_f32() as a torch.float32 CUDA tensor [7, rows, N] on the band's device, without leaving the device (the
+        materialisation is complete when it returns). It aliases library memory: the next local_grid_f32() or
+        local_grid_f32_tensor() overwrites it -- clone() what must outlive that. In peer-memory mode every rank must call it."""
+        def grid():
+            t = self.band.grid_f32_tensor()
+            self.band.synchronize()
+            return t
+        return self._fenced(grid)
+
+    def f32_stats(self):
+        """Tier counters of fp32 mode summed over the ranks: {cells, fp64_tier, literal} (see DeviceBand.f32_stats).
+        Collective when world_size > 1."""
+        self._flush()
+        s = self.band.f32_stats()
+        tot = self._sum_u64([s["cells"], s["fp64_tier"], s["literal"]])
+        self._check_peers()
+        return dict(cells=tot[0], fp64_tier=tot[1], literal=tot[2])
 
     # ---- diagnostics and plot feed (DESIGN.md §0 row (f) N3): what the reference's notebook helpers read from
     # RLDaisyWorld (notebook_helpers.py:45-57,139-150,210-223), reduced on the device per band and merged over the ranks.

@@ -66,24 +66,18 @@ __device__ __forceinline__ void dw_fast_x(const FastCoef &F, const StepCoef &C, 
     xd = __fma_rn(Rd, __fma_rn(rb, __fma_rn(-dTd, dTd, 1.0), -F.dtg), kd);
 }
 
-// fp64 tier of the bare fraction of one cell (rare: ~2 % of cells; out of line, called after the thread's stores so that
-// nothing of the fp32 evaluation is live across the call). Returns 1000 b' as the reference rounds it.
-// Measured alternatives (4000 worlds of 64x64, this in-place call: 0.185 ms): deferring the ~3e5 flagged cells to a dense second
-// kernel through a work list costs more than the divergence it removes -- one shared counter 0.257 ms (the warp-aggregated
-// atomics serialise), per-warp list segments without atomics 0.230 ms.
-__device__ __noinline__ float dw_f32_bare_slow(const DevParams *Pp, const FastCoef *Fp, const StepCoef *Cp, const uint32_t *g, unsigned N,
-                                               unsigned x, unsigned y, unsigned *nlit) {
-    const DevParams &P = *Pp;
-    const unsigned xm = x == 0 ? N - 1 : x - 1, xp = x == N - 1 ? 0 : x + 1;
-    const unsigned ym = y == 0 ? N - 1 : y - 1, yp = y == N - 1 ? 0 : y + 1;
-    const uint32_t *r0 = g + xm * N, *r1 = g + x * N, *r2 = g + xp * N;
-    const uint32_t pc = r1[y];
-    const uint32_t E = r1[ym] + r1[yp] + r0[y] + r2[y];
-    const uint32_t S = E + r0[ym] + r0[yp] + r2[ym] + r2[yp];
+// fp64 tier of the bare fraction of one cell, shared by the fp32-mode kernels of the ensemble and of the giant world
+// (csrc/dw_tiled.cuh) so that the tiers cannot diverge between the two lattice layouts. In: the cell's packed word pc, its
+// neighbourhood sums E, S, and win(a, c) = the packed word of the window cell in row a, column c (0..2; (1, 1) is the cell)
+// for the literal cell. Returns 1000 b' as the reference rounds it. A window over scalars: capturing index arrays makes
+// the compiler drop the non-coherent loads of k_forward_f32's main loop.
+template <class Win>
+__device__ __forceinline__ float dw_f32_bare_tiers(const DevParams &P, const FastCoef &F, const StepCoef &C, uint32_t pc, uint32_t E,
+                                                   uint32_t S, Win win, unsigned *nlit) {
     // lattice fast path, unrounded covers -> b' with the tie filter of the screened forward (P.eps_b, units of 0.001);
     // then the literal cell. (Range failures come here too: the fp64 fast path is exact-or-flagged on its own.)
     double dxl, dxd;
-    dw_fast_x(*Fp, *Cp, pc, E, S, dxl, dxd);
+    dw_fast_x(F, C, pc, E, S, dxl, dxd);
     dxl = fmin(fmax(dxl, 0.0), 1000.0);
     dxd = fmin(fmax(dxd, 0.0), 1000.0);
     const double dxb = (1000.0 * P.p - dxl) - dxd;
@@ -92,19 +86,36 @@ __device__ __noinline__ float dw_f32_bare_slow(const DevParams *Pp, const FastCo
     if (!in_range || !(0.5 - fabs(dxb - kb64) > P.eps_b)) {
         *nlit += 1;
         double l9[9], d9[9];
-        const unsigned xs[3] = {xm, x, xp}, ys[3] = {ym, y, yp};
 #pragma unroll
         for (int a = 0; a < 3; ++a)
 #pragma unroll
             for (int c = 0; c < 3; ++c) {
-                const uint32_t k = g[xs[a] * N + ys[c]];
+                const uint32_t k = win(a, c);
                 l9[a * 3 + c] = dw_milli(k & 0xffffu);
                 d9[a * 3 + c] = dw_milli(k >> 16);
             }
-        const LitCell o = dw_literal_cell(P, Cp->SL, l9, d9);
+        const LitCell o = dw_literal_cell(P, C.SL, l9, d9);
         kb64 = rint(o.nb * 1000.0);
     }
     return (float)kb64;
+}
+
+// fp64 tier of cell (x, y) of a wrapped N x N lattice (rare: ~2 % of cells; out of line, called after the thread's stores so
+// that nothing of the fp32 evaluation is live across the call).
+// Measured alternatives (4000 worlds of 64x64, this in-place call: 0.185 ms): deferring the ~3e5 flagged cells to a dense second
+// kernel through a work list costs more than the divergence it removes -- one shared counter 0.257 ms (the warp-aggregated
+// atomics serialise), per-warp list segments without atomics 0.230 ms.
+__device__ __noinline__ float dw_f32_bare_slow(const DevParams *Pp, const FastCoef *Fp, const StepCoef *Cp, const uint32_t *g, unsigned N,
+                                               unsigned x, unsigned y, unsigned *nlit) {
+    const unsigned xm = x == 0 ? N - 1 : x - 1, xp = x == N - 1 ? 0 : x + 1;
+    const unsigned ym = y == 0 ? N - 1 : y - 1, yp = y == N - 1 ? 0 : y + 1;
+    const uint32_t *r0 = g + xm * N, *r1 = g + x * N, *r2 = g + xp * N;
+    const uint32_t pc = r1[y];
+    const uint32_t E = r1[ym] + r1[yp] + r0[y] + r2[y];
+    const uint32_t S = E + r0[ym] + r0[yp] + r2[ym] + r2[yp];
+    return dw_f32_bare_tiers(*Pp, *Fp, *Cp, pc, E, S, [=](int a, int c) {
+        return g[(a == 0 ? xm : a == 1 ? x : xp) * N + (c == 0 ? ym : c == 1 ? y : yp)];
+    }, nlit);
 }
 
 struct F32Out { float b, T, Tl, Td; bool ok; };

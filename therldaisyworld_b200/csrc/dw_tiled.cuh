@@ -26,6 +26,7 @@
 #pragma once
 #include <cuda.h>
 
+#include "dw_f32.cuh"
 #include "dw_fused.cuh"
 
 struct BandGeom {
@@ -731,22 +732,113 @@ __global__ void __launch_bounds__(256) k_band_lookahead_decide(BandGeom G, const
 
 // ---- materialisation / synthetic reset -------------------------------------------------------------------------------
 // full reference grid [7, R, N] of the band, materialised by a literal forward from the post-graze state the last step
-// started from: the other lattice buffer, or the fp64 planes when that step was the first one after a reset
-template <class Pre>
-__global__ void __launch_bounds__(256) k_band_materialise(DevParams P, double SL, BandGeom G, Pre pre, double *__restrict__ out) {
+// started from: the other lattice buffer, or the fp64 planes when that step was the first one after a reset.
+// T = float: the fp32 grid of that state, each value rounded in fp64 and then converted once (fp32 mode of a planes pre-state).
+template <class Pre, class T>
+__global__ void __launch_bounds__(256) k_band_materialise(DevParams P, double SL, BandGeom G, Pre pre, T *__restrict__ out) {
     const size_t RN = (size_t)G.R * G.N;
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < RN; i += (size_t)gridDim.x * blockDim.x) {
         const int r = (int)(i / G.N), y = (int)(i - (size_t)r * G.N);
         double l9[9], d9[9];
         pre.load9(G, r, y, l9, d9);
         const LitCell o = dw_literal_cell(P, SL, l9, d9);
-        out[i] = dw_round3(o.nb);
-        out[RN + i] = dw_round3(o.nl);
-        out[2 * RN + i] = dw_round3(o.nd);
-        out[3 * RN + i] = dw_round3(o.T);
-        out[4 * RN + i] = dw_round3(o.Tl);
-        out[5 * RN + i] = dw_round3(o.Td);
-        out[6 * RN + i] = 0.0;
+        out[i] = (T)dw_round3(o.nb);
+        out[RN + i] = (T)dw_round3(o.nl);
+        out[2 * RN + i] = (T)dw_round3(o.nd);
+        out[3 * RN + i] = (T)dw_round3(o.T);
+        out[4 * RN + i] = (T)dw_round3(o.Tl);
+        out[5 * RN + i] = (T)dw_round3(o.Td);
+        out[6 * RN + i] = (T)0.0;
+    }
+}
+
+// ---- fp32 mode: the band's grid [7, R, N] as float32, evaluated with fp32 arithmetic from the lattice ---------------------
+// The per-cell arithmetic of k_forward_f32 (csrc/dw_f32.cuh) in the band geometry: the 3x3 neighbourhood of band row r comes
+// from stored rows r .. r+2 of the post-graze pre-state, columns c0 + y - 1 .. c0 + y + W, all in place with the ghost rows
+// and columns, so the kernel is a plain grid-stride walk over R x N cells without wrap arithmetic or tile masks. Traffic:
+// 4 B of pre-state and 4 B of current state read, 28 B written per cell.
+// fp64 tier of the cell at p of the padded lattice (out of line, after the thread's stores, like dw_f32_bare_slow)
+__device__ __noinline__ float dwt_f32_bare_slow(const DevParams *Pp, const FastCoef *Fp, const StepCoef *Cp, const uint32_t *p, int pitch,
+                                                unsigned *nlit) {
+    const uint32_t *q0 = p - pitch, *q2 = p + pitch;
+    const uint32_t pc = p[0];
+    const uint32_t E = p[-1] + p[1] + q0[0] + q2[0];
+    const uint32_t S = E + q0[-1] + q0[1] + q2[-1] + q2[1];
+    return dw_f32_bare_tiers(*Pp, *Fp, *Cp, pc, E, S, [=](int a, int c) { return p[(a - 1) * pitch + (c - 1)]; }, nlit);
+}
+// W cells per thread: W = 2 (N even) loads 8 B and stores float2 -- a stored row starts 16 B aligned (pitch a multiple of 4
+// words), c0 = 4 and y is even; W = 1 for odd N (3 CTAs per SM: at the 64 registers of 4 it spills around the fp64-tier call). pre: post-graze pre-state lattice, cur: the lattice after that step.
+// out: float [7, R, N], channels 0..6 (4 before the agent stamp). stats[0] += cells sent to the fp64 tier, stats[1] += cells
+// that needed the literal cell (per-warp sums).
+struct BandF32Args { DevParams P; FastCoef F; StepCoef C; F32Coef Q; BandGeom G; };
+template <int W>
+__global__ void __launch_bounds__(256, W == 2 ? 4 : 3) k_band_forward_f32(const __grid_constant__ BandF32Args A, const uint32_t *__restrict__ pre,
+                                                             const uint32_t *__restrict__ cur, float *__restrict__ out,
+                                                             unsigned long long *stats) {
+    const F32Coef &Q = A.Q;
+    const int pitch = A.G.pitch;
+    const unsigned N = (unsigned)A.G.N, gN = N / W;
+    const size_t RN = (size_t)A.G.R * N, total = (size_t)A.G.R * gN, stride = (size_t)gridDim.x * blockDim.x;
+    size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+    CellWalk w(i, stride, gN);                           // b: band row, c: group of W columns
+    unsigned n64 = 0, nlit = 0;
+    for (; i < total; i += stride, w.next()) {
+        const unsigned r = w.b, y = W * w.c;
+        const uint32_t *p = pre + (size_t)r * pitch + A.G.c0 + y;     // stored row r = the row above band row r
+        uint32_t row[3][W + 2];                          // rows r-1, r, r+1 of the band; columns y-1 .. y+W
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            const uint32_t *q = p + a * pitch;
+            row[a][0] = q[-1];
+            if (W == 2) {
+                const uint2 v = *reinterpret_cast<const uint2 *>(q);
+                row[a][1] = v.x; row[a][2] = v.y;
+            } else row[a][1] = q[0];
+            row[a][W + 1] = q[W];
+        }
+        const uint32_t *pc_cur = cur + (size_t)(r + 1) * pitch + A.G.c0 + y;
+        uint32_t pn[W];
+        if (W == 2) {
+            const uint2 v = *reinterpret_cast<const uint2 *>(pc_cur);
+            pn[0] = v.x; pn[W - 1] = v.y;
+        } else pn[0] = pc_cur[0];
+        float ch[7][W];
+        bool ok[W];
+#pragma unroll
+        for (int c = 0; c < W; ++c) {
+            const uint32_t pc = row[1][c + 1];
+            const uint32_t E = row[1][c] + row[1][c + 2] + row[0][c + 1] + row[2][c + 1];
+            const uint32_t S = E + row[0][c] + row[0][c + 2] + row[2][c] + row[2][c + 2];
+            const F32Out o = dw_f32_cell(Q, pc, E, S);
+            ok[c] = o.ok;
+            ch[0][c] = dw_div1000f(o.b);
+            ch[1][c] = dw_div1000f(dw_half2f<0>(pn[c]));
+            ch[2][c] = dw_div1000f(dw_half2f<1>(pn[c]));
+            ch[3][c] = dw_round3f(o.T * Q.inv_sqrt_g);
+            ch[4][c] = dw_round3f(o.Tl * Q.inv_sqrt_g);
+            ch[5][c] = dw_round3f(o.Td * Q.inv_sqrt_g);
+            ch[6][c] = 0.0f;
+        }
+        float *ob = out + (size_t)r * N + y;
+#pragma unroll
+        for (int q = 0; q < 7; ++q) {
+            if (W == 2) *reinterpret_cast<float2 *>(ob + (size_t)q * RN) = make_float2(ch[q][0], ch[q][W - 1]);
+            else ob[(size_t)q * RN] = ch[q][0];
+        }
+        // cells whose fp32 bare fraction sits within its error bound of a rounding tie (or outside the accepted range):
+        // fp64 tier, the stored channel 0 is overwritten
+#pragma unroll
+        for (int c = 0; c < W; ++c) {
+            if (!ok[c]) {
+                n64 += 1;
+                ob[c] = dw_div1000f(dwt_f32_bare_slow(&A.P, &A.F, &A.C, p + pitch + c, pitch, &nlit));
+            }
+        }
+    }
+    if (stats) {
+        n64 = __reduce_add_sync(__activemask(), n64);
+        nlit = __reduce_add_sync(__activemask(), nlit);
+        if ((threadIdx.x & 31) == 0 && n64) { atomicAdd(stats, (unsigned long long)n64); atomicAdd(stats + 1, (unsigned long long)nlit); }
     }
 }
 // lattice covers of the band as fp64 planes [2, R, N] (k/1000 exactly as np.round stores them)
@@ -784,14 +876,16 @@ __global__ void __launch_bounds__(256) k_band_stamp_claim(BandGeom G, const int3
     const int lr = band_owned_row(G, xy[2 * i]);
     if (lr >= 0) atomicMin(claim + (size_t)lr * G.N + xy[2 * i + 1], n - 1 - i);
 }
+// ch4: channel 4 of the fp64 grid, or of the fp32 grid (T = float: the agent's state converted once)
+template <class T>
 __global__ void __launch_bounds__(256) k_band_stamp_write(BandGeom G, const int32_t *__restrict__ xy, const double *__restrict__ st, int n,
-                                                          int *claim, double *ch4, int pass) {
+                                                          int *claim, T *ch4, int pass) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int lr = band_owned_row(G, xy[2 * i]);
     if (lr < 0) return;
     const size_t c = (size_t)lr * G.N + xy[2 * i + 1];
-    if (pass == 0) { if (claim[c] == n - 1 - i) ch4[(size_t)(lr - 1) * G.N + xy[2 * i + 1]] = st[i]; }
+    if (pass == 0) { if (claim[c] == n - 1 - i) ch4[(size_t)(lr - 1) * G.N + xy[2 * i + 1]] = (T)st[i]; }
     else claim[c] = 0x7fffffff;
 }
 

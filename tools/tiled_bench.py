@@ -24,7 +24,14 @@ lattice pre-state, 4 B per cell each), split into the band's copies between devi
 dwt_restore_state with in-memory arrays: DMA through the page-locked staging buffer, host copies, ghost-column kernel),
 the file I/O of the .npy shards (to a temporary directory), the checksums, and the whole calls; next to the raw PCIe rate
 of one pinned device -> host / host -> device copy of the same size. Host clock around synchronising calls, three
-repetitions after a warm-up."""
+repetitions after a warm-up.
+
+--f32 [N]: fp32 mode (default N = 16384, N agents, after 3 greedy steps: lattice pre-state): the device time of one
+materialisation in fp32 mode (k_band_forward_f32 + stamp) and of the fp64 grid (k_band_materialise + stamp) through
+dwt_debug_time_materialise, warmed up, the two arms alternating over five repetitions of 10 calls; cells/s, algorithmic
+bytes (fp32: 4 + 4 B read, 28 B written per cell; fp64: 4 B read, 56 B written) and their share of the 7.7 TB/s data-sheet
+HBM bandwidth; the fp64-tier and literal fractions (f32_stats); the host wall time of local_grid_f32() and local_grid()
+(download included), three repetitions each."""
 import sys, os, subprocess, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -265,6 +272,45 @@ def bench_snapshot(N, reps=3):
           f"{nbytes / np.median(times['pcie h2d (pinned, 1 copy)']) / 1e6:.1f} GB/s h2d", flush=True)
 
 
+def bench_f32(N, reps=5, calls=10):
+    w = BandedDaisyWorld(N, N)
+    w.reset_on_device(seed=1)
+    w.run(3, "greedy")
+    b = w.band
+    for fp32 in (True, False):                   # warm-up: module loading, the fp32 buffer and the fp64 scratch
+        b.time_materialise(fp32, 2)
+    s0 = b.f32_stats()
+    times = {True: [], False: []}
+    for _ in range(reps):
+        for fp32 in (True, False):
+            times[fp32].append(b.time_materialise(fp32, calls))
+    s1 = b.f32_stats()
+    cells = N * N
+    tier, lit = (s1["fp64_tier"] - s0["fp64_tier"]) / (s1["cells"] - s0["cells"]), (s1["literal"] - s0["literal"]) / (s1["cells"] - s0["cells"])
+    print(f"N={N}, {N} agents, after 3 greedy steps; device time per materialisation (dwt_debug_time_materialise, CUDA events), "
+          f"{reps} alternating repetitions of {calls} calls")
+    for fp32, name, nbytes in ((True, "fp32 mode", 36), (False, "fp64 grid", 60)):
+        ts = np.array(times[fp32])
+        med = np.median(ts)
+        rate = nbytes * cells / (med * 1e-6)
+        print(f"  {name} us: " + " ".join(f"{t:.0f}" for t in ts) + f" | median {med:.0f} us = {cells / (med * 1e-6):.3e} cells/s, "
+              f"{nbytes} B/cell algorithmic = {rate / 1e12:.2f} TB/s = {rate / 7.7e12:.2f} of the 7.7 TB/s data-sheet HBM bandwidth")
+    print(f"  fp32 / fp64 device time: {np.median(times[True]) / np.median(times[False]):.3f}")
+    print(f"  fp32 mode tiers: {100 * tier:.3f} % of cells to the fp64 tier, {100 * lit:.5f} % to the literal cell")
+    host = {"local_grid_f32()": [], "local_grid()": []}
+    for _ in range(3):
+        for name, fn in (("local_grid_f32()", w.local_grid_f32), ("local_grid()", w.local_grid)):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            g = fn()
+            host[name].append((time.perf_counter() - t0) * 1e3)
+            del g
+    for name, ts in host.items():
+        print(f"  {name:17s} ms (host clock, download included): " + " ".join(f"{t:.0f}" for t in ts) + f" | median {np.median(ts):.0f}")
+    t = w.local_grid_f32_tensor()
+    print(f"  check: local_grid_f32_tensor() {tuple(t.shape)} {t.dtype}, mean T {t[3].double().mean().item():.4f} K", flush=True)
+
+
 def bench_vs_ensemble(N, K=200, reps=5):
     from therldaisyworld_b200 import RLDaisyWorld
     n = 4
@@ -316,6 +362,11 @@ if __name__ == "__main__":
         args = [a for a in sys.argv[1:] if a != "--snapshot"]
         print(f"GPU: {gpu_label()}")
         bench_snapshot(int(args[0]) if args else 16384)
+        sys.exit(0)
+    if "--f32" in sys.argv:
+        args = [a for a in sys.argv[1:] if a != "--f32"]
+        print(f"GPU: {gpu_label()}")
+        bench_f32(int(args[0]) if args else 16384)
         sys.exit(0)
     if "--series" in sys.argv:
         args = [a for a in sys.argv[1:] if a != "--series"]
